@@ -21,6 +21,25 @@ def test_bench_algorithmic_bytes_formula():
     assert [bench.dim_of(k) for k in (3, 4, 5, 6, 7, 8, 10)] == [32, 136, 512, 2080, 8192, 32896, 524800]
 
 
+def test_bench_dump_rows_is_a_fixed_sample_within_the_cap(tmp_path):
+    """--dump-outputs: small outputs are written whole; large ones as the same seeded row sample every run, under
+    DUMP_BYTES; f32 rows stay float32, u32 counts become exact float64."""
+    import torch
+    import bench
+    small = torch.arange(6 * 32, dtype=torch.int32).view(6, 32)
+    bench.dump_rows(small, "u32", tmp_path / "s.npy")
+    got = np.load(tmp_path / "s.npy")
+    assert got.dtype == np.float64 and np.array_equal(got, small.numpy())
+    big = torch.rand(2 * bench.DUMP_BYTES // (512 * 4), 512, generator=torch.Generator().manual_seed(0))
+    bench.dump_rows(big, "f32", tmp_path / "a.npy")
+    bench.dump_rows(big, "f32", tmp_path / "b.npy")
+    a, b = np.load(tmp_path / "a.npy"), np.load(tmp_path / "b.npy")
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_BYTES // (512 * 4), 512) and np.array_equal(a, b)
+    assert (tmp_path / "a.npy").stat().st_size <= bench.DUMP_BYTES + 4096
+    pick = np.sort(np.random.default_rng(bench.DUMP_SEED).choice(len(big), size=len(a), replace=False))
+    assert np.array_equal(a, big.numpy()[pick]) and len(np.unique(pick)) == len(a)
+
+
 def test_pack_helper_matches_oracle_pack():
     from kmertools_b200.oligo import _pack
     seqs = ["ACGT", "", "NNACGTTT", "acgu"]
