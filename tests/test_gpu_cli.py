@@ -73,6 +73,76 @@ def test_random_file_matches_oracle_text(tmp_path, k):
         assert out.read_bytes() == O.comp_oligo_text(fa, k, **kw), flags
 
 
+def _fasta(path, records, opener=open):
+    """records: (name, u8 array); sequences wrapped at 70 columns."""
+    with opener(path, "wb") as fh:
+        for name, seq in records:
+            fh.write(b">" + name + b"\n")
+            full = len(seq) // 70
+            lines = np.empty((full, 71), dtype=np.uint8)
+            lines[:, :70] = seq[:full * 70].reshape(full, 70)
+            lines[:, 70] = ord("\n")
+            fh.write(lines.tobytes())
+            if len(seq) % 70:
+                fh.write(seq[full * 70:].tobytes() + b"\n")
+
+
+def _oversized_seq(rng, n, runs):
+    seq = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, size=n, dtype=np.uint8)]
+    for _ in range(runs):
+        a = int(rng.integers(0, n - 100_000))
+        seq[a:a + int(rng.integers(1, 100_000))] = ord("N")
+    return seq
+
+
+OVERSIZED_FLAGS = ((["-k", 4], {}), (["-k", 7, "-c"], {"norm": False}), (["-k", 5, "-r"], {"canonical": False}))
+
+
+def test_records_larger_than_the_base_buffer(tmp_path):
+    """A FASTA file above 32 MiB whose records do not fit the 32 MiB base buffer of a batch: the driver grows the buffer
+    set that meets the 36 Mbp record to 1.25 x its size (45 Mbp), and the other set meets a 50 Mbp record after that,
+    so both grow, the second from the capacity the first growth set.  The same bytes on stdin, where the buffer starts
+    at 32 MiB whatever the input.  Totals above 2^23 also take format_norm_kernel's f64 division."""
+    rng = np.random.default_rng(36)
+
+    def short(n):
+        return [(b"s%d" % i, _oversized_seq(rng, int(m), 0)) for i, m in enumerate(rng.integers(0, 400, size=n))]
+
+    records = short(5) + [(b"big1", _oversized_seq(rng, 36_000_000, 4))] + short(7) + \
+        [(b"big2", _oversized_seq(rng, 50_000_000, 3))] + short(3)
+    fa = tmp_path / "big.fa"
+    _fasta(fa, records)
+    assert fa.stat().st_size > 32 << 20
+    data = fa.read_bytes()
+    out = tmp_path / "o"
+    for flags, kw in OVERSIZED_FLAGS:
+        want = O.comp_oligo_text(fa, flags[1], **kw)
+        r = run(["-i", fa, "-o", out, *flags])
+        assert r.returncode == 0 and r.stderr == b"", r.stderr
+        assert out.read_bytes() == want, flags
+        r = run(["-i", "-", "-o", out, *flags], stdin=data)
+        assert r.returncode == 0 and r.stderr == b"", r.stderr
+        assert out.read_bytes() == want, ["stdin", *flags]
+
+
+def test_gzip_record_far_larger_than_its_file(tmp_path):
+    """A 40 Mbp record of a repeated 1 kbp block compresses far below 1/8 of its size, so the base buffer sized from
+    the file (8 x its size + 1 MiB) is too small and grows from there."""
+    import gzip
+    rng = np.random.default_rng(40)
+    seq = np.tile(_oversized_seq(rng, 1000, 0), 40_000)
+    for a in rng.integers(0, seq.size - 5000, size=4):
+        seq[a:a + int(rng.integers(1, 5000))] = ord("N")
+    fa = tmp_path / "big.fa.gz"
+    _fasta(fa, [(b"s0", seq[:999]), (b"big", seq), (b"s2", seq[5:300])], opener=gzip.open)
+    assert fa.stat().st_size * 8 + (1 << 20) < seq.size
+    out = tmp_path / "o"
+    for flags, kw in OVERSIZED_FLAGS:
+        r = run(["-i", fa, "-o", out, *flags])
+        assert r.returncode == 0 and r.stderr == b"", r.stderr
+        assert out.read_bytes() == O.comp_oligo_text(fa, flags[1], **kw), flags
+
+
 def test_python_driver_and_many_batches(tmp_path):
     """comp_oligo() through ctypes; enough records for several GPU batches (rows stay in input order)."""
     from kmertools_b200 import io as kio
