@@ -118,6 +118,9 @@ int ktb_oligo_vectorise(ktb_oligo *h, const uint8_t *bases, const uint64_t *offs
 /* DEVICE-buffer entry point: same contract, but bases/offsets/out/totals are device pointers on the
  * handle's GPU and the work is enqueued on `stream` (a cudaStream_t; NULL = default stream).
  * Returns after enqueueing; results are ready when the stream reaches that point.
+ * Offsets are absolute positions in d_bases: offsets[0] may be any value <= offsets[n], so a sub-batch view
+ * (d_offsets + lo, n = hi - lo) of a batch resident in a larger buffer is valid input, at any offset.  total_bases must
+ * equal offsets[n]: the call reads no byte of d_bases at or beyond it (a smaller value changes the rows).
  * d_bases and d_out must be 16-byte aligned.  The handle owns work counters and scratch buffers, so calls
  * on ONE handle must be ordered with respect to each other (same stream, or event-chained); use one handle
  * per concurrent stream.  Scratch buffers (reject lists, the pool of the bucket path, the order list of long contigs)
