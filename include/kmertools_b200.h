@@ -99,7 +99,9 @@ int ktb_kmer_pairs(const uint8_t *seq, uint64_t len, int k, int device, uint64_t
                    uint64_t cap, uint64_t *count);
 
 /* Same on DEVICE buffers of the current device, enqueued on `stream` (a cudaStream_t; NULL = default stream);
- * scratch comes from the stream-ordered allocator.  Returns after enqueueing. */
+ * scratch comes from the stream-ordered allocator.  Returns after enqueueing.  *d_count is the full count (it may
+ * exceed 2^32) whatever cap is; no element of d_out_f / d_out_r at or beyond min(*d_count, cap) is written.  d_seq
+ * needs no alignment and may be NULL when len = 0; no byte outside [d_seq, d_seq + len) is read. */
 int ktb_kmer_pairs_device(const uint8_t *d_seq, uint64_t len, int k, uint64_t *d_out_f, uint64_t *d_out_r,
                           uint64_t cap, uint64_t *d_count, void *stream);
 

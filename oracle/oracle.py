@@ -95,6 +95,24 @@ def kmers(seq: bytes, k: int) -> list[tuple[int, int]]:
     return [(int(f[i]), int(r[i])) for i in range(m)]
 
 
+def kmer_arrays(buf, k: int, want_pairs: bool = True):
+    """kmers() as two uint64 arrays and the count, without building tuples: (f, r, count).  `buf` is bytes or a uint8
+    array (copied only when not contiguous).  With want_pairs=False only the count is computed and returned."""
+    if isinstance(buf, (bytes, bytearray, memoryview)):
+        buf = np.frombuffer(buf, dtype=np.uint8)
+    buf = np.ascontiguousarray(buf, dtype=np.uint8).reshape(-1)
+    n = buf.size
+    src = buf if n else np.zeros(1, dtype=np.uint8)
+    if not want_pairs:
+        return int(lib().ktb_oracle_kmers(src.ctypes.data, n, k, None, None))
+    cap = max(n - k + 1, 0)
+    f = np.empty(max(cap, 1), dtype=np.uint64)
+    r = np.empty(max(cap, 1), dtype=np.uint64)
+    m = int(lib().ktb_oracle_kmers(src.ctypes.data, n, k, f.ctypes.data, r.ctypes.data))
+    assert m <= cap
+    return f[:m], r[:m], m
+
+
 def kmer_pos_maps(k: int) -> tuple[np.ndarray, np.ndarray, int]:
     """(pos_map[4^k], pos_to_kmer[count], count) — kmer/src/kmer.rs:54-73."""
     n = 4 ** k

@@ -26,6 +26,25 @@ def test_kmers_generated_ambiguous():  # kmer.rs:130-145
     assert O.kmers(b"ACNGTT", 2) == [(1, 11), (11, 1), (15, 0)]
 
 
+def test_kmer_arrays_match_kmers():
+    """kmer_arrays (uint64 arrays, what the large GPU tests compare with) == kmers (tuples) on short sequences."""
+    rng = np.random.default_rng(11)
+    mixed = np.frombuffer(b"ACGTacgtUuNR\x00\x01\x02\x03\xc3\xa9", dtype=np.uint8)
+    seqs = [b"", b"A", b"ACGT", b"ACNGTT", b"NNNN", bytes(range(256)) * 2]
+    seqs += [mixed[rng.integers(0, len(mixed), size=n)].tobytes() for n in (5, 31, 32, 100, 777)]
+    for seq in seqs:
+        for k in (1, 2, 3, 15, 16, 17, 30, 31):
+            want = O.kmers(seq, k)
+            for buf in (seq, np.frombuffer(seq, dtype=np.uint8)):
+                f, r, m = O.kmer_arrays(buf, k)
+                assert f.dtype == r.dtype == np.uint64 and m == len(f) == len(r) == len(want), (seq[:16], k)
+                assert list(zip(f.tolist(), r.tolist())) == want, (seq[:16], k)
+                assert O.kmer_arrays(buf, k, want_pairs=False) == m
+    arr = np.frombuffer(b"ACGTTGCAACGTAGCT" * 4, dtype=np.uint8)
+    f, r, m = O.kmer_arrays(arr[::3], 5)   # a strided view is read as the bytes it shows
+    assert list(zip(f.tolist(), r.tolist())) == O.kmers(arr[::3].tobytes(), 5) and m > 0
+
+
 def test_rev_comp():  # kmer.rs:147-153
     assert O.rev_comp(0b00011011, 4) == 0b00011011
     assert O.rev_comp(0b001101101011, 6) == 0b000101100011
