@@ -9,6 +9,7 @@
 #include "span_writer.h"
 #include "textfmt.cuh"
 
+#include <atomic>
 #include <charconv>
 #include <sys/stat.h>
 #include <chrono>
@@ -76,6 +77,18 @@ struct Dev {
     ~Dev() { if (p) cudaFree(p); }
 };
 
+// Host-formatted text.  resize() leaves new bytes uninitialised: a part sized for the longest text its rows can have
+// touches (and keeps resident) only the pages the text is written to.
+template <class T>
+struct NoInitAlloc : std::allocator<T> {
+    template <class U> struct rebind { using other = NoInitAlloc<U>; };
+    NoInitAlloc() = default;
+    template <class U> NoInitAlloc(const NoInitAlloc<U> &) noexcept {}
+    template <class U> void construct(U *p) noexcept { ::new ((void *)p) U; }
+    template <class U, class... A> void construct(U *p, A &&...a) { ::new ((void *)p) U(std::forward<A>(a)...); }
+};
+using Text = std::vector<char, NoInitAlloc<char>>;
+
 struct Set {
     Pinned h_bases, h_offsets, h_out;
     Dev d_bases, d_offsets, d_counts, d_totals, d_text;
@@ -85,7 +98,7 @@ struct Set {
     bool pending = false;
     bool writing = false;                      // rows handed to the writer, buffers not reusable yet
     ktb::SpanWriter::Ticket ticket;
-    std::vector<std::vector<char>> parts;      // host-formatted text (counts / CGR), one part per formatting thread
+    std::vector<Text> parts;                   // host-formatted text (counts / CGR), one part per formatting thread
     ~Set() {
         if (kernels_done) cudaEventDestroy(kernels_done);
         if (stream) cudaStreamDestroy(stream);
@@ -144,7 +157,7 @@ void release_sets(SetPair *sp) {
 }
 
 // u32 counts of rows [r0, r1) -> "c0<d>c1<d>...\n" (format!("{}", f64) prints integral values without ".0", oligo.rs:138)
-void format_counts_rows(const uint32_t *counts, uint64_t r0, uint64_t r1, uint32_t dim, char delim, std::vector<char> *out) {
+void format_counts_rows(const uint32_t *counts, uint64_t r0, uint64_t r1, uint32_t dim, char delim, Text *out) {
     out->resize((size_t)(r1 - r0) * dim * 11 + 16);
     char *o = out->data();
     size_t w = 0;
@@ -161,7 +174,7 @@ void format_counts_rows(const uint32_t *counts, uint64_t r0, uint64_t r1, uint32
 
 // rows [0, n) cut into `threads` contiguous ranges, fn(r0, r1, part) run on one thread each (the `-t` of the CLI)
 template <typename F>
-void format_parallel(uint64_t n, int threads, std::vector<std::vector<char>> *parts, F fn) {
+void format_parallel(uint64_t n, int threads, std::vector<Text> *parts, F fn) {
     const uint64_t nt = std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)threads, n));
     parts->resize(nt);
     if (nt == 1) { fn(0, n, &(*parts)[0]); return; }
@@ -171,15 +184,22 @@ void format_parallel(uint64_t n, int threads, std::vector<std::vector<char>> *pa
     for (auto &x : th) x.join();
 }
 
-// Rust's `{}` for f64: shortest digits that round-trip, never an exponent (std::to_chars fixed does the same)
-inline char *put_f64(char *o, double v) {
-    auto r = std::to_chars(o, o + 400, v, std::chars_format::fixed);
-    return r.ptr;
+// Rust's `{}` for f64: shortest digits that round-trip, never an exponent (std::to_chars fixed does the same).
+// nullptr when the text does not fit in [o, end).
+inline char *put_f64(char *o, char *end, double v) {
+    auto r = std::to_chars(o, end, v, std::chars_format::fixed);
+    return r.ec == std::errc() ? r.ptr : nullptr;
 }
+
+// Longest text of one CGR value.  A count is a u32: at most 10 digits.  A frequency c / t with 1 <= c <= t < 2^64 is
+// 0, 1 or at least 2^-64 > 1e-20: "0." then at most 19 zeros before the first significant digit, and the shortest
+// round-trip form of an f64 has at most 17 significant digits, so 38 characters.
+constexpr size_t kCgrCountChars = 10;
+constexpr size_t kCgrFreqChars = 2 + 19 + 17;
 
 // composition/src/oligocgr.rs:123-143,165-190: every canonical k-mer gets a fixed point, the midpoint
 // recurrence from the centre towards the corner of each base (A (0,0), T (v,0), G (v,v), C (0,v))
-void cgr_prefixes(const ktb_oligo *h, int k, uint64_t dim, double vecsize, std::vector<std::string> *pref) {
+bool cgr_prefixes(const ktb_oligo *h, int k, uint64_t dim, double vecsize, std::vector<std::string> *pref) {
     std::vector<char> hb(dim * k);
     ktb_oligo_header(h, 1, hb.data(), hb.size());
     pref->resize(dim);
@@ -199,32 +219,39 @@ void cgr_prefixes(const ktb_oligo *h, int k, uint64_t dim, double vecsize, std::
         char buf[900];
         char *o = buf;
         *o++ = '(';
-        o = put_f64(o, x);
+        if (!(o = put_f64(o, buf + 440, x))) return false;
         *o++ = ',';
-        o = put_f64(o, y);
+        if (!(o = put_f64(o, buf + 880, y))) return false;
         *o++ = ',';
         (*pref)[j].assign(buf, o);
     }
+    return true;
 }
 
-// rows [r0, r1) -> "(x,y,freq) (x,y,freq) ...\n" (oligocgr.rs:88-101)
-void format_cgr_rows(const void *rows, bool norm, uint64_t r0, uint64_t r1, uint32_t dim, const std::vector<std::string> &pref,
-                     std::vector<char> *out) {
+// rows [r0, r1) -> "(x,y,freq) (x,y,freq) ...\n" (oligocgr.rs:88-101); false when a value's text exceeds its bound
+bool format_cgr_rows(const void *rows, bool norm, uint64_t r0, uint64_t r1, uint32_t dim, const std::vector<std::string> &pref,
+                     Text *out) {
+    const size_t vmax = norm ? kCgrFreqChars : kCgrCountChars;
     size_t plen = 0;
     for (auto &p : pref) plen += p.size();
-    out->resize((size_t)(r1 - r0) * (plen + (size_t)dim * 420) + 16);
+    out->resize((size_t)(r1 - r0) * (plen + (size_t)dim * (vmax + 2)));
     char *o = out->data();
     for (uint64_t i = r0; i < r1; ++i) {
         for (uint32_t j = 0; j < dim; ++j) {
             memcpy(o, pref[j].data(), pref[j].size());
             o += pref[j].size();
-            if (norm) o = put_f64(o, ((const double *)rows)[i * dim + j]);
-            else o = put_f64(o, (double)((const uint32_t *)rows)[i * dim + j]);
+            if (norm) o = put_f64(o, o + vmax, ((const double *)rows)[i * dim + j]);
+            else o = put_f64(o, o + vmax, (double)((const uint32_t *)rows)[i * dim + j]);
+            if (!o) {
+                out->clear();
+                return false;
+            }
             *o++ = ')';
             *o++ = (j + 1 == dim) ? '\n' : ' ';
         }
     }
     out->resize((size_t)(o - out->data()));
+    return true;
 }
 
 }  // namespace
@@ -373,7 +400,8 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
     std::string header_line;
 
     std::vector<std::string> cgr_pref;
-    if (cgr) cgr_prefixes(h, o->k, dim, (double)cgr_vecsize, &cgr_pref);
+    if (cgr && !cgr_prefixes(h, o->k, dim, (double)cgr_vecsize, &cgr_pref))
+        return ktb_internal_fail(KTB_ERR_ARG, "CGR coordinate text exceeds its bound");
     if (o->header && !cgr) {  // get_header().join(delim) + "\n", oligo.rs:114-117
         std::vector<char> hb(dim * o->k);
         if (int rc = ktb_oligo_header(h, o->canonical, hb.data(), hb.size())) return rc;
@@ -439,14 +467,16 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
         } else {
             const uint32_t *counts = (const uint32_t *)s.h_out.p;
             const void *rows = s.h_out.p;
+            std::atomic<bool> text_ok{true};
             if (cgr)
-                format_parallel(s.n, nthreads, &s.parts, [&](uint64_t r0, uint64_t r1, std::vector<char> *part) {
-                    format_cgr_rows(rows, norm, r0, r1, (uint32_t)dim, cgr_pref, part);
+                format_parallel(s.n, nthreads, &s.parts, [&](uint64_t r0, uint64_t r1, Text *part) {
+                    if (!format_cgr_rows(rows, norm, r0, r1, (uint32_t)dim, cgr_pref, part)) text_ok = false;
                 });
             else
-                format_parallel(s.n, nthreads, &s.parts, [&](uint64_t r0, uint64_t r1, std::vector<char> *part) {
+                format_parallel(s.n, nthreads, &s.parts, [&](uint64_t r0, uint64_t r1, Text *part) {
                     format_counts_rows(counts, r0, r1, (uint32_t)dim, o->delim, part);
                 });
+            if (!text_ok) return ktb_internal_fail(KTB_ERR_IO, "CGR value text exceeds its bound");
             for (auto &part : s.parts) wr.submit(part.data(), part.size(), &s.ticket);
         }
         s.writing = true;

@@ -238,6 +238,46 @@ def comp_oligo_text(path: str | os.PathLike, k: int, canonical: bool = True, nor
     return body
 
 
+def _rust_f64(v: float) -> str:
+    """Rust's `{}` of an f64: the shortest digits that round-trip, never an exponent, no trailing ".0"."""
+    return np.format_float_positional(v, unique=True, trim="-")
+
+
+def cgr_points(k: int, vecsize: int) -> list[tuple[float, float]]:
+    """The fixed point of every canonical k-mer, in header(k, True) order (composition/src/oligocgr.rs:123-143,165-190):
+    the midpoint recurrence from (v/2, v/2) towards the corner of each base, A (0,0), T (v,0), G (v,v), C (0,v)."""
+    v = float(vecsize)
+    corner = {"A": (0.0, 0.0), "T": (v, 0.0), "G": (v, v), "C": (0.0, v)}
+    pts = []
+    for kmer in header(k, True):
+        x = y = v / 2.0
+        for b in kmer:
+            cx, cy = corner[b]
+            x, y = (cx + x) / 2.0, (cy + y) / 2.0
+        pts.append((x, y))
+    return pts
+
+
+def comp_cgr_text(path: str | os.PathLike, k: int, vecsize: int, norm: bool = True) -> bytes:
+    """What `kmertools comp cgr -i path -k k -v vecsize [-c]` writes (composition/src/oligocgr.rs:88-101,123-190):
+    one line per record, "(x,y,value)" per canonical k-mer joined by spaces; a frequency is `{}` of the f64 quotient,
+    a count `{}` of an integral f64."""
+    seqs = [s for _, s in read_fastx(path)]
+    rows, _ = vectorise_batch(*pack(seqs), k, True, 1 if norm else 0)
+    pref = ["(%s,%s," % (_rust_f64(x), _rust_f64(y)) for x, y in cgr_points(k, vecsize)]
+    d = len(pref)
+    zero = [p + "0) " for p in pref]
+    zero[-1] = zero[-1][:-1] + "\n"
+    lines = []
+    for row in rows:   # most cells of short records are 0: rebuild only the others
+        cells = list(zero)
+        for j in np.flatnonzero(row):
+            v = row[j]
+            cells[j] = pref[j] + (_rust_f64(v) if norm else str(int(v))) + (")\n" if j == d - 1 else ") ")
+        lines.append("".join(cells))
+    return "".join(lines).encode()
+
+
 # ----------------------------------------------------------------------------- feeder
 
 def read_fastx(path: str | os.PathLike) -> list[tuple[str, bytes]]:

@@ -144,23 +144,21 @@ def test_gzip_record_far_larger_than_its_file(tmp_path):
 
 
 def test_python_driver_and_many_batches(tmp_path):
-    """comp_oligo() through ctypes; enough records for several GPU batches (rows stay in input order)."""
+    """comp_oligo() through ctypes; enough records for four GPU batches (rows stay in input order), whole output."""
     from kmertools_b200 import io as kio
     rng = np.random.default_rng(2)
     fq = tmp_path / "big.fq"
-    n = 12_000
+    n = 3_000
     with open(fq, "wb") as fh:
         arr = np.frombuffer(b"ACGT", dtype=np.uint8)[rng.integers(0, 4, size=(n, 100))]
         for i in range(n):
             fh.write(b"@r\n" + arr[i].tobytes() + b"\n+\n" + b"I" * 100 + b"\n")
-    out = tmp_path / "o"
-    st = kio.comp_oligo(fq, out, k=7)          # 8192 cols * 9 B = 73.7 kB/row -> ~3600 rows per batch
+    out, want = tmp_path / "o", tmp_path / "want"
+    st = kio.comp_oligo(fq, out, k=7)          # 8192 cols * 9 B = 73.7 kB/row -> 910 rows per 64 MiB batch
     assert st["records"] == n and st["bases"] == n * 100 and st["launches"] >= 8
-    data = out.read_bytes()
-    assert len(data) == n * 8192 * 9
-    rows, _ = O.vectorise_batch(arr.reshape(-1).copy(), np.arange(n + 1, dtype=np.uint64) * 100, 7, True, 1)
-    for i in (0, 1, 3639, 3640, 3641, 3642, n // 2, n - 1):
-        assert data[i * 73728:(i + 1) * 73728] == O.format_rows(rows[i:i + 1], True), i
+    O.baseline_text(arr.reshape(-1).copy(), np.arange(n + 1, dtype=np.uint64) * 100, 7, path=str(want))
+    assert out.stat().st_size == n * 8192 * 9
+    assert out.read_bytes() == want.read_bytes()
 
 
 def test_comp_cgr_kmer_mode_golden(golden, tmp_path):
@@ -173,18 +171,10 @@ def test_comp_cgr_kmer_mode_golden(golden, tmp_path):
 
 
 def test_comp_cgr_normalised_values(golden, tmp_path):
-    """Normalised k-mer CGR: freq is Rust's `{}` of the f64 quotient = Python's repr (shortest round-trip)."""
+    """Normalised k-mer CGR: freq is Rust's `{}` of the f64 quotient (shortest round-trip digits, never an exponent)."""
     from kmertools_b200 import io as kio
     out = tmp_path / "o.cgr"
     kio.comp_cgr(golden / "reads.fa", out, k=4)
-    seqs = [s for _, s in O.read_fastx(golden / "reads.fa")]
-    rows, _ = O.vectorise_batch(*O.pack(seqs), 4, True, 1)
-    lines = out.read_text().splitlines()
-    assert len(lines) == 2
-    for ln, row in zip(lines, rows):
-        trip = [t.strip("()").split(",") for t in ln.split(" ")]
-        assert len(trip) == 136
-        assert trip[0][:2] == ["0.5", "0.5"]                 # AAAA -> (0.5, 0.5), oligocgr.rs:205-206
-        for (x, y, f), want in zip(trip, row):
-            w = repr(float(want))
-            assert f == (w[:-2] if w.endswith(".0") else w), (f, w)
+    want = O.comp_cgr_text(golden / "reads.fa", 4, 16)
+    assert want.count(b"\n") == 2 and want.startswith(b"(0.5,0.5,")     # AAAA -> (0.5, 0.5), oligocgr.rs:205-206
+    assert out.read_bytes() == want

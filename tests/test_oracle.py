@@ -108,6 +108,15 @@ def test_golden_header(golden):  # vec_batch_with_header_test / vec_mmap_with_he
     assert got == (golden / "expected_fa_header.kmers").read_bytes()
 
 
+def test_cgr_text_golden(golden):  # oligo_cgr_complete_unnorm_test, composition/src/oligocgr.rs:219-238
+    assert O.comp_cgr_text(golden / "reads.fq", 4, 16, norm=False) == (golden / "expected_reads.k4.cgr").read_bytes()
+    assert O.cgr_points(4, 16)[0] == (0.5, 0.5)   # AAAA, oligocgr.rs:205-206
+    # Rust's `{}` never switches to an exponent and drops a trailing ".0"
+    for v, want in ((0.0, "0"), (1.0, "1"), (8.5, "8.5"), (1 / 3, "0.3333333333333333"), (1e-7, "0.0000001"),
+                    (1 / 16777219, "0.000000059604634117251494"), (123456.0, "123456")):
+        assert O._rust_f64(v) == want
+
+
 def test_python_binding_golden(golden):  # tests/test_oligo.py:8-25
     seqs = [s for _, s in O.read_fastx(golden / "reads.fq")]
     bases, offsets = O.pack(seqs)
