@@ -12,11 +12,19 @@
 
 #include <algorithm>
 #include <chrono>
+#include <climits>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
 #include <string>
 #include <vector>
+
+// The module declares the kernels' extern __shared__ arrays in the order the kernels are first instantiated, and a
+// kernel's dynamic shared memory starts at the strictest alignment declared up to its own array.  Instantiating these
+// two first keeps the histograms of seq_kernel and short_kernel 16 bytes after their static variables (not 128, as
+// behind long_kernel's and count_kernel's arrays) whatever order the launchers below are written in.
+template __global__ void ktb::seq_kernel<ktb::OUT_U32, 3, false>(ktb::SeqParams);
+template __global__ void ktb::short_kernel<ktb::OUT_U32, false>(ktb::ShortParams);
 
 void ktb_internal_register_host(void *p, size_t bytes);   // multi.cu: registry of page-locked blocks
 void ktb_internal_free_host(void *p);
@@ -55,6 +63,12 @@ uint64_t rev_comp(uint64_t x, int k) {  // kmer/src/kmer.rs:43-52
 struct DevBuf {
     void *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() {
+        if (p) cudaFree(p);
+    }
     int ensure(size_t bytes) {
         if (bytes <= cap) return KTB_OK;
         if (p) cudaFree(p);
@@ -73,18 +87,13 @@ struct DevBuf {
         cap = want;
         return KTB_OK;
     }
-    void release() {
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
-    }
 };
 
 constexpr int NBUF = 3;
 
 struct ChunkSet {
     cudaStream_t stream = nullptr;
-    cudaEvent_t ev[6] = {};  // h2d start/end, kernel end, d2h end  (+2 spare)
+    cudaEvent_t ev[5] = {};  // h2d start/end, kernel end, d2h end, kernel start
     DevBuf bases, offsets, out, totals;
     bool busy = false;
 };
@@ -170,6 +179,43 @@ int set_smem(K kern, size_t bytes) {
     return KTB_OK;
 }
 
+// Grid of a launch: the CTAs of `kern` that fit the GPU at once (at most `max_per_sm` per SM), no more than `items`,
+// and at least one.
+template <typename K>
+int fit_grid(const ktb_oligo *h, K kern, int threads, size_t smem, uint64_t items, unsigned *grid,
+             int max_per_sm = INT_MAX) {
+    int per_sm = 1;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+    per_sm = std::max(1, std::min(per_sm, max_per_sm));
+    *grid = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)h->sm_count * per_sm, items));
+    return KTB_OK;
+}
+
+// Checks the launches just enqueued and counts them in the stats of the call.
+int launched(ktb_oligo *h, int count = 1) {
+    CU(cudaGetLastError());
+    h->stats.launches += count;
+    return KTB_OK;
+}
+
+// Work items per trip to the (same-address) work counter: one atomic per 150-base read capped the GPU at ~330 M
+// reads/s, so short sequences take several; long sequences keep one item per trip for the tail.
+uint32_t grab(const ktb_oligo *h, uint64_t mean_len) {
+    return h->seq_grab > 0 ? (uint32_t)h->seq_grab
+                           : (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(16, 4096 / std::max<uint64_t>(mean_len, 1)));
+}
+
+// The batch of one call: device inputs and outputs, the row width and the caller's stream.
+struct Batch {
+    const uint8_t *bases;
+    const uint64_t *offsets;
+    uint64_t n, total_bases, dim;
+    int canonical, norm_mode;
+    void *out;
+    uint64_t *totals;
+    cudaStream_t st;
+};
+
 struct ShortCfg {
     bool ok = false;
     uint32_t words = 0, max_len = 0;
@@ -189,24 +235,31 @@ ShortCfg short_config(const ktb_oligo *h, uint64_t dim) {
 }
 
 template <int OUT>
-int launch_short(ktb_oligo *h, const ShortParams &p, const ShortCfg &c, cudaStream_t st) {
+int launch_short(ktb_oligo *h, const Batch &b, const ShortCfg &c) {
+    ShortParams p{};
+    p.ngroups = (b.n + SHORT_G - 1) / SHORT_G;
+    if (int rc = h->ws_list.ensure(p.ngroups * 4)) return rc;
+    p.bases = b.bases; p.offsets = b.offsets; p.n = b.n;
+    p.total_bases = b.total_bases;
+    p.out = b.out; p.totals = b.totals;
+    p.tab = b.canonical ? h->d_short_tab_canon : h->d_short_tab_raw;
+    p.counter = h->d_counters + 0;
+    p.reject_list = (uint32_t *)h->ws_list.p;
+    p.reject_count = h->d_counters + 2;
+    p.k = h->k; p.ncodes = (uint32_t)h->ncodes; p.dim = (uint32_t)b.dim; p.words = c.words;
+    p.words_recip = c.words > 1 ? (uint32_t)(0xFFFFFFFFu / c.words + 1u) : 0u;
+    p.max_len = c.max_len;
+    p.norm_mode = b.norm_mode; p.canonical = b.canonical;
     auto kern = (p.norm_mode != NORM_COUNTS) ? short_kernel<OUT, true> : short_kernel<OUT, false>;
     if (int rc = set_smem(kern, c.smem)) return rc;
-    int per_sm = 1;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, SHORT_WARPS * 32, c.smem));
-    if (per_sm < 1) per_sm = 1;
-    uint64_t grid = (uint64_t)h->sm_count * per_sm;
-    const uint64_t need = (p.ngroups + SHORT_WARPS - 1) / SHORT_WARPS;
-    if (grid > need) grid = need;
-    if (grid < 1) grid = 1;
-    kern<<<(unsigned)grid, SHORT_WARPS * 32, c.smem, st>>>(p);
-    CU(cudaGetLastError());
-    h->stats.launches++;
-    return KTB_OK;
+    unsigned grid;
+    if (int rc = fit_grid(h, kern, SHORT_WARPS * 32, c.smem, (p.ngroups + SHORT_WARPS - 1) / SHORT_WARPS, &grid)) return rc;
+    kern<<<grid, SHORT_WARPS * 32, c.smem, b.st>>>(p);
+    return launched(h);
 }
 
 template <int OUT>
-int launch_seq(ktb_oligo *h, const SeqParams &p, int hist_mode, cudaStream_t st) {
+int launch_seq(ktb_oligo *h, SeqParams p, int hist_mode, cudaStream_t st) {
     const size_t smem = (hist_mode == 5) ? ((((size_t)p.hist_entries + 3) & ~(size_t)3) * 4 + (size_t)p.even_words * 5 + 16)
                         : (hist_mode == 7) ? ((((size_t)p.hist_entries + 3) & ~(size_t)3) * 4 + (size_t)p.even_words * 6 + 16)
                                          : (size_t)p.hist_entries * 4;
@@ -231,7 +284,6 @@ int launch_seq(ktb_oligo *h, const SeqParams &p, int hist_mode, cudaStream_t st)
         }
     }
     if (int rc = set_smem(kern, smem)) return rc;
-    int per_sm = 1;
     // measured (bench.py --seq-threads): 10 kbp reads with a <= 16 KB histogram run 20 % faster with 4 warps
     // per CTA (less barrier / priming overhead, occupancy is not the limit); long contigs and the big
     // histograms want 8 warps.
@@ -241,23 +293,13 @@ int launch_seq(ktb_oligo *h, const SeqParams &p, int hist_mode, cudaStream_t st)
     int threads = h->seq_threads > 0 ? h->seq_threads : auto_threads;
     if (hist_mode == 5 && threads > 256) threads = 256;
     if (hist_mode != 2 && hist_mode != 5 && hist_mode != 7 && threads > KTB_SEQ_MAXTHREADS) threads = KTB_SEQ_MAXTHREADS;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
-    if (per_sm < 1) per_sm = 1;
-    uint64_t grid = (uint64_t)h->sm_count * per_sm;
     const uint64_t nitems = ((p.n + p.group_size - 1) / p.group_size) * p.group_size;   // one sequence per item
-    if (grid > nitems) grid = nitems;
-    if (grid < 1) grid = 1;
-    // short sequences: several work items per trip to the (same-address) work counter — one atomic per
-    // 150-base read capped the GPU at ~330 M reads/s; long sequences keep one item per trip for the tail
-    SeqParams q = p;
-    q.grab = h->seq_grab > 0 ? (uint32_t)h->seq_grab
-                             : (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(16, 4096 / std::max<uint64_t>(mean_len, 1)));
-    kern<<<(unsigned)grid, threads, smem, st>>>(q);
-    CU(cudaGetLastError());
-    h->stats.launches++;
-    return KTB_OK;
+    unsigned grid;
+    if (int rc = fit_grid(h, kern, threads, smem, nitems, &grid)) return rc;
+    p.grab = grab(h, mean_len);
+    kern<<<grid, threads, smem, st>>>(p);
+    return launched(h);
 }
-
 
 // Splits the (bin word, rank) pairs of a row into groups of 32 whose source banks (word % 32) are all distinct and
 // whose destination banks (rank % 32) are all distinct, so that a warp moves a group between two shared-memory
@@ -319,12 +361,31 @@ std::vector<uint32_t> conflict_free_groups(const std::vector<uint32_t> &word_of_
     return order;
 }
 
+// long_kernel over the groups on `list` (every group when it is null) in `mode`.
 template <int OUT>
-int launch_long(ktb_oligo *h, const LongParams &p, int mode, cudaStream_t st) {
+int launch_long(ktb_oligo *h, const Batch &b, int mode, const uint32_t *list, unsigned long long *list_count) {
     if constexpr (OUT == OUT_F64) {
-        (void)h; (void)p; (void)mode; (void)st;
+        (void)h; (void)b; (void)mode; (void)list; (void)list_count;
         return fail(KTB_ERR_ARG, "long_kernel has no f64 instance");
     } else {
+        LongParams p{};
+        p.bases = b.bases; p.offsets = b.offsets; p.n = b.n; p.total_bases = b.total_bases;
+        p.out = b.out; p.totals = b.totals;
+        p.counter = h->d_counters + 1;
+        p.list = list; p.list_count = list_count;
+        p.group_shift = 4;   // SHORT_G
+        static_assert(SHORT_G == 16, "group_shift");
+        p.k = h->k; p.dim = (uint32_t)b.dim;
+        p.norm_mode = b.norm_mode; p.canonical = b.canonical;
+        if (mode == MODE_K8) {
+            // the packed 16-bit rank-space histogram of seq_kernel mode 5; sequences it cannot count go on out_list
+            p.even_tab = h->d_even_tab; p.even_words = h->even_words;
+            p.out_list = (uint32_t *)h->ws_list2.p; p.out_count = h->d_counters + 3;
+            p.hist_words = (uint32_t)(h->dim_canon / 2);
+        } else {
+            p.sched = mode == MODE_K7 ? h->d_k7_sched : h->d_fwd_sched;
+            p.hist_words = mode == MODE_K7 ? K7_BINS : (uint32_t)h->ncodes + 4;
+        }
         const bool nrm = p.norm_mode != NORM_COUNTS;
         const uint64_t mean_len = p.total_bases / std::max<uint64_t>(p.n, 1);
         // 4 warps per CTA for reads of a few steps per warp (10 kbp = 20 steps: 5 per warp, balanced, half the per-warp
@@ -355,21 +416,15 @@ int launch_long(ktb_oligo *h, const LongParams &p, int mode, cudaStream_t st) {
                 if (p.k == 5) { kern = nrm ? long_kernel<OUT, true, MODE_FWD, 8, 5, 3> : long_kernel<OUT, false, MODE_FWD, 8, 5, 3>; rs = 3; }
             }
         }
-        LongParams q = p;
-        if (rs) q.hist_words = (((uint32_t)1 << (2 * p.k)) << rs) + (1u << rs);   // + the always-zero replicas (rc slot of palindromes)
-        const size_t smem = mode == MODE_K8 ? ((((size_t)q.hist_words + 3) & ~(size_t)3) * 4 + (size_t)p.even_words * 5 + 16)
-                                            : ((((size_t)q.hist_words + 31) & ~(size_t)31) + p.dim) * 4;
+        if (rs) p.hist_words = (((uint32_t)1 << (2 * p.k)) << rs) + (1u << rs);   // + the always-zero replicas (rc slot of palindromes)
+        const size_t smem = mode == MODE_K8 ? ((((size_t)p.hist_words + 3) & ~(size_t)3) * 4 + (size_t)p.even_words * 5 + 16)
+                                            : ((((size_t)p.hist_words + 31) & ~(size_t)31) + p.dim) * 4;
         if (int rc = set_smem(kern, smem)) return rc;
-        int per_sm = 1;
         const int threads = nw * 32;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
-        if (per_sm < 1) per_sm = 1;
-        uint64_t grid = (uint64_t)h->sm_count * per_sm;
         const uint64_t nitems = ((p.n + SHORT_G - 1) / SHORT_G) * SHORT_G;
-        if (grid > nitems) grid = nitems;
-        if (grid < 1) grid = 1;
-        q.grab = h->seq_grab > 0 ? (uint32_t)h->seq_grab
-                                 : (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(16, 4096 / std::max<uint64_t>(mean_len, 1)));
+        unsigned grid;
+        if (int rc = fit_grid(h, kern, threads, smem, nitems, &grid)) return rc;
+        p.grab = grab(h, mean_len);
         if (rs && h->longest_first && p.n > grid && p.n < (1ull << 32)) {
             // more contigs than CTAs: the queue order decides how long the last CTA runs alone (see order_count_kernel)
             if (int rc = h->ws_order.ensure(p.n * 4 + 129 * 8 + 64)) return rc;
@@ -377,371 +432,327 @@ int launch_long(ktb_oligo *h, const LongParams &p, int mode, cudaStream_t st) {
             op.offsets = p.offsets; op.n = p.n; op.list = p.list; op.list_count = p.list_count; op.group_shift = p.group_shift;
             op.cls = (unsigned long long *)h->ws_order.p;
             op.order = (uint32_t *)((uint8_t *)h->ws_order.p + 129 * 8 + 56);
-            CU(cudaMemsetAsync(op.cls, 0, 129 * 8, st));
+            CU(cudaMemsetAsync(op.cls, 0, 129 * 8, b.st));
             const unsigned ogrid = (unsigned)std::min<uint64_t>((nitems + 255) / 256, (uint64_t)h->sm_count * 4);
-            order_count_kernel<<<ogrid, 256, 0, st>>>(op);
-            order_scatter_kernel<<<ogrid, 256, 0, st>>>(op);
-            CU(cudaGetLastError());
-            h->stats.launches += 2;
-            q.list = op.order; q.list_count = op.cls + 128; q.group_shift = 0;
-            q.grab = 1;
+            order_count_kernel<<<ogrid, 256, 0, b.st>>>(op);
+            order_scatter_kernel<<<ogrid, 256, 0, b.st>>>(op);
+            if (int rc = launched(h, 2)) return rc;
+            p.list = op.order; p.list_count = op.cls + 128; p.group_shift = 0;
+            p.grab = 1;
         }
-        kern<<<(unsigned)grid, threads, smem, st>>>(q);
-        CU(cudaGetLastError());
-        h->stats.launches++;
-        return KTB_OK;
+        kern<<<grid, threads, smem, b.st>>>(p);
+        return launched(h);
     }
 }
 
+// u32 counts of rows [i0, i0 + cnt) -> normalised output rows (the counts are the u32 output itself)
 template <int OUT>
-int run_device(ktb_oligo *h, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
-               uint64_t total_bases, int canonical, int norm_mode, void *d_out, uint64_t *d_totals,
-               cudaStream_t st) {
-    const uint64_t dim = canonical ? h->dim_canon : h->ncodes;
+int launch_finalize(ktb_oligo *h, const Batch &b, const uint32_t *counts, const unsigned long long *tot, uint64_t i0,
+                    uint64_t cnt, cudaStream_t st) {
+    if (OUT == OUT_U32) return KTB_OK;
     const size_t esize = (OUT == OUT_F64) ? 8 : 4;
-    if (n == 0) return KTB_OK;
+    const unsigned grid = (unsigned)std::min<uint64_t>((cnt * b.dim + 255) / 256, (uint64_t)h->sm_count * 16);
+    finalize_kernel<OUT><<<grid, 256, 0, st>>>(counts, tot + i0, (uint8_t *)b.out + i0 * b.dim * esize, nullptr, cnt,
+                                               b.dim, b.norm_mode, b.canonical);
+    return launched(h);
+}
 
-    // which histogram lives in shared memory?
-    const size_t smem_limit = h->smem_optin - 1024;
-    int hist_mode = -1;
-    uint64_t hist_entries = 0;
-    if (h->force_path != 1) {
-        if (!canonical) {
-            if (h->ncodes * 4 <= smem_limit) { hist_mode = 0; hist_entries = h->ncodes; }
-        } else if ((h->k & 1) && h->ncodes * 4 > 32 * 1024 && h->ncodes * 2 <= 64 * 1024 && h->dense_odd) {
-            hist_mode = 4; hist_entries = (h->mb_entries + 3) & ~3ull;   // k = 7: dense middle-base index, 32 KB + skew
-        } else if (h->ncodes * 4 <= 64 * 1024) {
-            hist_mode = 1; hist_entries = h->ncodes;
-        } else if (h->d_even_tab && h->even_rank && h->packed16 && (h->dim_canon % 8) == 0 &&
-                   h->dim_canon * 2 + h->even_words * 6 + 64 <= smem_limit / 2) {
-            hist_mode = 5; hist_entries = h->dim_canon / 2;   // k = 8: packed 16-bit rank space, 2 CTAs/SM
-        } else if (h->d_even_tab && h->even_rank && h->dim_canon * 4 + h->even_words * 6 + 64 <= smem_limit) {
-            hist_mode = 7; hist_entries = h->dim_canon;      // k = 8: rank from shared-memory bitmap tables
-        } else if (h->dim_canon * 4 <= smem_limit) {
-            hist_mode = 2; hist_entries = h->dim_canon;
-        }
+// Bucket-then-count (bucket_kernels.cuh): partition the k-mer codes of every tile by their high bits, then count each
+// (sequence, code segment) in shared memory and write its part of the row once.  Writes the totals itself.
+template <int OUT>
+int launch_bucket(ktb_oligo *h, const Batch &b, unsigned long long *tot, uint64_t nseg) {
+    const uint32_t log2_seg = (uint32_t)h->bucket_log2_seg;
+    const uint64_t n = b.n, total_bases = b.total_bases;
+    const cudaStream_t st = b.st;
+    const uint64_t tile_bases = (uint64_t)BK_TILE_CHUNKS * 16;
+    const uint64_t ntiles_bound = total_bases / tile_bases + 2 * n + 2;
+    if (ntiles_bound >= (1ull << 31)) return fail(KTB_ERR_ARG, "batch too large for the bucket path");
+    if (int rc = h->ws_tiles.ensure((n + 1) * 4 + 64 + ntiles_bound * sizeof(TileInfo))) return rc;
+    if (int rc = h->ws_pool.ensure(ntiles_bound * (uint64_t)BK_TILE_CAP * 2 + 64)) return rc;
+    if (int rc = h->ws_runs.ensure(ntiles_bound * nseg * 4)) return rc;
+    uint32_t *tile_prefix = (uint32_t *)h->ws_tiles.p;
+    TileInfo *tiles = (TileInfo *)((uint8_t *)h->ws_tiles.p + (((n + 1) * 4 + 63) & ~(uint64_t)63));
+    tile_prefix_kernel<<<1, 1024, 0, st>>>(b.offsets, n, (uint32_t)h->k, tile_prefix);
+    tile_info_kernel<<<(unsigned)std::min<uint64_t>((ntiles_bound + 255) / 256, (uint64_t)h->sm_count * 8), 256, 0, st>>>(
+        b.offsets, n, tile_prefix, tiles);
+    if (int rc = launched(h, 2)) return rc;
+    BucketParams bp{};
+    bp.bases = b.bases; bp.n = n; bp.total_bases = total_bases;
+    bp.tile_prefix = tile_prefix; bp.tiles = tiles;
+    bp.pool = (uint16_t *)h->ws_pool.p; bp.runs = (uint32_t *)h->ws_runs.p; bp.totals = tot;
+    bp.k = (uint32_t)h->k; bp.nseg = (uint32_t)nseg; bp.log2_seg = log2_seg;
+    CountParams cp{};
+    cp.tile_prefix = tile_prefix; cp.pool = bp.pool; cp.runs = bp.runs; cp.totals_in = tot;
+    cp.totals_out = b.totals; cp.out = b.out;
+    cp.rank_tab = h->d_wave_tab; cp.tab_words = h->wave_tab_words;
+    cp.n = n; cp.dim = b.dim; cp.nseg = (uint32_t)nseg; cp.log2_seg = log2_seg;
+    cp.norm_mode = b.norm_mode; cp.canonical = b.canonical;
+#ifdef KTB_COUNT_PROBE
+    if (const char *e = getenv("KTB_COUNT_PROBE")) cp.probe = (uint32_t)atoi(e);
+#endif
+    void (*bkern)(const BucketParams) = b.canonical ? bucket_kernel<true> : bucket_kernel<false>;
+    if (b.canonical && log2_seg == 14) {   // the two shapes BASELINE.json names get their constants at compile time
+        if (h->k == 10) bkern = bucket_kernel<true, 10, 14>;
+        else if (h->k == 9) bkern = bucket_kernel<true, 9, 14>;
     }
+    const bool nrm = b.norm_mode != NORM_COUNTS;
+    void (*ckern)(const CountParams) =
+        b.canonical ? (nrm ? count_kernel<OUT, true, true> : count_kernel<OUT, false, true>)
+                    : (nrm ? count_kernel<OUT, true, false> : count_kernel<OUT, false, false>);
+    // histogram memory: 64 KB either way — one buffer of 2^14 bins (segments with at most half as many columns
+    // alternate between its halves) or two buffers of 2^13
+    const size_t S = (size_t)1 << log2_seg;
+    cp.hist_words = (uint32_t)(log2_seg < 14 ? 2 * S : S);
+    if (h->bucket_hist_kb == 96) cp.hist_words = 24576;   // segments of up to 12,288 columns alternate between two halves
+    const size_t csmem = ((size_t)cp.hist_words + 2 * (S / 32)) * 4;
+    if (int rc = set_smem(ckern, csmem)) return rc;
+    // Waves (option "bucket_waves", default 1): bucket_kernel is bound by the integer pipe, count_kernel by latency and
+    // the row writes, so the batch can be cut into waves with bucket_kernel(w+1) on one helper stream and
+    // count_kernel(w) on the other, sharing the SMs.  Measured on config 5ii (profiles/r2_sweeps.txt, batch r2i):
+    // 1.57 ms with one wave, 1.63 - 1.77 ms with 2 - 16 — the two kernels take each other's shared memory and
+    // registers and both lose more occupancy than the overlap returns.  Kept as an option.
+    const uint64_t nchunks = (n + CK_SEQ_CHUNK - 1) / CK_SEQ_CHUNK;
+    const uint64_t nwaves = std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)std::max(1, h->bucket_waves), nchunks / 16));
+    if (int rc = h->ws_wavectr.ensure(nwaves * sizeof(unsigned long long))) return rc;
+    CU(cudaMemsetAsync(h->ws_wavectr.p, 0, nwaves * sizeof(unsigned long long), st));
+    CU(cudaEventRecord(h->aux_ev[2], st));
+    cudaStream_t sb = nwaves > 1 ? h->aux[0] : st, sc = nwaves > 1 ? h->aux[1] : st;
+    if (nwaves > 1) {
+        CU(cudaStreamWaitEvent(sb, h->aux_ev[2], 0));
+        CU(cudaStreamWaitEvent(sc, h->aux_ev[2], 0));
+    }
+    const int b_ctas = nwaves > 1 ? h->bucket_wave_ctas : INT_MAX;   // beside count_kernel when the waves overlap
+    for (uint64_t w = 0; w < nwaves; ++w) {
+        const uint64_t c_lo = nchunks * w / nwaves, c_hi = nchunks * (w + 1) / nwaves;
+        bp.seq_lo = std::min(n, c_lo * CK_SEQ_CHUNK); bp.seq_hi = std::min(n, c_hi * CK_SEQ_CHUNK);
+        const uint64_t wave_tiles = (bp.seq_hi - bp.seq_lo) * 2 + (total_bases / tile_bases) / nwaves + 2;   // grid bound only
+        unsigned grid;
+        if (int rc = fit_grid(h, bkern, BK_WARPS * 32, 0, wave_tiles, &grid, b_ctas)) return rc;
+        bkern<<<grid, BK_WARPS * 32, 0, sb>>>(bp);
+        if (int rc = launched(h)) return rc;
+        if (nwaves > 1) {
+            if (h->wave_ev.size() <= w) {
+                cudaEvent_t e = nullptr;
+                CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+                h->wave_ev.push_back(e);
+            }
+            CU(cudaEventRecord(h->wave_ev[w], sb));
+            CU(cudaStreamWaitEvent(sc, h->wave_ev[w], 0));
+        }
+        cp.chunk_lo = c_lo; cp.chunk_hi = c_hi;
+        cp.counter = (unsigned long long *)h->ws_wavectr.p + w;
+        if (int rc = fit_grid(h, ckern, CK_THREADS, csmem, (c_hi - c_lo) * nseg, &grid)) return rc;
+        ckern<<<grid, CK_THREADS, csmem, sc>>>(cp);
+        if (int rc = launched(h)) return rc;
+    }
+    if (nwaves > 1) {
+        CU(cudaEventRecord(h->aux_ev[0], sb));
+        CU(cudaEventRecord(h->aux_ev[1], sc));
+        CU(cudaStreamWaitEvent(st, h->aux_ev[0], 0));
+        CU(cudaStreamWaitEvent(st, h->aux_ev[1], 0));
+    }
+    return KTB_OK;
+}
 
+// The flat-decomposition fallback (testing, force_path 1): the whole batch at once.
+template <int OUT>
+int launch_flat(ktb_oligo *h, const Batch &b, unsigned long long *tot) {
+    const uint64_t row_bytes = b.dim * 4;
+    uint32_t *counts = (uint32_t *)b.out;
+    if (OUT == OUT_F64) {
+        if (int rc = h->ws_counts.ensure(b.n * row_bytes)) return rc;
+        counts = (uint32_t *)h->ws_counts.p;
+    }
+    CU(cudaMemsetAsync(counts, 0, b.n * row_bytes, b.st));
+    if (b.total_bases > 0) {
+        FlatParams fp{};
+        fp.bases = b.bases; fp.offsets = b.offsets; fp.n = b.n; fp.total_bases = b.total_bases;
+        fp.counts = counts; fp.totals = tot;
+        fp.rank_full = b.canonical ? h->d_rank_full : nullptr;
+        fp.dim = b.dim; fp.k = h->k;
+        const uint64_t nchunks = (b.total_bases + FLAT_CHUNK - 1) / FLAT_CHUNK;
+        const unsigned grid = (unsigned)std::min<uint64_t>((nchunks + 255) / 256, (uint64_t)h->sm_count * 32);
+        flat_kernel<<<grid, 256, 0, b.st>>>(fp);
+        if (int rc = launched(h)) return rc;
+    }
+    return launch_finalize<OUT>(h, b, counts, tot, 0, b.n, b.st);
+}
+
+// One persistent cooperative launch: the wave loop (zero next rows / count / normalise previous rows) runs on the
+// device with a grid barrier per wave instead of three launches per wave.
+template <int OUT>
+int launch_wave_kernel(ktb_oligo *h, const Batch &b, unsigned long long *tot) {
+    WaveParams wp{};
+    wp.bases = b.bases; wp.offsets = b.offsets; wp.n = b.n; wp.total_bases = b.total_bases;
+    wp.rows = (uint32_t *)b.out; wp.totals = tot;
+    wp.rank_full = b.canonical ? h->d_rank_full : nullptr;
+    wp.dim = b.dim; wp.k = (uint32_t)h->k; wp.norm_mode = b.norm_mode; wp.canonical = b.canonical;
+    // a wave is a third of the budget: the wave being counted and the next one (zeroed at the end of the
+    // iteration) are live together, the rest is slack for lines on their way out (32 MB waves measured best)
+    wp.wave_rows = std::max<uint64_t>(1, std::min<uint64_t>(256, (uint64_t)h->wave_budget_bytes / 3 / (b.dim * 4)));
+    const int rank_mode = !b.canonical ? 0 : (h->d_wave_tab && h->wave_tab_in_smem && h->wave_smem_rank) ? 2 : 1;
+    wp.rank_tab = h->d_wave_tab; wp.tab_words = h->wave_tab_words;
+    constexpr bool F32 = (OUT == OUT_F32);
+    const void *kern = rank_mode == 0 ? (const void *)wave_kernel<0, F32>
+                     : rank_mode == 1 ? (const void *)wave_kernel<1, F32> : (const void *)wave_kernel<2, F32>;
+    const int threads = 1024;
+    const size_t smem = rank_mode == 2 ? ((size_t)h->wave_tab_words * 6 + 16) : 0;
+    if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    int per_sm = 1;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
+    if (per_sm < 1) return fail(KTB_ERR_CUDA, "wave_kernel does not fit on an SM (%zu bytes of shared memory)", smem);
+    const unsigned grid = (unsigned)h->sm_count;   // one CTA per SM: the RED rate of an SM does not grow with occupancy
+    void *args[] = {&wp};
+    CU(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(threads), args, smem, b.st));
+    h->stats.launches++;
+    return KTB_OK;
+}
+
+// Waves of rows that fit L2 together: zero the wave's rows, let every CTA of the GPU work on that wave (sequences
+// are split into tiles), normalise it, move on.  The REDs then hit rows that are still L2-resident and each row goes
+// to HBM once; one big memset + one launch over the whole batch made every RED a 32-byte DRAM read-modify-write
+// (measured 8.5 ms vs the 0.7 ms roofline).
+template <int OUT>
+int launch_wave_loop(ktb_oligo *h, const Batch &b, unsigned long long *tot) {
+    const uint64_t n = b.n, dim = b.dim, row_bytes = dim * 4;
+    SeqParams qp{};
+    qp.bases = b.bases; qp.offsets = b.offsets; qp.n = n; qp.total_bases = b.total_bases;
+    qp.rank_full = b.canonical ? h->d_rank_full : nullptr;
+    qp.counter = h->d_counters + 1;
+    qp.k = h->k; qp.dim = (uint32_t)dim; qp.hist_entries = 0;
+    qp.norm_mode = b.norm_mode; qp.canonical = b.canonical;
+    qp.list = nullptr; qp.list_count = nullptr; qp.group_size = 1;
+    qp.gtotals = tot;
+    auto kern = seq_kernel<OUT_U32, 3, false>;
+    const int threads = h->seq_threads > 0 ? h->seq_threads : 128;
+    // two waves in flight (one per helper stream), each half of the L2 budget
+    const uint64_t wave = std::max<uint64_t>(1, std::min<uint64_t>(n, (uint64_t)h->global_wave_bytes / 2 / row_bytes));
+    if (OUT == OUT_F64)
+        if (int rc = h->ws_counts.ensure(2 * wave * row_bytes)) return rc;
+    // a work item = (sequence, tile).  A wave is small (rows must fit L2), so parallelism has to come from
+    // splitting sequences finely: about `global_steps_per_warp` steps of 512 bases per warp (the first
+    // version used 4 and ran 5 warps per SM; one step per warp fills the machine).
+    const uint64_t mean_steps = (b.total_bases / std::max<uint64_t>(n, 1)) / 512 + 1;
+    const uint64_t per_item = (uint64_t)std::max(1, h->global_steps_per_warp) * (threads / 32);
+    const uint32_t tiles = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(4096, mean_steps / per_item));
+    CU(cudaEventRecord(h->aux_ev[2], b.st));
+    uint64_t w = 0;
+    for (uint64_t i0 = 0; i0 < n; i0 += wave, ++w) {
+        const int x = (int)(w & 1);
+        cudaStream_t sx = h->aux[x];
+        if (w < 2) CU(cudaStreamWaitEvent(sx, h->aux_ev[2], 0));
+        const uint64_t cnt = std::min(wave, n - i0);
+        uint32_t *counts = (OUT == OUT_F64) ? (uint32_t *)h->ws_counts.p + (uint64_t)x * wave * dim
+                                            : (uint32_t *)b.out + i0 * dim;
+        CU(cudaMemsetAsync(counts, 0, cnt * row_bytes, sx));
+        CU(cudaMemsetAsync(h->d_counters + 4 + x, 0, sizeof(unsigned long long), sx));
+        qp.counter = h->d_counters + 4 + x;
+        qp.gcounts = counts; qp.seq_base = i0; qp.seq_count = cnt; qp.tiles = tiles;
+        unsigned grid;
+        if (int rc = fit_grid(h, kern, threads, 0, cnt * tiles, &grid)) return rc;
+        kern<<<grid, threads, 0, sx>>>(qp);
+        if (int rc = launched(h)) return rc;
+        if (int rc = launch_finalize<OUT>(h, b, counts, tot, i0, cnt, sx)) return rc;
+    }
+    for (int x = 0; x < 2; ++x) {   // join the helper streams back into the caller's stream
+        CU(cudaEventRecord(h->aux_ev[x], h->aux[x]));
+        CU(cudaStreamWaitEvent(b.st, h->aux_ev[x], 0));
+    }
+    return KTB_OK;
+}
+
+// Which histogram of seq_kernel fits shared memory (its mode), and its entries; -1 when none does.
+int smem_hist_mode(const ktb_oligo *h, int canonical, uint64_t *entries) {
+    const size_t smem_limit = h->smem_optin - 1024;
+    if (h->force_path == 1) return -1;
+    if (!canonical) {
+        if (h->ncodes * 4 <= smem_limit) { *entries = h->ncodes; return 0; }
+    } else if ((h->k & 1) && h->ncodes * 4 > 32 * 1024 && h->ncodes * 2 <= 64 * 1024 && h->dense_odd) {
+        *entries = (h->mb_entries + 3) & ~3ull; return 4;   // k = 7: dense middle-base index, 32 KB + skew
+    } else if (h->ncodes * 4 <= 64 * 1024) {
+        *entries = h->ncodes; return 1;
+    } else if (h->d_even_tab && h->even_rank && h->packed16 && (h->dim_canon % 8) == 0 &&
+               h->dim_canon * 2 + h->even_words * 6 + 64 <= smem_limit / 2) {
+        *entries = h->dim_canon / 2; return 5;   // k = 8: packed 16-bit rank space, 2 CTAs/SM
+    } else if (h->d_even_tab && h->even_rank && h->dim_canon * 4 + h->even_words * 6 + 64 <= smem_limit) {
+        *entries = h->dim_canon; return 7;      // k = 8: rank from shared-memory bitmap tables
+    } else if (h->dim_canon * 4 <= smem_limit) {
+        *entries = h->dim_canon; return 2;
+    }
+    return -1;
+}
+
+template <int OUT>
+int run_device(ktb_oligo *h, const Batch &b) {
+    if (b.n == 0) return KTB_OK;
+    uint64_t hist_entries = 0;
+    const int hist_mode = smem_hist_mode(h, b.canonical, &hist_entries);
     if (hist_mode >= 0) {
-        CU(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(unsigned long long), st));
-        const ShortCfg sc = short_config(h, dim);
-        const uint64_t ngroups = (n + SHORT_G - 1) / SHORT_G;
-        if (sc.ok) {
-            if (int rc = h->ws_list.ensure(ngroups * 4)) return rc;
-            ShortParams sp{};
-            sp.bases = d_bases; sp.offsets = d_offsets; sp.n = n; sp.ngroups = ngroups;
-            sp.total_bases = total_bases;
-            sp.out = d_out; sp.totals = d_totals;
-            sp.tab = canonical ? h->d_short_tab_canon : h->d_short_tab_raw;
-            sp.counter = h->d_counters + 0;
-            sp.reject_list = (uint32_t *)h->ws_list.p;
-            sp.reject_count = h->d_counters + 2;
-            sp.k = h->k; sp.ncodes = (uint32_t)h->ncodes; sp.dim = (uint32_t)dim; sp.words = sc.words;
-            sp.words_recip = sc.words > 1 ? (uint32_t)(0xFFFFFFFFu / sc.words + 1u) : 0u;
-            sp.max_len = sc.max_len;
-            sp.norm_mode = norm_mode; sp.canonical = canonical;
-            if (int rc = launch_short<OUT>(h, sp, sc, st)) return rc;
-        }
+        CU(cudaMemsetAsync(h->d_counters, 0, 4 * sizeof(unsigned long long), b.st));
+        const ShortCfg sc = short_config(h, b.dim);
+        if (sc.ok)
+            if (int rc = launch_short<OUT>(h, b, sc)) return rc;
+        // the CTA-per-sequence kernels take the groups the short kernel rejected, or every group when it did not run
+        const uint32_t *list = sc.ok ? (const uint32_t *)h->ws_list.p : nullptr;
+        unsigned long long *list_count = sc.ok ? h->d_counters + 2 : nullptr;
         // second-generation CTA-per-sequence kernel (long_kernel.cuh) where it applies
-        const uint64_t mean_len = total_bases / std::max<uint64_t>(n, 1);
-        int long_mode = -1;
-        if (OUT != OUT_F64 && canonical && h->force_path != 3) {
-            if (h->k == 7 && h->k7_mid && h->d_k7_sched) long_mode = MODE_K7;
-            else if (h->d_fwd_sched && h->fwd_fold && (int64_t)mean_len >= h->fwd_min_len) long_mode = MODE_FWD;
-        }
-        if (long_mode >= 0) {
-            LongParams lp{};
-            lp.bases = d_bases; lp.offsets = d_offsets; lp.n = n; lp.total_bases = total_bases;
-            lp.out = d_out; lp.totals = d_totals;
-            lp.sched = long_mode == MODE_K7 ? h->d_k7_sched : h->d_fwd_sched;
-            lp.counter = h->d_counters + 1;
-            lp.list = sc.ok ? (const uint32_t *)h->ws_list.p : nullptr;
-            lp.list_count = sc.ok ? h->d_counters + 2 : nullptr;
-            lp.group_shift = 4;   // SHORT_G
-            static_assert(SHORT_G == 16, "group_shift");
-            lp.k = h->k; lp.dim = (uint32_t)dim;
-            lp.hist_words = long_mode == MODE_K7 ? K7_BINS : (uint32_t)h->ncodes + 4;
-            lp.norm_mode = norm_mode; lp.canonical = canonical;
-            return launch_long<OUT>(h, lp, long_mode, st);
-        }
+        const bool long_ok = OUT != OUT_F64 && b.canonical && h->force_path != 3;
+        const uint64_t mean_len = b.total_bases / std::max<uint64_t>(b.n, 1);
+        if (long_ok && h->k == 7 && h->k7_mid && h->d_k7_sched) return launch_long<OUT>(h, b, MODE_K7, list, list_count);
+        if (long_ok && h->d_fwd_sched && h->fwd_fold && (int64_t)mean_len >= h->fwd_min_len)
+            return launch_long<OUT>(h, b, MODE_FWD, list, list_count);
         SeqParams qp{};
-        qp.bases = d_bases; qp.offsets = d_offsets; qp.n = n; qp.total_bases = total_bases;
-        qp.out = d_out; qp.totals = d_totals;
+        qp.bases = b.bases; qp.offsets = b.offsets; qp.n = b.n; qp.total_bases = b.total_bases;
+        qp.out = b.out; qp.totals = b.totals;
         qp.rank_full = h->d_rank_full;
         qp.canon_of_rank = hist_mode == 4 ? h->d_mb_of_rank : h->d_canon_of_rank;
         qp.canon_perm = hist_mode == 4 ? h->d_mb_perm : h->d_canon_perm;
         qp.counter = h->d_counters + 1;
-        qp.k = h->k; qp.dim = (uint32_t)dim; qp.hist_entries = (uint32_t)hist_entries;
-        qp.norm_mode = norm_mode; qp.canonical = canonical;
-        qp.list = sc.ok ? (const uint32_t *)h->ws_list.p : nullptr;
-        qp.list_count = sc.ok ? h->d_counters + 2 : nullptr;
+        qp.k = h->k; qp.dim = (uint32_t)b.dim; qp.hist_entries = (uint32_t)hist_entries;
+        qp.norm_mode = b.norm_mode; qp.canonical = b.canonical;
+        qp.list = list; qp.list_count = list_count;
         qp.group_size = SHORT_G;
         qp.even_tab = h->d_even_tab; qp.even_words = h->even_words;
-        if (hist_mode == 5) {
-            // packed 16-bit counters: sequences with more than 65535 windows come back on out_list and are
-            // redone with 32-bit counters (mode 7) in a second launch
-            if (int rc = h->ws_list2.ensure(n * 4)) return rc;
-            qp.out_list = (uint32_t *)h->ws_list2.p; qp.out_count = h->d_counters + 3;
-            if (OUT != OUT_F64 && h->k8_long && h->k == 8 && canonical && h->force_path != 3) {
-                // same arithmetic inside long_kernel's loop (look-back lane, look-ahead across sequences)
-                LongParams lp{};
-                lp.bases = d_bases; lp.offsets = d_offsets; lp.n = n; lp.total_bases = total_bases;
-                lp.out = d_out; lp.totals = d_totals;
-                lp.even_tab = h->d_even_tab; lp.even_words = h->even_words;
-                lp.out_list = qp.out_list; lp.out_count = qp.out_count;
-                lp.counter = h->d_counters + 1;
-                lp.list = qp.list; lp.list_count = qp.list_count;
-                lp.group_shift = 4;   // SHORT_G
-                lp.k = h->k; lp.dim = (uint32_t)dim; lp.hist_words = (uint32_t)hist_entries;
-                lp.norm_mode = norm_mode; lp.canonical = canonical;
-                if (int rc = launch_long<OUT>(h, lp, MODE_K8, st)) return rc;
-            } else if (int rc = launch_seq<OUT>(h, qp, 5, st)) return rc;
-            SeqParams q2 = qp;
-            q2.hist_entries = (uint32_t)h->dim_canon;
-            q2.counter = h->d_counters + 0;   // unused by the short kernel for this k, zeroed above
-            q2.list = (const uint32_t *)h->ws_list2.p; q2.list_count = h->d_counters + 3; q2.group_size = 1;
-            return launch_seq<OUT>(h, q2, 7, st);
-        }
-        return launch_seq<OUT>(h, qp, hist_mode, st);
+        if (hist_mode != 5) return launch_seq<OUT>(h, qp, hist_mode, b.st);
+        // packed 16-bit counters: sequences with more than 65535 windows come back on out_list and are
+        // redone with 32-bit counters (mode 7) in a second launch
+        if (int rc = h->ws_list2.ensure(b.n * 4)) return rc;
+        qp.out_list = (uint32_t *)h->ws_list2.p; qp.out_count = h->d_counters + 3;
+        if (long_ok && h->k8_long && h->k == 8) {
+            // same arithmetic inside long_kernel's loop (look-back lane, look-ahead across sequences)
+            if (int rc = launch_long<OUT>(h, b, MODE_K8, list, list_count)) return rc;
+        } else if (int rc = launch_seq<OUT>(h, qp, 5, b.st)) return rc;
+        qp.hist_entries = (uint32_t)h->dim_canon;
+        qp.counter = h->d_counters + 0;   // unused by the short kernel for this k, zeroed above
+        qp.list = (const uint32_t *)h->ws_list2.p; qp.list_count = h->d_counters + 3; qp.group_size = 1;
+        return launch_seq<OUT>(h, qp, 7, b.st);
     }
 
-    // ---- global-atomic path: zeroed u32 rows in HBM/L2, RED atomics, finalize
-    if (int rc = h->ws_totals.ensure(n * 8)) return rc;
+    // ---- rows larger than shared memory: zeroed u32 rows in HBM/L2, RED atomics, finalize
+    if (int rc = h->ws_totals.ensure(b.n * 8)) return rc;
     unsigned long long *tot = (unsigned long long *)h->ws_totals.p;
-    CU(cudaMemsetAsync(tot, 0, n * 8, st));
-    const uint64_t row_bytes = dim * 4;
-    auto finalize = [&](const uint32_t *counts, uint64_t i0, uint64_t cnt) -> int {
-        if (OUT == OUT_U32) return KTB_OK;   // counts are already the output
-        const uint64_t nel = cnt * dim;
-        uint64_t grid = (nel + 255) / 256;
-        const uint64_t cap = (uint64_t)h->sm_count * 16;
-        if (grid > cap) grid = cap;
-        finalize_kernel<OUT><<<(unsigned)grid, 256, 0, st>>>(counts, tot + i0, (uint8_t *)d_out + i0 * dim * esize,
-                                                            nullptr, cnt, dim, norm_mode, canonical);
-        CU(cudaGetLastError());
-        h->stats.launches++;
-        return KTB_OK;
-    };
-    // ---- bucket-then-count (bucket_kernels.cuh): partition the k-mer codes of every tile by their high bits, then
-    // count each (sequence, code segment) in shared memory and write its part of the row once
-    const uint32_t log2_seg = (uint32_t)h->bucket_log2_seg;
-    const uint64_t nseg = (h->ncodes + (1ull << log2_seg) - 1) >> log2_seg;
-    if (h->bucket && h->force_path == 0 && nseg <= (uint64_t)BK_MAX_SEG && (dim & 3) == 0 && h->k <= 10 &&
-        (!canonical || (h->d_wave_tab && h->wave_seg_aligned)) && n < (1ull << 31) && total_bases < (1ull << 44)) {
-        const uint64_t tile_bases = (uint64_t)BK_TILE_CHUNKS * 16;
-        const uint64_t ntiles_bound = total_bases / tile_bases + 2 * n + 2;
-        if (ntiles_bound >= (1ull << 31)) return fail(KTB_ERR_ARG, "batch too large for the bucket path");
-        if (int rc = h->ws_tiles.ensure((n + 1) * 4 + 64 + ntiles_bound * sizeof(TileInfo))) return rc;
-        if (int rc = h->ws_pool.ensure(ntiles_bound * (uint64_t)BK_TILE_CAP * 2 + 64)) return rc;
-        if (int rc = h->ws_runs.ensure(ntiles_bound * nseg * 4)) return rc;
-        uint32_t *tile_prefix = (uint32_t *)h->ws_tiles.p;
-        TileInfo *tiles = (TileInfo *)((uint8_t *)h->ws_tiles.p + (((n + 1) * 4 + 63) & ~(uint64_t)63));
-        tile_prefix_kernel<<<1, 1024, 0, st>>>(d_offsets, n, (uint32_t)h->k, tile_prefix);
-        tile_info_kernel<<<(unsigned)std::min<uint64_t>((ntiles_bound + 255) / 256, (uint64_t)h->sm_count * 8), 256, 0, st>>>(
-            d_offsets, n, tile_prefix, tiles);
-        CU(cudaGetLastError());
-        h->stats.launches += 2;
-        BucketParams bp{};
-        bp.bases = d_bases; bp.n = n; bp.total_bases = total_bases;
-        bp.tile_prefix = tile_prefix; bp.tiles = tiles;
-        bp.pool = (uint16_t *)h->ws_pool.p; bp.runs = (uint32_t *)h->ws_runs.p; bp.totals = tot;
-        bp.k = (uint32_t)h->k; bp.nseg = (uint32_t)nseg; bp.log2_seg = log2_seg;
-        CountParams cp{};
-        cp.tile_prefix = tile_prefix; cp.pool = bp.pool; cp.runs = bp.runs; cp.totals_in = tot;
-        cp.totals_out = d_totals; cp.out = d_out;
-        cp.rank_tab = h->d_wave_tab; cp.tab_words = h->wave_tab_words;
-        cp.n = n; cp.dim = dim; cp.nseg = (uint32_t)nseg; cp.log2_seg = log2_seg;
-        cp.norm_mode = norm_mode; cp.canonical = canonical;
-#ifdef KTB_COUNT_PROBE
-        if (const char *e = getenv("KTB_COUNT_PROBE")) cp.probe = (uint32_t)atoi(e);
-#endif
-        void (*bkern)(const BucketParams) = canonical ? bucket_kernel<true> : bucket_kernel<false>;
-        if (canonical && log2_seg == 14) {   // the two shapes BASELINE.json names get their constants at compile time
-            if (h->k == 10) bkern = bucket_kernel<true, 10, 14>;
-            else if (h->k == 9) bkern = bucket_kernel<true, 9, 14>;
-        }
-        const bool nrm = norm_mode != NORM_COUNTS;
-        void (*ckern)(const CountParams) =
-            canonical ? (nrm ? count_kernel<OUT, true, true> : count_kernel<OUT, false, true>)
-                      : (nrm ? count_kernel<OUT, true, false> : count_kernel<OUT, false, false>);
-        // histogram memory: 64 KB either way — one buffer of 2^14 bins (segments with at most half as many columns
-        // alternate between its halves) or two buffers of 2^13
-        const size_t S = (size_t)1 << log2_seg;
-        cp.hist_words = (uint32_t)(log2_seg < 14 ? 2 * S : S);
-        if (h->bucket_hist_kb == 96) cp.hist_words = 24576;   // segments of up to 12,288 columns alternate between two halves
-        const size_t csmem = ((size_t)cp.hist_words + 2 * (S / 32)) * 4;
-        if (int rc = set_smem(ckern, csmem)) return rc;
-        int b_per_sm = 1, c_per_sm = 1;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&b_per_sm, bkern, BK_WARPS * 32, 0));
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&c_per_sm, ckern, CK_THREADS, csmem));
-        // Waves (option "bucket_waves", default 1): bucket_kernel is bound by the integer pipe, count_kernel by latency and
-        // the row writes, so the batch can be cut into waves with bucket_kernel(w+1) on one helper stream and
-        // count_kernel(w) on the other, sharing the SMs.  Measured on config 5ii (profiles/r2_sweeps.txt, batch r2i):
-        // 1.57 ms with one wave, 1.63 - 1.77 ms with 2 - 16 — the two kernels take each other's shared memory and
-        // registers and both lose more occupancy than the overlap returns.  Kept as an option.
-        const uint64_t nchunks = (n + CK_SEQ_CHUNK - 1) / CK_SEQ_CHUNK;
-        const uint64_t nwaves = std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)std::max(1, h->bucket_waves), nchunks / 16));
-        if (int rc = h->ws_wavectr.ensure(nwaves * sizeof(unsigned long long))) return rc;
-        CU(cudaMemsetAsync(h->ws_wavectr.p, 0, nwaves * sizeof(unsigned long long), st));
-        CU(cudaEventRecord(h->aux_ev[2], st));
-        cudaStream_t sb = nwaves > 1 ? h->aux[0] : st, sc = nwaves > 1 ? h->aux[1] : st;
-        if (nwaves > 1) {
-            CU(cudaStreamWaitEvent(sb, h->aux_ev[2], 0));
-            CU(cudaStreamWaitEvent(sc, h->aux_ev[2], 0));
-        }
-        const int b_ctas = nwaves > 1 ? std::min(b_per_sm, h->bucket_wave_ctas) : b_per_sm;
-        for (uint64_t w = 0; w < nwaves; ++w) {
-            const uint64_t c_lo = nchunks * w / nwaves, c_hi = nchunks * (w + 1) / nwaves;
-            bp.seq_lo = std::min(n, c_lo * CK_SEQ_CHUNK); bp.seq_hi = std::min(n, c_hi * CK_SEQ_CHUNK);
-            const uint64_t wave_tiles = (bp.seq_hi - bp.seq_lo) * 2 + (total_bases / tile_bases) / nwaves + 2;   // grid bound only
-            bkern<<<(unsigned)std::min<uint64_t>((uint64_t)h->sm_count * std::max(b_ctas, 1), wave_tiles), BK_WARPS * 32, 0, sb>>>(bp);
-            CU(cudaGetLastError());
-            if (nwaves > 1) {
-                if (h->wave_ev.size() <= w) {
-                    cudaEvent_t e = nullptr;
-                    CU(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-                    h->wave_ev.push_back(e);
-                }
-                CU(cudaEventRecord(h->wave_ev[w], sb));
-                CU(cudaStreamWaitEvent(sc, h->wave_ev[w], 0));
-            }
-            cp.chunk_lo = c_lo; cp.chunk_hi = c_hi;
-            cp.counter = (unsigned long long *)h->ws_wavectr.p + w;
-            const uint64_t units = (c_hi - c_lo) * nseg;
-            ckern<<<(unsigned)std::min<uint64_t>((uint64_t)h->sm_count * std::max(c_per_sm, 1), std::max<uint64_t>(units, 1)), CK_THREADS, csmem, sc>>>(cp);
-            CU(cudaGetLastError());
-            h->stats.launches += 2;
-        }
-        if (nwaves > 1) {
-            CU(cudaEventRecord(h->aux_ev[0], sb));
-            CU(cudaEventRecord(h->aux_ev[1], sc));
-            CU(cudaStreamWaitEvent(st, h->aux_ev[0], 0));
-            CU(cudaStreamWaitEvent(st, h->aux_ev[1], 0));
-        }
-        return KTB_OK;
-    }
-    if (h->force_path == 1) {   // testing: the flat-decomposition fallback, whole batch at once
-        uint32_t *counts = (uint32_t *)d_out;
-        if (OUT == OUT_F64) {
-            if (int rc = h->ws_counts.ensure(n * row_bytes)) return rc;
-            counts = (uint32_t *)h->ws_counts.p;
-        }
-        CU(cudaMemsetAsync(counts, 0, n * row_bytes, st));
-        if (total_bases > 0) {
-            FlatParams fp{};
-            fp.bases = d_bases; fp.offsets = d_offsets; fp.n = n; fp.total_bases = total_bases;
-            fp.counts = counts; fp.totals = tot;
-            fp.rank_full = canonical ? h->d_rank_full : nullptr;
-            fp.dim = dim; fp.k = h->k;
-            const uint64_t nchunks = (total_bases + FLAT_CHUNK - 1) / FLAT_CHUNK;
-            uint64_t grid = (nchunks + 255) / 256;
-            const uint64_t cap = (uint64_t)h->sm_count * 32;
-            if (grid > cap) grid = cap;
-            flat_kernel<<<(unsigned)grid, 256, 0, st>>>(fp);
-            CU(cudaGetLastError());
-            h->stats.launches++;
-        }
-        if (int rc = finalize(counts, 0, n)) return rc;
-    } else if (h->wave_persistent && h->coop_launch && OUT != OUT_F64 && n > 0) {
-        // One persistent cooperative launch: the wave loop (zero next rows / count / normalise previous rows)
-        // runs on the device with a grid barrier per wave instead of three launches per wave.
-        WaveParams wp{};
-        wp.bases = d_bases; wp.offsets = d_offsets; wp.n = n; wp.total_bases = total_bases;
-        wp.rows = (uint32_t *)d_out; wp.totals = tot;
-        wp.rank_full = canonical ? h->d_rank_full : nullptr;
-        wp.dim = dim; wp.k = (uint32_t)h->k; wp.norm_mode = norm_mode; wp.canonical = canonical;
-        // a wave is a third of the budget: the wave being counted and the next one (zeroed at the end of the
-        // iteration) are live together, the rest is slack for lines on their way out (32 MB waves measured best)
-        wp.wave_rows = std::max<uint64_t>(1, std::min<uint64_t>(256, (uint64_t)h->wave_budget_bytes / 3 / row_bytes));
-        const int rank_mode = !canonical ? 0 : (h->d_wave_tab && h->wave_tab_in_smem && h->wave_smem_rank) ? 2 : 1;
-        wp.rank_tab = h->d_wave_tab; wp.tab_words = h->wave_tab_words;
-        constexpr bool F32 = (OUT == OUT_F32);
-        const void *kern = rank_mode == 0 ? (const void *)wave_kernel<0, F32>
-                         : rank_mode == 1 ? (const void *)wave_kernel<1, F32> : (const void *)wave_kernel<2, F32>;
-        const int threads = 1024;
-        const size_t smem = rank_mode == 2 ? ((size_t)h->wave_tab_words * 6 + 16) : 0;
-        if (smem > 48 * 1024) CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        int per_sm = 1;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, smem));
-        if (per_sm < 1) return fail(KTB_ERR_CUDA, "wave_kernel does not fit on an SM (%zu bytes of shared memory)", smem);
-        const unsigned grid = (unsigned)h->sm_count;   // one CTA per SM: the RED rate of an SM does not grow with occupancy
-        void *args[] = {&wp};
-        CU(cudaLaunchCooperativeKernel(kern, dim3(grid), dim3(threads), args, smem, st));
-        h->stats.launches++;
-    } else {
-        // Waves of rows that fit L2 together: zero the wave's rows, let every CTA of the GPU work on that
-        // wave (sequences are split into tiles), normalise it, move on.  The REDs then hit rows that are
-        // still L2-resident and each row goes to HBM once; one big memset + one launch over the whole
-        // batch made every RED a 32-byte DRAM read-modify-write (measured 8.5 ms vs the 0.7 ms roofline).
-        SeqParams qp{};
-        qp.bases = d_bases; qp.offsets = d_offsets; qp.n = n; qp.total_bases = total_bases;
-        qp.rank_full = canonical ? h->d_rank_full : nullptr;
-        qp.counter = h->d_counters + 1;
-        qp.k = h->k; qp.dim = (uint32_t)dim; qp.hist_entries = 0;
-        qp.norm_mode = norm_mode; qp.canonical = canonical;
-        qp.list = nullptr; qp.list_count = nullptr; qp.group_size = 1;
-        qp.gtotals = tot;
-        auto kern = seq_kernel<OUT_U32, 3, false>;
-        const int threads = h->seq_threads > 0 ? h->seq_threads : 128;
-        int per_sm = 1;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, threads, 0));
-        const uint64_t ctas = (uint64_t)h->sm_count * std::max(per_sm, 1);
-        // two waves in flight (one per helper stream), each half of the L2 budget
-        const uint64_t wave = std::max<uint64_t>(1, std::min<uint64_t>(n, (uint64_t)h->global_wave_bytes / 2 / row_bytes));
-        if (OUT == OUT_F64)
-            if (int rc = h->ws_counts.ensure(2 * wave * row_bytes)) return rc;
-        // a work item = (sequence, tile).  A wave is small (rows must fit L2), so parallelism has to come from
-        // splitting sequences finely: about `global_steps_per_warp` steps of 512 bases per warp (the first
-        // version used 4 and ran 5 warps per SM; one step per warp fills the machine).
-        const uint64_t mean_steps = (total_bases / std::max<uint64_t>(n, 1)) / 512 + 1;
-        const uint64_t per_item = (uint64_t)std::max(1, h->global_steps_per_warp) * (threads / 32);
-        const uint32_t tiles = (uint32_t)std::max<uint64_t>(1, std::min<uint64_t>(4096, mean_steps / per_item));
-        CU(cudaEventRecord(h->aux_ev[2], st));
-        uint64_t w = 0;
-        for (uint64_t i0 = 0; i0 < n; i0 += wave, ++w) {
-            const int x = (int)(w & 1);
-            cudaStream_t sx = h->aux[x];
-            if (w < 2) CU(cudaStreamWaitEvent(sx, h->aux_ev[2], 0));
-            const uint64_t cnt = std::min(wave, n - i0);
-            uint32_t *counts = (OUT == OUT_F64) ? (uint32_t *)h->ws_counts.p + (uint64_t)x * wave * dim
-                                                : (uint32_t *)d_out + i0 * dim;
-            CU(cudaMemsetAsync(counts, 0, cnt * row_bytes, sx));
-            CU(cudaMemsetAsync(h->d_counters + 4 + x, 0, sizeof(unsigned long long), sx));
-            qp.counter = h->d_counters + 4 + x;
-            qp.gcounts = counts; qp.seq_base = i0; qp.seq_count = cnt; qp.tiles = tiles;
-            const uint64_t items = cnt * tiles;
-            kern<<<(unsigned)std::min(ctas, items), threads, 0, sx>>>(qp);
-            CU(cudaGetLastError());
-            h->stats.launches++;
-            if (OUT != OUT_U32) {
-                const uint64_t nel = cnt * dim;
-                uint64_t grid = std::min<uint64_t>((nel + 255) / 256, (uint64_t)h->sm_count * 16);
-                finalize_kernel<OUT><<<(unsigned)grid, 256, 0, sx>>>(counts, tot + i0, (uint8_t *)d_out + i0 * dim * esize,
-                                                                    nullptr, cnt, dim, norm_mode, canonical);
-                CU(cudaGetLastError());
-                h->stats.launches++;
-            }
-        }
-        for (int x = 0; x < 2; ++x) {   // join the helper streams back into the caller's stream
-            CU(cudaEventRecord(h->aux_ev[x], h->aux[x]));
-            CU(cudaStreamWaitEvent(st, h->aux_ev[x], 0));
-        }
-    }
-    if (d_totals) CU(cudaMemcpyAsync(d_totals, tot, n * 8, cudaMemcpyDeviceToDevice, st));
-    (void)esize;
+    CU(cudaMemsetAsync(tot, 0, b.n * 8, b.st));
+    const uint64_t nseg = (h->ncodes + (1ull << h->bucket_log2_seg) - 1) >> h->bucket_log2_seg;
+    if (h->bucket && h->force_path == 0 && nseg <= (uint64_t)BK_MAX_SEG && (b.dim & 3) == 0 && h->k <= 10 &&
+        (!b.canonical || (h->d_wave_tab && h->wave_seg_aligned)) && b.n < (1ull << 31) && b.total_bases < (1ull << 44))
+        return launch_bucket<OUT>(h, b, tot, nseg);
+    const int rc = h->force_path == 1 ? launch_flat<OUT>(h, b, tot)
+                 : (h->wave_persistent && h->coop_launch && OUT != OUT_F64) ? launch_wave_kernel<OUT>(h, b, tot)
+                 : launch_wave_loop<OUT>(h, b, tot);
+    if (rc) return rc;
+    if (b.totals) CU(cudaMemcpyAsync(b.totals, tot, b.n * 8, cudaMemcpyDeviceToDevice, b.st));
     return KTB_OK;
 }
 
 int dispatch_device(ktb_oligo *h, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
                     uint64_t total_bases, int canonical, int norm_mode, int out_dtype, void *d_out,
                     uint64_t *d_totals, cudaStream_t st) {
+    const Batch b{d_bases, d_offsets, n, total_bases, canonical ? h->dim_canon : h->ncodes, canonical, norm_mode,
+                  d_out, d_totals, st};
     switch (out_dtype) {
-        case KTB_OUT_U32:
-            return run_device<OUT_U32>(h, d_bases, d_offsets, n, total_bases, canonical, norm_mode, d_out, d_totals, st);
-        case KTB_OUT_F32:
-            return run_device<OUT_F32>(h, d_bases, d_offsets, n, total_bases, canonical, norm_mode, d_out, d_totals, st);
-        default:
-            return run_device<OUT_F64>(h, d_bases, d_offsets, n, total_bases, canonical, norm_mode, d_out, d_totals, st);
+        case KTB_OUT_U32: return run_device<OUT_U32>(h, b);
+        case KTB_OUT_F32: return run_device<OUT_F32>(h, b);
+        default: return run_device<OUT_F64>(h, b);
     }
 }
 
@@ -757,7 +768,6 @@ __attribute__((visibility("hidden"))) int ktb_internal_dispatch(ktb_oligo *h, co
     return dispatch_device(h, d_bases, d_offsets, n, total_bases, canonical, norm_mode, out_dtype, d_out, d_totals, st);
 }
 __attribute__((visibility("hidden"))) int ktb_internal_fail(int code, const char *msg) { return fail(code, "%s", msg); }
-__attribute__((visibility("hidden"))) int ktb_internal_device(const ktb_oligo *h) { return h->device; }
 __attribute__((visibility("hidden"))) int ktb_internal_sms(const ktb_oligo *h) { return h->sm_count; }
 __attribute__((visibility("hidden"))) uint64_t ktb_internal_launches(const ktb_oligo *h) { return h->stats.launches; }
 
@@ -782,6 +792,12 @@ __global__ void rebase_offsets_kernel(uint64_t *offs, uint64_t count, uint64_t b
 double now_ms() {
     using namespace std::chrono;
     return duration<double, std::milli>(steady_clock::now().time_since_epoch()).count();
+}
+
+// Copies a table into a new device allocation of exactly its size.
+cudaError_t upload(uint32_t **d, const std::vector<uint32_t> &tab) {
+    const cudaError_t e = cudaMalloc(d, tab.size() * 4);
+    return e != cudaSuccess ? e : cudaMemcpy(*d, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice);
 }
 
 }  // namespace
@@ -849,20 +865,17 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
             return bail(fail(KTB_ERR_CUDA, "%s failed: %s", #call, cudaGetErrorString(e_)));       \
     } while (0)
 
-    CUB(cudaMalloc(&h->d_rank_full, h->ncodes * 4));
-    CUB(cudaMemcpy(h->d_rank_full, rank_full.data(), h->ncodes * 4, cudaMemcpyHostToDevice));
+    CUB(upload(&h->d_rank_full, rank_full));
     std::vector<uint32_t> cor(h->canon_of_rank);
     while (cor.size() % 4) cor.push_back(0);
-    CUB(cudaMalloc(&h->d_canon_of_rank, cor.size() * 4));
-    CUB(cudaMemcpy(h->d_canon_of_rank, cor.data(), cor.size() * 4, cudaMemcpyHostToDevice));
+    CUB(upload(&h->d_canon_of_rank, cor));
     {
         std::vector<uint32_t> perm(cor.size(), 0);
         const uint64_t nblk = h->dim_canon / 128;
         for (uint64_t b = 0; b < nblk; ++b)
             for (uint32_t l = 0; l < 32; ++l)
                 for (uint32_t e = 0; e < 4; ++e) perm[b * 128 + 4 * l + e] = cor[b * 128 + 32 * e + l];
-        CUB(cudaMalloc(&h->d_canon_perm, perm.size() * 4));
-        CUB(cudaMemcpy(h->d_canon_perm, perm.data(), perm.size() * 4, cudaMemcpyHostToDevice));
+        CUB(upload(&h->d_canon_perm, perm));
         if (!(k & 1) && k >= 6 && k <= 8) {  // rank tables of seq_kernel mode 7 (see kernels.cuh)
             const uint32_t hd = k / 2, H = 1u << (2 * hd), wpr = H / 32;   // halves of hd bases, words per row
             std::vector<uint32_t> tab((size_t)H * wpr + ((size_t)H * wpr + 1) / 2, 0);
@@ -880,8 +893,7 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
             }
             if (running == h->dim_canon && h->dim_canon <= 65535u + 32u) {
                 h->even_words = H * wpr;
-                CUB(cudaMalloc(&h->d_even_tab, tab.size() * 4));
-                CUB(cudaMemcpy(h->d_even_tab, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice));
+                CUB(upload(&h->d_even_tab, tab));
             }
         }
         if (k & 1) {  // dense half-size index of seq_kernel mode 4 (see kernels.cuh)
@@ -899,10 +911,8 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
             for (uint64_t b = 0; b < nblk; ++b)
                 for (uint32_t l = 0; l < 32; ++l)
                     for (uint32_t e = 0; e < 4; ++e) mbp[b * 128 + 4 * l + e] = mb[b * 128 + 32 * e + l];
-            CUB(cudaMalloc(&h->d_mb_of_rank, mb.size() * 4));
-            CUB(cudaMemcpy(h->d_mb_of_rank, mb.data(), mb.size() * 4, cudaMemcpyHostToDevice));
-            CUB(cudaMalloc(&h->d_mb_perm, mbp.size() * 4));
-            CUB(cudaMemcpy(h->d_mb_perm, mbp.data(), mbp.size() * 4, cudaMemcpyHostToDevice));
+            CUB(upload(&h->d_mb_of_rank, mb));
+            CUB(upload(&h->d_mb_perm, mbp));
         }
     }
     if (k == 7) {   // long_kernel MODE_K7: bin of a class = [b3 b4 b5 b6 | b0 b1 b2] of the strand whose middle base is A/C
@@ -921,8 +931,7 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
                     const uint32_t j = order[g * 32 + l];
                     sched[((g >> 2) * 32 + l) * 4 + (g & 3)] = (word[j] * 4u) | ((j * 4u) << 16);
                 }
-            CUB(cudaMalloc(&h->d_k7_sched, sched.size() * 4));
-            CUB(cudaMemcpy(h->d_k7_sched, sched.data(), sched.size() * 4, cudaMemcpyHostToDevice));
+            CUB(upload(&h->d_k7_sched, sched));
         }
     }
     // long_kernel MODE_FWD: fold table, rank -> (c, rc(c)).  k = 6 stays with seq_kernel: its fold gathers hist[rc(c)] for
@@ -933,8 +942,7 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
             const uint32_t c = h->canon_of_rank[j], r = (uint32_t)rev_comp(c, k);
             sched[j] = (c * 4u) | (((r == c) ? (uint32_t)h->ncodes : r) * 4u) << 16;
         }
-        CUB(cudaMalloc(&h->d_fwd_sched, sched.size() * 4));
-        CUB(cudaMemcpy(h->d_fwd_sched, sched.data(), sched.size() * 4, cudaMemcpyHostToDevice));
+        CUB(upload(&h->d_fwd_sched, sched));
     }
     {   // bitmap of the canonical codes + running rank per pair of words: rank(c) = prefix[w / 2] + popc(bits below c).
         // wave_kernel<2> keeps the whole table in shared memory (k <= 10); count_kernel loads one segment's slice.
@@ -958,8 +966,7 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
             h->wave_tab_words = (uint32_t)words;
             h->wave_tab_in_smem = bytes + 4096 <= h->smem_optin;
             h->wave_seg_aligned = aligned;
-            CUB(cudaMalloc(&h->d_wave_tab, tab.size() * 4));
-            CUB(cudaMemcpy(h->d_wave_tab, tab.data(), tab.size() * 4, cudaMemcpyHostToDevice));
+            CUB(upload(&h->d_wave_tab, tab));
         }
     }
     if (h->ncodes <= (uint64_t)ktb::SHORT_MAX_CODES) {
@@ -969,10 +976,8 @@ int ktb_oligo_create(int k, int device, ktb_oligo **out) {
             tc[x] = ((a & ~3u) << 22) | ((a & 3u) * 8u);
             tr[x] = ((b & ~3u) << 22) | ((b & 3u) * 8u);
         }
-        CUB(cudaMalloc(&h->d_short_tab_canon, h->ncodes * 4));
-        CUB(cudaMalloc(&h->d_short_tab_raw, h->ncodes * 4));
-        CUB(cudaMemcpy(h->d_short_tab_canon, tc.data(), h->ncodes * 4, cudaMemcpyHostToDevice));
-        CUB(cudaMemcpy(h->d_short_tab_raw, tr.data(), h->ncodes * 4, cudaMemcpyHostToDevice));
+        CUB(upload(&h->d_short_tab_canon, tc));
+        CUB(upload(&h->d_short_tab_raw, tr));
     }
     CUB(cudaMalloc(&h->d_counters, 16 * sizeof(unsigned long long)));
     for (auto &s : h->sets) {
@@ -1000,37 +1005,16 @@ void ktb_oligo_destroy(ktb_oligo *h) {
         }
         for (auto &e : s.ev)
             if (e) cudaEventDestroy(e);
-        s.bases.release();
-        s.offsets.release();
-        s.out.release();
-        s.totals.release();
     }
     for (auto &a : h->aux) if (a) { cudaStreamSynchronize(a); cudaStreamDestroy(a); }
     for (auto &e : h->aux_ev) if (e) cudaEventDestroy(e);
     if (h->ref_ev) cudaEventDestroy(h->ref_ev);
-    h->ws_totals.release();
-    h->ws_counts.release();
-    h->ws_list.release();
-    h->ws_list2.release();
-    h->ws_order.release();
-    h->ws_tiles.release();
-    h->ws_pool.release();
-    h->ws_runs.release();
-    h->ws_wavectr.release();
     for (auto &e : h->wave_ev) if (e) cudaEventDestroy(e);
-    if (h->d_rank_full) cudaFree(h->d_rank_full);
-    if (h->d_canon_of_rank) cudaFree(h->d_canon_of_rank);
-    if (h->d_canon_perm) cudaFree(h->d_canon_perm);
-    if (h->d_mb_of_rank) cudaFree(h->d_mb_of_rank);
-    if (h->d_mb_perm) cudaFree(h->d_mb_perm);
-    if (h->d_even_tab) cudaFree(h->d_even_tab);
-    if (h->d_wave_tab) cudaFree(h->d_wave_tab);
-    if (h->d_k7_sched) cudaFree(h->d_k7_sched);
-    if (h->d_fwd_sched) cudaFree(h->d_fwd_sched);
-    if (h->d_short_tab_canon) cudaFree(h->d_short_tab_canon);
-    if (h->d_short_tab_raw) cudaFree(h->d_short_tab_raw);
+    for (uint32_t *t : {h->d_rank_full, h->d_canon_of_rank, h->d_canon_perm, h->d_mb_of_rank, h->d_mb_perm, h->d_even_tab,
+                        h->d_wave_tab, h->d_k7_sched, h->d_fwd_sched, h->d_short_tab_canon, h->d_short_tab_raw})
+        if (t) cudaFree(t);
     if (h->d_counters) cudaFree(h->d_counters);
-    delete h;
+    delete h;   // the scratch buffers free themselves, on this device
 }
 
 int ktb_oligo_k(const ktb_oligo *h) { return h ? h->k : 0; }
@@ -1213,8 +1197,6 @@ int ktb_oligo_vectorise(ktb_oligo *h, const uint8_t *bases, const uint64_t *offs
 
     int b = 0;
     cudaEvent_t prev_kernels_done = nullptr;
-    const uint64_t launches_before = 0;
-    (void)launches_before;
     uint64_t total_launches = 0;
     uint64_t checked = 0;   // offsets[0 .. checked] are known to be non-decreasing and <= offsets[n]
     auto bad_offsets = [&](uint64_t upto) -> int64_t {

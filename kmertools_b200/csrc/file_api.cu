@@ -26,7 +26,6 @@ int ktb_internal_dispatch(ktb_oligo *h, const uint8_t *d_bases, const uint64_t *
                           uint64_t total_bases, int canonical, int norm_mode, int out_dtype, void *d_out,
                           uint64_t *d_totals, cudaStream_t st);
 int ktb_internal_fail(int code, const char *msg);
-int ktb_internal_device(const ktb_oligo *h);
 int ktb_internal_sms(const ktb_oligo *h);
 uint64_t ktb_internal_launches(const ktb_oligo *h);
 
