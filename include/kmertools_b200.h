@@ -139,7 +139,8 @@ int ktb_oligo_last_stats(const ktb_oligo *h, ktb_stats *out);
 /* Tuning knobs (testing / benchmarking).  Known keys:
  *   "chunk_bytes"        target bytes of output per pipeline chunk in the host entry point
  *   "force_path"         0 auto, 1 flat-decomposition global-atomic kernel only, 2 no short-read kernel
- *   "seq_threads"        CTA size of the CTA-per-sequence kernel (0 = heuristic)
+ *   "seq_threads"        CTA size of the CTA-per-sequence kernel (0 = heuristic); each kernel clamps it to its own
+ *                        launch bound: 1024 for the 32-bit rank-space histograms of k = 8, 256 everywhere else
  *   "seq_grab"           sequences a CTA of that kernel takes per trip to the work counter (0 = heuristic)
  *   "dense_odd"          1 (default): dense middle-base histogram for k = 7 in seq_kernel (mode 4), 0: code-space histogram
  *   "even_rank"          1 (default): even k whose rank-space histogram fits shared memory (k = 8) compute the rank from two

@@ -624,7 +624,8 @@ int launch_wave_loop(ktb_oligo *h, const Batch &b, unsigned long long *tot) {
     qp.list = nullptr; qp.list_count = nullptr; qp.group_size = 1;
     qp.gtotals = tot;
     auto kern = seq_kernel<OUT_U32, 3, false>;
-    const int threads = h->seq_threads > 0 ? h->seq_threads : 128;
+    // mode 3 is compiled for at most KTB_SEQ_MAXTHREADS threads: a larger CTA would not launch
+    const int threads = std::min(h->seq_threads > 0 ? h->seq_threads : 128, KTB_SEQ_MAXTHREADS);
     // two waves in flight (one per helper stream), each half of the L2 budget
     const uint64_t wave = std::max<uint64_t>(1, std::min<uint64_t>(n, (uint64_t)h->global_wave_bytes / 2 / row_bytes));
     if (OUT == OUT_F64)
