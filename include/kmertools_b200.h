@@ -132,6 +132,41 @@ int ktb_oligo_vectorise_device(ktb_oligo *h, const uint8_t *d_bases, const uint6
                                uint64_t n, uint64_t total_bases, int canonical, int norm_mode,
                                int out_dtype, void *d_out, uint64_t *d_totals, void *stream);
 
+/* ---- sparse rows: per-sequence k-mer counts as CSR, 1 <= k <= KTB_MAX_SPARSE_K -------------------------------
+ * The histogram of ktb_oligo_vectorise, stored as its non-zero entries.  For every sequence i and every valid window
+ * (same decoding, validity and codes as ktb_kmer_pairs) key = min(forward, reverse complement) when canonical, the
+ * forward code otherwise.  Row i holds every distinct key of sequence i in ascending order: codes[j] is the key (2-bit
+ * code, A=0 C=1 G=2 T=3, first base most significant), values[j] its count as out_dtype with the normalisation of
+ * the dense rows (the same divisor, the same f64 quotient, the same f32 rounding), so for k <= KTB_MAX_K scattering a
+ * row through ktb_oligo_pos_maps (canonical) or by code (raw) gives the dense row bit for bit.  totals[i] = number of
+ * valid windows.  Empty sequences, sequences shorter than k and all-ambiguous ones give empty rows.
+ * Counts are 32-bit: a sequence must have fewer than 2^32 windows.  No handle: no tables are involved. */
+#define KTB_MAX_SPARSE_K 31
+
+/* HOST buffers.  row_ptr: n+1 entries, row_ptr[0] = 0, row i = entries [row_ptr[i], row_ptr[i+1]).
+ * row_ptr (and totals, if not NULL) is always complete; codes / values are written only below cap
+ * (cap = sum over sequences of max(0, len - k + 1) always suffices; cap = 0 with NULL arrays only sizes).
+ * The batch is processed in chunks of whole sequences (about 2^26 bases each) on two streams: chunk c + 1 is copied
+ * in and computed while the rows of chunk c are copied out (row_ptr and totals through page-locked staging).
+ * A sequence with 2^32 or more windows is KTB_ERR_ARG. */
+int ktb_sparse_vectorise(const uint8_t *bases, const uint64_t *offsets, uint64_t n, int k, int canonical,
+                         int norm_mode, int out_dtype, int device, uint64_t *row_ptr, uint64_t *codes,
+                         void *values, uint64_t cap, uint64_t *totals);
+
+/* DEVICE buffers of the current device, enqueued on `stream` (a cudaStream_t; NULL = default stream); returns after
+ * enqueueing, with no host round trip and no state shared between calls, so calls on different streams are
+ * independent.  Offsets are absolute positions in d_bases as in ktb_oligo_vectorise_device (offsets[0] may be > 0);
+ * total_bases must be at least offsets[n] (equal is the tightest): no byte at or beyond offsets[n] is read, and the
+ * scratch is sized from total_bases.  d_row_ptr (n+1) and d_totals (n, may be NULL) are always complete; no element
+ * of d_codes / d_values at or beyond cap is written.  Precondition: every sequence has fewer than 2^32 windows.
+ * Scratch from the stream-ordered allocator: 24 bytes per base of total_bases (rounded up to 4096 bases) plus
+ * 40 bytes per sequence.  The bases before offsets[0] count too: for a small batch deep inside a large buffer, pass
+ * d_bases + offsets[0] with rebased offsets to keep the scratch small. */
+int ktb_sparse_vectorise_device(const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
+                                uint64_t total_bases, int k, int canonical, int norm_mode, int out_dtype,
+                                uint64_t *d_row_ptr, uint64_t *d_codes, void *d_values, uint64_t cap,
+                                uint64_t *d_totals, void *stream);
+
 /* Stats of the most recent vectorise call (host entry point: complete; device entry point: launch
  * counts and class sizes only). */
 int ktb_oligo_last_stats(const ktb_oligo *h, ktb_stats *out);

@@ -55,6 +55,8 @@ SYMBOLS = {
     "ktb_kmer_pairs_device": (_I, [_VP, _U64, _I, _VP, _VP, _U64, _VP, _VP]),
     "ktb_oligo_vectorise": (_I, [_VP, _VP, _VP, _U64, _I, _I, _I, _VP, _VP]),
     "ktb_oligo_vectorise_device": (_I, [_VP, _VP, _VP, _U64, _U64, _I, _I, _I, _VP, _VP, _VP]),
+    "ktb_sparse_vectorise": (_I, [_VP, _VP, _U64, _I, _I, _I, _I, _I, _VP, _VP, _VP, _U64, _VP]),
+    "ktb_sparse_vectorise_device": (_I, [_VP, _VP, _U64, _U64, _I, _I, _I, _I, _VP, _VP, _VP, _U64, _VP, _VP]),
     "ktb_oligo_last_stats": (_I, [_VP, C.POINTER(Stats)]),
     "ktb_oligo_set_option": (_I, [_VP, C.c_char_p, C.c_int64]),
     "ktb_host_alloc": (_VP, [_SZ]),
