@@ -167,6 +167,54 @@ int ktb_sparse_vectorise_device(const uint8_t *d_bases, const uint64_t *d_offset
                                 uint64_t *d_row_ptr, uint64_t *d_codes, void *d_values, uint64_t cap,
                                 uint64_t *d_totals, void *stream);
 
+/* ---- batch-wide k-mer counting: one table of a whole data set, 1 <= k <= KTB_MAX_SPARSE_K ----------------------
+ * Replaces CountComputer (`kmertools ctr`).  A counter has a fixed k and mode.  Adding a batch counts every valid
+ * window of every sequence (same decoding, validity and codes as ktb_kmer_pairs), keyed by min(forward, reverse
+ * complement) when canonical, by the forward code otherwise.  After any sequence of adds the table is every distinct
+ * key seen, in ascending order, with a u64 count of its windows; it does not depend on how the input was split into
+ * adds or on their order.  The sum of the counts is the number of valid windows added (nwindows).  Empty sequences,
+ * sequences shorter than k and all-ambiguous ones contribute nothing.
+ *
+ * The table lives on the counter's device: 16 bytes per distinct key.  An add also needs scratch from the
+ * stream-ordered allocator: 33 bytes per base of the batch (per base of total_bases for a device add; per base of a
+ * chunk for a host add) plus, while the merge runs, the new table: 16 bytes per distinct key of the old table plus
+ * 16 bytes per base (at most 16 * 4^k in all).  A table or scratch that does not fit device memory is KTB_ERR_NOMEM
+ * and leaves the counter as it was; nothing spills to the host or to disk.
+ * Every add returns when the batch is in the table: it waits for its stream once, at the end, to learn the new table
+ * size.  Calls on ONE counter must be ordered by the caller; different counters are independent. */
+typedef struct ktb_counter ktb_counter;
+
+/* 1 <= k <= KTB_MAX_SPARSE_K, canonical 0 or 1, device a CUDA ordinal.  Arguments are checked before any device work;
+ * without a device the call is KTB_ERR_NODEVICE (there is no CPU path). */
+int ktb_counter_create(int k, int canonical, int device, ktb_counter **out);
+void ktb_counter_destroy(ktb_counter *c);
+
+/* HOST buffers, layout of ktb_sparse_vectorise (offsets: n+1 entries, non-decreasing).  The batch is processed in
+ * chunks of whole sequences (about 2^26 bases each; a longer sequence is a chunk of its own) on two streams of the
+ * counter's device: chunk c + 1 is copied in while chunk c is counted and merged.  Returns when the batch is in the
+ * table; synchronises only its own streams. */
+int ktb_counter_add(ktb_counter *c, const uint8_t *bases, const uint64_t *offsets, uint64_t n);
+
+/* DEVICE buffers on the counter's device, enqueued on `stream` (a cudaStream_t; NULL = default stream).  Offsets are
+ * absolute positions in d_bases as in ktb_sparse_vectorise_device (offsets[0] may be > 0); total_bases must be at least
+ * offsets[n]: no byte at or beyond offsets[n] is read, and the scratch is sized from total_bases (for a small batch
+ * deep inside a large buffer, pass d_bases + offsets[0] with rebased offsets).  Waits for `stream` once, after the
+ * merge, to read the new table size; the buffers may be reused when the call returns. */
+int ktb_counter_add_device(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
+                           uint64_t total_bases, void *stream);
+
+/* Distinct keys of the table and valid windows added so far (either pointer may be NULL).  Every add has finished
+ * when it returns, so this reads host fields and synchronises nothing. */
+int ktb_counter_size(ktb_counter *c, uint64_t *nkeys, uint64_t *nwindows);
+
+/* The first min(nkeys, cap) keys (ascending) and their counts into HOST memory; synchronous.  Nothing at or beyond
+ * that index is written; cap = 0 writes nothing, and a NULL array is skipped. */
+int ktb_counter_read(ktb_counter *c, uint64_t *keys, uint64_t *counts, uint64_t cap);
+
+/* Same into DEVICE memory of the counter's device: device-to-device copies enqueued on `stream`, returns after
+ * enqueueing.  The copies read the table in place, so the next add on the counter must be ordered after them. */
+int ktb_counter_read_device(ktb_counter *c, uint64_t *d_keys, uint64_t *d_counts, uint64_t cap, void *stream);
+
 /* Stats of the most recent vectorise call (host entry point: complete; device entry point: launch
  * counts and class sizes only). */
 int ktb_oligo_last_stats(const ktb_oligo *h, ktb_stats *out);
@@ -271,6 +319,15 @@ int ktb_comp_oligo_file(const ktb_file_opts *opts, ktb_file_stats *stats /* opti
  * canonical histogram, printed as "(x,y,freq)" triples where (x,y) is the fixed chaos-game point of the
  * column's k-mer in a vecsize x vecsize square.  Uses in_path, out_path, k, norm, device of `opts`. */
 int ktb_comp_cgr_file(const ktb_file_opts *opts, int vecsize, ktb_file_stats *stats /* optional */);
+
+/* `kmertools ctr`: the canonical k-mer counts of a whole file (ktb_counter_*, 1 <= k <= KTB_MAX_SPARSE_K).  Uses
+ * in_path, out_path, k, threads and device of `opts`; the input format follows ktb_comp_oligo_file (the extension
+ * decides, "-" = stdin sniffs the first byte).  The file is parsed in batches into one counter, parsing batch b + 1
+ * while batch b is added.  out_path is a directory, created if missing; the table is written to out_path/kmers.counts,
+ * one line per distinct k-mer in ascending code order: "<code>\t<count>\n" with the code in decimal, or with acgt != 0
+ * the k-mer as k characters of ACGT (first base first).  The table is read back in slices through page-locked staging
+ * and formatted by `threads` host threads.  stats->bases counts the bases parsed, stats->bytes_written the text. */
+int ktb_count_file(const ktb_file_opts *opts, int acgt, ktb_file_stats *stats /* optional */);
 
 /* The file-level drivers keep their pinned / device buffer sets (at most ~0.5 GB) for the next call on the same
  * device; this frees them. */

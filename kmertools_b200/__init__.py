@@ -7,6 +7,7 @@ it under the reference's module name.
 from .oligo import OligoComputer, MultiOligoComputer, HostBuffer, shard_bounds  # noqa: F401
 from .kmers import KmerGenerator, kmer_pairs  # noqa: F401
 from .sparse import kmer_counts, kmer_counts_tensors  # noqa: F401
+from .counter import KmerCounter  # noqa: F401
 from ._lib import KtbError  # noqa: F401
 
 __version__ = "0.1.0"

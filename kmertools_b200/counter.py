@@ -1,0 +1,111 @@
+"""Batch-wide k-mer counting for 1 <= k <= 31 on top of ktb_counter_* (the table of `kmertools ctr`).
+
+A KmerCounter keeps one table on its GPU: every distinct key seen so far (canonical: min(forward, reverse complement);
+raw: forward) in ascending order, with a u64 count of its windows.  Keys are 2-bit codes (A=0 C=1 G=2 T=3, first base
+most significant), as kmer_pairs and kmer_counts return them.  The table does not depend on how the input is split
+into adds or on their order.
+"""
+from __future__ import annotations
+
+import ctypes as C
+
+import numpy as np
+
+from . import _lib
+from .sparse import _check_k, _packed
+
+
+class KmerCounter:
+    """KmerCounter(ksize, mins=True, device=0): add batches with add / add_tensors, read the table with result /
+    result_tensors.  Every add returns when the batch is in the table."""
+
+    def __init__(self, ksize: int, mins: bool = True, device: int = 0):
+        self.ksize = _check_k(ksize)
+        self.mins = bool(mins)
+        self.device = int(device)
+        self._h = C.c_void_p()
+        _lib.check(_lib.load().ktb_counter_create(self.ksize, int(self.mins), self.device, C.byref(self._h)))
+
+    def _handle(self):
+        if not self._h:
+            raise ValueError("the counter is closed")
+        return self._h
+
+    def add(self, seqs_or_packed) -> None:
+        """Counts a list of str / bytes, or a packed (bases u8, offsets u64[n+1]) pair, from host memory."""
+        bases, offsets = _packed(seqs_or_packed)
+        n = len(offsets) - 1
+        _lib.check(_lib.load().ktb_counter_add(self._handle(), bases.ctypes.data if bases.size else None,
+                                               offsets.ctypes.data, max(n, 0)))
+
+    def add_tensors(self, bases, offsets) -> None:
+        """Counts CUDA tensors on the counter's device, on torch's current stream: `bases` uint8, `offsets` int64 (n+1,
+        absolute positions in `bases`).  The scratch is sized from bases.numel(): for a small batch inside a large
+        buffer, pass the slice bases[offsets[0]:offsets[n]] and offsets - offsets[0]."""
+        import torch
+        if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
+            raise ValueError("bases and offsets must be CUDA tensors on one device")
+        if bases.device.index != self.device:
+            raise ValueError(f"the tensors are on {bases.device}, the counter on cuda:{self.device}")
+        if bases.dtype != torch.uint8 or offsets.dtype != torch.int64:
+            raise TypeError(f"bases must be uint8 and offsets int64 (got {bases.dtype}, {offsets.dtype})")
+        if not (bases.is_contiguous() and offsets.is_contiguous()):
+            raise ValueError("bases and offsets must be contiguous")
+        n = offsets.numel() - 1
+        total = bases.numel()
+        with torch.cuda.device(bases.device):
+            stream = torch.cuda.current_stream(bases.device).cuda_stream
+            _lib.check(_lib.load().ktb_counter_add_device(self._handle(), bases.data_ptr() if total else None,
+                                                          offsets.data_ptr(), max(n, 0), total, stream))
+
+    def _size(self):
+        nkeys, nwin = C.c_uint64(), C.c_uint64()
+        _lib.check(_lib.load().ktb_counter_size(self._handle(), C.byref(nkeys), C.byref(nwin)))
+        return nkeys.value, nwin.value
+
+    def __len__(self) -> int:
+        return self._size()[0]
+
+    @property
+    def windows(self) -> int:
+        """Valid windows added so far (the sum of the counts)."""
+        return self._size()[1]
+
+    def result(self):
+        """(keys u64, counts u64) as numpy arrays, keys ascending."""
+        n = len(self)
+        keys = np.empty(n, dtype=np.uint64)
+        counts = np.empty(n, dtype=np.uint64)
+        _lib.check(_lib.load().ktb_counter_read(self._handle(), keys.ctypes.data if n else None,
+                                                counts.ctypes.data if n else None, n))
+        return keys, counts
+
+    def result_tensors(self):
+        """(keys, counts) as int64 CUDA tensors on the counter's device, copied on torch's current stream."""
+        import torch
+        n = len(self)
+        dev = torch.device("cuda", self.device)
+        keys = torch.empty(n, dtype=torch.int64, device=dev)
+        counts = torch.empty(n, dtype=torch.int64, device=dev)
+        with torch.cuda.device(dev):
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            _lib.check(_lib.load().ktb_counter_read_device(self._handle(), keys.data_ptr() if n else None,
+                                                           counts.data_ptr() if n else None, n, stream))
+        return keys, counts
+
+    def close(self) -> None:
+        if self._h:
+            _lib.load().ktb_counter_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass

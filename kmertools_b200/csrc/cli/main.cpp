@@ -1,6 +1,7 @@
 // kmertools — drop-in for the reference CLI's `comp oligo` subcommand (kmertools/src/args.rs:70-103,
 // 242-263).  Same flags, same defaults, same output bytes; compute runs on the GPU through
-// libkmertools_b200.so.  Other subcommands of the reference are out of scope (SURVEY.md §2).
+// libkmertools_b200.so.  Also `comp cgr -k` and `ctr` (batch-wide k-mer counts, with this build's own output file).
+// Other subcommands of the reference are out of scope (SURVEY.md §2).
 #include "../../../include/kmertools_b200.h"
 
 #include <cstdio>
@@ -61,11 +62,80 @@ static int main_cgr(int argc, char **argv) {
     return 0;
 }
 
+static void usage_ctr() {
+    fprintf(stderr,
+            "Count the canonical k-mers of a whole file (GPU)\n\n"
+            "Usage: kmertools ctr [OPTIONS] --input <INPUT> --output <OUTPUT> --k-size <K_SIZE>\n\n"
+            "Writes OUTPUT/kmers.counts (OUTPUT is a directory, created if missing): one line per distinct canonical\n"
+            "k-mer, min(forward, reverse complement), in ascending code order, as \"<code>\\t<count>\\n\" with the 2-bit\n"
+            "code (A=0 C=1 G=2 T=3, first base most significant) in decimal.  The file name and line form are this\n"
+            "build's own; the reference writes its counts in another order.\n\n"
+            "Options:\n"
+            "  -i, --input <INPUT>    Input file path (FASTA/FASTQ by extension, optionally .gz; - = stdin)\n"
+            "  -o, --output <OUTPUT>  Output directory\n"
+            "  -k, --k-size <K_SIZE>  k-mer size, 10..=31\n"
+            "  -m, --memory <GB>      Accepted and ignored: the table lives in GPU memory\n"
+            "  -a, --acgt             Write each k-mer as k characters of ACGT instead of its code\n"
+            "  -t, --threads <N>      Threads formatting and writing the output 0=auto [default: 0]\n"
+            "      --device <N>       CUDA device ordinal [default: 0]\n"
+            "      --any-k            Accept any k in 1..=31\n"
+            "  -h, --help             Print help\n");
+}
+
+// `kmertools ctr`: batch-wide canonical k-mer counts (CountComputer)
+static int main_ctr(int argc, char **argv) {
+    ktb_file_opts o{};
+    std::string in, out;
+    o.k = 0; o.canonical = 1; o.delim = '\t'; o.device = 0;
+    int acgt = 0;
+    bool any_k = false, have_k = false;
+    for (int i = 2; i < argc; ++i) {
+        const std::string a = argv[i];
+        auto val = [&](const char *name) -> const char * {
+            if (i + 1 >= argc) { fprintf(stderr, "error: a value is required for '%s'\n", name); exit(2); }
+            return argv[++i];
+        };
+        if (a == "-i" || a == "--input") in = val("--input");
+        else if (a == "-o" || a == "--output") out = val("--output");
+        else if (a == "-k" || a == "--k-size") { o.k = atoi(val("--k-size")); have_k = true; }
+        else if (a == "-m" || a == "--memory") val("--memory");
+        else if (a == "-a" || a == "--acgt") acgt = 1;
+        else if (a == "-t" || a == "--threads") o.threads = atoi(val("--threads"));
+        else if (a == "--device") o.device = atoi(val("--device"));
+        else if (a == "--any-k") any_k = true;
+        else if (a == "-h" || a == "--help") { usage_ctr(); return 0; }
+        else { fprintf(stderr, "error: unexpected argument '%s' found\n", a.c_str()); usage_ctr(); return 2; }
+    }
+    if (in.empty() || out.empty() || !have_k) {
+        fprintf(stderr, "error: the following required arguments were not provided:\n%s%s%s", in.empty() ? "  --input <INPUT>\n" : "",
+                out.empty() ? "  --output <OUTPUT>\n" : "", have_k ? "" : "  --k-size <K_SIZE>\n");
+        return 2;
+    }
+    const int lo = any_k ? 1 : 10;
+    if (o.k < lo || o.k > 31) {
+        fprintf(stderr, "error: invalid value '%d' for '--k-size <K_SIZE>': %d is not in %d..=31\n", o.k, o.k, lo);
+        return 2;
+    }
+    o.in_path = in.c_str();
+    o.out_path = out.c_str();
+    ktb_file_stats st{};
+    if (ktb_count_file(&o, acgt, &st) != KTB_OK) {
+        fprintf(stderr, "Error: %s\n", ktb_last_error());   // exit 0, as for `comp oligo` (args.rs:260-262)
+        return 0;
+    }
+    if (getenv("KTB_VERBOSE"))
+        fprintf(stderr, "records %llu bases %llu written %llu B | parse %.1f ms add-wait %.1f ms write %.1f ms total %.1f ms\n",
+                (unsigned long long)st.records, (unsigned long long)st.bases, (unsigned long long)st.bytes_written,
+                st.parse_ms, st.gpu_wait_ms, st.write_ms, st.total_ms);
+    return 0;
+}
+
 int main(int argc, char **argv) {
+    if (argc >= 2 && !strcmp(argv[1], "ctr")) return main_ctr(argc, argv);
     if (argc >= 3 && !strcmp(argv[1], "comp") && !strcmp(argv[2], "cgr")) return main_cgr(argc, argv);
     if (argc < 3 || strcmp(argv[1], "comp") != 0 || strcmp(argv[2], "oligo") != 0) {
         if (argc >= 2 && (!strcmp(argv[1], "-h") || !strcmp(argv[1], "--help"))) { usage(); return 0; }
-        fprintf(stderr, "error: this build provides only `kmertools comp oligo` and `kmertools comp cgr -k` (GPU oligo path)\n");
+        fprintf(stderr, "error: this build provides only `kmertools comp oligo`, `kmertools comp cgr -k` and `kmertools ctr`\n");
         usage();
         return 2;
     }

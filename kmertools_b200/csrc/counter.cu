@@ -1,0 +1,326 @@
+// counter.cu — C ABI of batch-wide k-mer counting (ktb_counter_*): a table of (key, u64 count) in ascending key order
+// on one GPU, grown by adds of batches.  An add enqueues the kernels of count_kernels.cuh and waits for its stream once,
+// at the end, to learn the new table size.
+#include "count_kernels.cuh"
+#include "device_guard.h"
+#include "device_scan.cuh"
+
+#include <cuda_runtime.h>
+#include <stdint.h>
+#include <algorithm>
+#include <cstdio>
+#include <vector>
+
+using namespace ktb;
+
+struct ktb_counter {
+    int k = 0, canonical = 1, device = 0;
+    uint64_t *keys = nullptr, *counts = nullptr;   // the table (stream-ordered allocations)
+    uint64_t nkeys = 0, nwindows = 0;
+    unsigned long long *h_sizes = nullptr;         // page-locked [2]: valid windows and table keys of the last add
+};
+
+namespace {
+
+// bases of one chunk of the host entry point (a longer single sequence is a chunk of its own)
+constexpr uint64_t COUNT_CHUNK_BASES = 1ull << 26;
+
+int check_k(int k, int canonical) {
+    char msg[128];
+    if (k < 1 || k > KTB_MAX_SPARSE_K) {
+        snprintf(msg, sizeof msg, "k must be in 1..%d for the k-mer counter (got %d)", KTB_MAX_SPARSE_K, k);
+        return ktb_internal_fail(KTB_ERR_ARG, msg);
+    }
+    if (canonical != 0 && canonical != 1) return ktb_internal_fail(KTB_ERR_ARG, "canonical must be 0 or 1");
+    return KTB_OK;
+}
+
+// Enqueues the add of one batch (device buffers) on st and points the counter at the new table; the caller then waits
+// for st and takes the sizes from h_sizes (finish_add).  Nothing is enqueued when the scratch or the new table does not
+// fit: the counter is unchanged.
+int enqueue_add(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n, uint64_t total,
+                cudaStream_t st) {
+    const uint64_t nt_k = div_up(total, CT_T);               // key tiles
+    if (nt_k > 0x7fffffffull) return ktb_internal_fail(KTB_ERR_ARG, "batch too large for one add");
+    const uint64_t W = total;                                // bound of the valid windows
+    const uint64_t nt_r = div_up(W, RX_T);                   // radix tiles
+    const uint64_t nblk = div_up(W, SP_WB);                  // run-length blocks
+    const uint64_t space = c->k >= 31 ? ~0ull : (1ull << (2 * c->k));
+    const uint64_t ncap = c->nkeys + std::min(W, space);     // bound of the merged table
+    const uint64_t nbsum = div_up(std::max({nt_k, (uint64_t)RX_DIGITS * nt_r, nblk, W}), SP_WB);
+
+    int dev = 0, sms = 148;
+    CUP(cudaGetDevice(&dev));
+    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+
+    Carve s;
+    unsigned long long *tile_valid, *tile_base, *hist, *hoff, *bheads, *bbase, *R, *D, *bsum, *sizes;
+    uint64_t *X, *Y;
+    auto layout = [&] {
+        tile_valid = s.take<unsigned long long>(nt_k);
+        tile_base = s.take<unsigned long long>(nt_k + 1);
+        X = s.take<uint64_t>(W);
+        Y = s.take<uint64_t>(W);
+        hist = s.take<unsigned long long>(RX_DIGITS * nt_r);
+        hoff = s.take<unsigned long long>(RX_DIGITS * nt_r + 1);
+        bheads = s.take<unsigned long long>(nblk);
+        bbase = s.take<unsigned long long>(nblk + 1);
+        R = s.take<unsigned long long>(W);
+        D = s.take<unsigned long long>(W + 1);
+        bsum = s.take<unsigned long long>(nbsum);
+        sizes = s.take<unsigned long long>(2);
+    };
+    layout();   // sizes only
+    const size_t bytes = s.used;
+    uint64_t *okey = nullptr, *ocnt = nullptr;
+    {
+        cudaError_t e = cudaMallocAsync((void **)&s.base, bytes, st);
+        if (e == cudaSuccess) e = cudaMallocAsync((void **)&okey, std::max<uint64_t>(ncap, 1) * 8, st);
+        if (e == cudaSuccess) e = cudaMallocAsync((void **)&ocnt, std::max<uint64_t>(ncap, 1) * 8, st);
+        if (e != cudaSuccess) {
+            cudaFreeAsync(s.base, st);
+            cudaFreeAsync(okey, st);
+            cudaGetLastError();
+            return cuda_fail("cudaMallocAsync(counter scratch and table)", e);
+        }
+    }
+    s.used = 0;
+    layout();
+
+    int rc = KTB_OK;
+    auto step = [&](cudaError_t e, const char *what) {
+        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
+    };
+    // keys: count, scan, write
+    CountKeysParams kp{d_bases, d_offsets, n, (uint32_t)c->k, c->canonical, tile_valid, tile_base, X};
+    count_valid_kernel<<<(unsigned)nt_k, CT_THREADS, 0, st>>>(kp);
+    step(cudaGetLastError(), "count_valid_kernel");
+    if (rc == KTB_OK) rc = scan_u64(tile_valid, nt_k, tile_base, bsum, st);
+    if (rc == KTB_OK) {
+        count_keys_kernel<<<(unsigned)nt_k, CT_THREADS, 0, st>>>(kp);
+        step(cudaGetLastError(), "count_keys_kernel");
+    }
+    const unsigned long long *nkeys = tile_base + nt_k;
+    // sort: ceil(2k / 8) passes of 8 bits
+    uint64_t *in = X, *out = Y;
+    step(cudaFuncSetAttribute(count_scatter_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RX_SM_TOTAL),
+         "cudaFuncSetAttribute(count_scatter_kernel)");
+    for (uint32_t shift = 0; rc == KTB_OK && shift < 2u * (uint32_t)c->k; shift += 8) {
+        RadixParams rp{in, out, nkeys, nt_r, shift, hist, hoff};
+        count_upsweep_kernel<<<(unsigned)nt_r, RX_UTHREADS, 0, st>>>(rp);
+        step(cudaGetLastError(), "count_upsweep_kernel");
+        if (rc == KTB_OK) rc = scan_u64(hist, RX_DIGITS * nt_r, hoff, bsum, st);
+        if (rc == KTB_OK) {
+            count_scatter_kernel<<<(unsigned)nt_r, RX_THREADS, RX_SM_TOTAL, st>>>(rp);
+            step(cudaGetLastError(), "count_scatter_kernel");
+        }
+        std::swap(in, out);
+    }
+    // run-length encoding: runs' keys to `out`, head positions to R, counts to `in` (the sorted keys are done by then)
+    RleParams lp{in, nkeys, bheads, bbase, out, (uint64_t *)R};
+    const unsigned grid = (unsigned)std::min<uint64_t>(std::max<uint64_t>(div_up(W, SP_MTHREADS), 1), (uint64_t)sms * 16);
+    if (rc == KTB_OK) {
+        count_rle_heads_kernel<<<(unsigned)nblk, SP_MTHREADS, 0, st>>>(lp);
+        step(cudaGetLastError(), "count_rle_heads_kernel");
+    }
+    if (rc == KTB_OK) rc = scan_u64(bheads, nblk, bbase, bsum, st);
+    const unsigned long long *nruns = bbase + nblk;
+    if (rc == KTB_OK) {
+        count_rle_write_kernel<<<(unsigned)nblk, SP_MTHREADS, 0, st>>>(lp);
+        count_rle_len_kernel<<<grid, SP_MTHREADS, 0, st>>>((const uint64_t *)R, nruns, nkeys, in);
+        step(cudaGetLastError(), "count_rle_write_kernel / count_rle_len_kernel");
+    }
+    // merge into the table
+    MergeParams mp{c->keys, c->counts, c->nkeys, out, in, nruns, W, R, D, okey, ocnt, nkeys, sizes};
+    if (rc == KTB_OK) {
+        count_merge_dup_kernel<<<grid, SP_MTHREADS, 0, st>>>(mp);
+        step(cudaGetLastError(), "count_merge_dup_kernel");
+    }
+    if (rc == KTB_OK) rc = scan_u64(R, W, D, bsum, st);
+    if (rc == KTB_OK) {
+        const unsigned mgrid = (unsigned)std::min<uint64_t>(std::max<uint64_t>(div_up(c->nkeys + W, SP_MTHREADS), 1),
+                                                            (uint64_t)sms * 16);
+        count_merge_write_kernel<<<mgrid, SP_MTHREADS, 0, st>>>(mp);
+        step(cudaGetLastError(), "count_merge_write_kernel");
+    }
+    step(cudaMemcpyAsync(c->h_sizes, sizes, 2 * sizeof(uint64_t), cudaMemcpyDeviceToHost, st), "cudaMemcpyAsync(sizes)");
+    step(cudaFreeAsync(s.base, st), "cudaFreeAsync(scratch)");
+    if (rc != KTB_OK) {
+        cudaFreeAsync(okey, st);
+        cudaFreeAsync(ocnt, st);
+        return rc;
+    }
+    step(cudaFreeAsync(c->keys, st), "cudaFreeAsync(table)");
+    step(cudaFreeAsync(c->counts, st), "cudaFreeAsync(table)");
+    c->keys = okey;
+    c->counts = ocnt;
+    return rc;
+}
+
+int finish_add(ktb_counter *c, cudaStream_t st) {
+    CUP(cudaStreamSynchronize(st));
+    c->nwindows += c->h_sizes[0];
+    c->nkeys = c->h_sizes[1];
+    return KTB_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int ktb_counter_create(int k, int canonical, int device, ktb_counter **out) {
+    if (!out) return ktb_internal_fail(KTB_ERR_ARG, "out is NULL");
+    *out = nullptr;
+    if (int rc = check_k(k, canonical)) return rc;
+    if (device < 0) return ktb_internal_fail(KTB_ERR_ARG, "device out of range");
+    const int ndev = ktb_device_count();
+    if (ndev <= 0) return ktb_internal_fail(KTB_ERR_NODEVICE, "no CUDA device available (this library has no CPU path)");
+    if (device < 0 || device >= ndev) return ktb_internal_fail(KTB_ERR_ARG, "device out of range");
+    ktb::DeviceGuard device_guard(device);
+    CUP(device_guard.err);
+    ktb_counter *c = new ktb_counter();
+    c->k = k;
+    c->canonical = canonical;
+    c->device = device;
+    const cudaError_t e = cudaHostAlloc((void **)&c->h_sizes, 2 * sizeof(uint64_t), cudaHostAllocDefault);
+    if (e != cudaSuccess) {
+        delete c;
+        return cuda_fail("cudaHostAlloc(sizes)", e);
+    }
+    *out = c;
+    return KTB_OK;
+}
+
+void ktb_counter_destroy(ktb_counter *c) {
+    if (!c) return;
+    ktb::DeviceGuard device_guard(c->device);
+    cudaFree(c->keys);   // the adds that used the table have finished: every add waits for its stream
+    cudaFree(c->counts);
+    cudaFreeHost(c->h_sizes);
+    delete c;
+}
+
+int ktb_counter_add(ktb_counter *c, const uint8_t *bases, const uint64_t *offsets, uint64_t n) {
+    if (!c || !offsets) return ktb_internal_fail(KTB_ERR_ARG, "counter / offsets is NULL");
+    char msg[160];
+    for (uint64_t i = 0; i < n; ++i)
+        if (offsets[i + 1] < offsets[i]) {
+            snprintf(msg, sizeof msg, "offsets must be non-decreasing (at %llu)", (unsigned long long)i);
+            return ktb_internal_fail(KTB_ERR_ARG, msg);
+        }
+    if (offsets[n] > offsets[0] && !bases) return ktb_internal_fail(KTB_ERR_ARG, "bases is NULL");
+    if (n == 0 || offsets[n] == offsets[0]) return KTB_OK;
+    ktb::DeviceGuard device_guard(c->device);
+    CUP(device_guard.err);
+
+    // chunks of whole sequences, at most COUNT_CHUNK_BASES bases each unless one sequence is longer
+    std::vector<uint64_t> cut{0};
+    uint64_t max_bases = 0, max_n = 0;
+    for (uint64_t i0 = 0; i0 < n;) {
+        uint64_t i1 = i0 + 1;
+        while (i1 < n && offsets[i1 + 1] - offsets[i0] <= COUNT_CHUNK_BASES) ++i1;
+        max_bases = std::max(max_bases, offsets[i1] - offsets[i0]);
+        max_n = std::max(max_n, i1 - i0);
+        cut.push_back(i1);
+        i0 = i1;
+    }
+    // Two slots: chunk c + 1 is copied in on one stream while chunk c is counted and merged on the other.
+    struct Slot {
+        cudaStream_t st = nullptr;
+        uint8_t *bases = nullptr;
+        uint64_t *offsets = nullptr, *h_offsets = nullptr;
+    } slot[2];
+    int rc = KTB_OK;
+    auto step = [&](cudaError_t e, const char *what) {
+        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
+    };
+    for (Slot &s : slot) {
+        step(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking), "cudaStreamCreate");
+        step(cudaMalloc((void **)&s.bases, std::max<uint64_t>(max_bases, 1)), "cudaMalloc(bases)");
+        step(cudaMalloc((void **)&s.offsets, (max_n + 1) * sizeof(uint64_t)), "cudaMalloc(offsets)");
+        step(cudaHostAlloc((void **)&s.h_offsets, (max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
+             "cudaHostAlloc(offsets)");
+    }
+    const uint64_t nchunks = cut.size() - 1;
+    auto copy_in = [&](uint64_t ci) {
+        Slot &s = slot[ci & 1];
+        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, b0 = offsets[i0], nb = offsets[cut[ci + 1]] - b0;
+        for (uint64_t i = 0; i <= cn; ++i) s.h_offsets[i] = offsets[i0 + i] - b0;
+        if (nb) step(cudaMemcpyAsync(s.bases, bases + b0, nb, cudaMemcpyHostToDevice, s.st), "cudaMemcpyAsync(bases)");
+        step(cudaMemcpyAsync(s.offsets, s.h_offsets, (cn + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s.st),
+             "cudaMemcpyAsync(offsets)");
+    };
+    if (rc == KTB_OK) copy_in(0);
+    for (uint64_t ci = 0; ci < nchunks && rc == KTB_OK; ++ci) {
+        Slot &s = slot[ci & 1];
+        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, nb = offsets[cut[ci + 1]] - offsets[i0];
+        const bool work = nb > 0;
+        if (work) rc = enqueue_add(c, s.bases, s.offsets, cn, nb, s.st);
+        if (rc == KTB_OK && ci + 1 < nchunks) {   // the other slot's stream finished its chunk in the last iteration
+            copy_in(ci + 1);
+        }
+        if (rc == KTB_OK && work) rc = finish_add(c, s.st);
+    }
+    for (Slot &s : slot) {
+        if (s.st) step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");
+        cudaFree(s.bases);
+        cudaFree(s.offsets);
+        cudaFreeHost(s.h_offsets);
+        if (s.st) cudaStreamDestroy(s.st);
+    }
+    return rc;
+}
+
+int ktb_counter_add_device(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
+                           uint64_t total_bases, void *stream) {
+    if (!c || !d_offsets) return ktb_internal_fail(KTB_ERR_ARG, "counter / d_offsets is NULL");
+    if (total_bases > 0 && !d_bases) return ktb_internal_fail(KTB_ERR_ARG, "d_bases is NULL");
+    if (n == 0 || total_bases == 0) return KTB_OK;
+    ktb::DeviceGuard device_guard(c->device);
+    CUP(device_guard.err);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = enqueue_add(c, d_bases, d_offsets, n, total_bases, st)) {
+        cudaStreamSynchronize(st);
+        return rc;
+    }
+    return finish_add(c, st);
+}
+
+int ktb_counter_size(ktb_counter *c, uint64_t *nkeys, uint64_t *nwindows) {
+    if (!c) return ktb_internal_fail(KTB_ERR_ARG, "counter is NULL");
+    if (nkeys) *nkeys = c->nkeys;
+    if (nwindows) *nwindows = c->nwindows;
+    return KTB_OK;
+}
+
+int ktb_counter_read(ktb_counter *c, uint64_t *keys, uint64_t *counts, uint64_t cap) {
+    if (!c) return ktb_internal_fail(KTB_ERR_ARG, "counter is NULL");
+    const uint64_t m = std::min(c->nkeys, cap);
+    if (m == 0 || (!keys && !counts)) return KTB_OK;
+    ktb::DeviceGuard device_guard(c->device);
+    CUP(device_guard.err);
+    if (keys) CUP(cudaMemcpy(keys, c->keys, m * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    if (counts) CUP(cudaMemcpy(counts, c->counts, m * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+    return KTB_OK;
+}
+
+int ktb_counter_read_device(ktb_counter *c, uint64_t *d_keys, uint64_t *d_counts, uint64_t cap, void *stream) {
+    if (!c) return ktb_internal_fail(KTB_ERR_ARG, "counter is NULL");
+    const uint64_t m = std::min(c->nkeys, cap);
+    if (m == 0 || (!d_keys && !d_counts)) return KTB_OK;
+    ktb::DeviceGuard device_guard(c->device);
+    CUP(device_guard.err);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (d_keys) CUP(cudaMemcpyAsync(d_keys, c->keys, m * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+    if (d_counts) CUP(cudaMemcpyAsync(d_counts, c->counts, m * sizeof(uint64_t), cudaMemcpyDeviceToDevice, st));
+    return KTB_OK;
+}
+
+}  // extern "C"
+
+// The table in place, for the file driver's read-back in slices (file_api.cu).
+__attribute__((visibility("hidden"))) void ktb_internal_counter_table(const ktb_counter *c, const uint64_t **keys,
+                                                                       const uint64_t **counts) {
+    *keys = c->keys;
+    *counts = c->counts;
+}

@@ -16,6 +16,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <filesystem>
 #include <mutex>
 #include <string>
 #include <sched.h>
@@ -28,6 +29,7 @@ int ktb_internal_dispatch(ktb_oligo *h, const uint8_t *d_bases, const uint64_t *
 int ktb_internal_fail(int code, const char *msg);
 int ktb_internal_sms(const ktb_oligo *h);
 uint64_t ktb_internal_launches(const ktb_oligo *h);
+void ktb_internal_counter_table(const ktb_counter *c, const uint64_t **keys, const uint64_t **counts);
 
 namespace {
 
@@ -155,6 +157,47 @@ void release_sets(SetPair *sp) {
     delete old;
 }
 
+// `-t` (kmertools/src/args.rs:249-251; 0 = all cores): threads of the output writer and of the host formatter
+// (all cores = the CPUs this process may run on, at most 8: sixteen writer threads measured no faster on tmpfs —
+// 149 against 145 ms per GB, profiles/r2_cli_writer.txt — and write() on a disk file system uses one anyway)
+int host_threads(int threads) {
+    int hw = (int)std::max(1u, std::thread::hardware_concurrency());
+    cpu_set_t set;
+    CPU_ZERO(&set);
+    if (sched_getaffinity(0, sizeof(set), &set) == 0 && CPU_COUNT(&set) > 0) hw = CPU_COUNT(&set);
+    return threads > 0 ? std::min(threads, 64) : std::min(hw, 8);
+}
+
+// Bases per input batch: 32 MB, less for a small regular file (which should not page-lock 32 MB per buffer).
+size_t input_bases_cap(const std::string &in) {
+    size_t cap = 32u << 20;
+    struct stat sb;
+    if (in != "-" && stat(in.c_str(), &sb) == 0 && S_ISREG(sb.st_mode)) {
+        const bool gz = in.size() > 3 && in.compare(in.size() - 3, 3, ".gz") == 0;
+        const size_t est = (size_t)sb.st_size * (gz ? 8 : 1) + (1u << 20);
+        if (est < cap) cap = est;
+    }
+    return cap;
+}
+
+// Fills `bases` with the next batch of records (offs: its n + 1 offsets), growing the buffer and *cap when one record
+// does not fit.
+int fill_batch(ktb::FastxParser &parser, Pinned &bases, size_t *cap, size_t max_records, size_t *used,
+               std::vector<uint64_t> *offs) {
+    offs->assign(1, 0);
+    *used = 0;
+    for (;;) {
+        const long got = parser.fill((uint8_t *)bases.p, bases.cap, used, offs, max_records);
+        if (got < 0) return ktb_internal_fail(KTB_ERR_IO, parser.error().c_str());
+        if (got == 0 && parser.need_bytes() && *used == 0) {  // one record larger than the buffer
+            *cap = parser.need_bytes() + (parser.need_bytes() >> 2) + 4096;
+            if (!bases.grow_keep(*cap, 0)) return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
+            continue;
+        }
+        return KTB_OK;
+    }
+}
+
 // u32 counts of rows [r0, r1) -> "c0<d>c1<d>...\n" (format!("{}", f64) prints integral values without ".0", oligo.rs:138)
 void format_counts_rows(const uint32_t *counts, uint64_t r0, uint64_t r1, uint32_t dim, char delim, Text *out) {
     out->resize((size_t)(r1 - r0) * dim * 11 + 16);
@@ -251,6 +294,25 @@ bool format_cgr_rows(const void *rows, bool norm, uint64_t r0, uint64_t r1, uint
     }
     out->resize((size_t)(o - out->data()));
     return true;
+}
+
+// table entries [r0, r1) -> "<code>\t<count>\n", the code in decimal or (acgt) as k characters of ACGT
+void format_count_lines(const uint64_t *keys, const uint64_t *counts, uint64_t r0, uint64_t r1, int k, bool acgt,
+                        Text *out) {
+    out->resize((size_t)(r1 - r0) * ((acgt ? (size_t)k : 20) + 22));
+    char *o = out->data();
+    for (uint64_t i = r0; i < r1; ++i) {
+        if (acgt) {
+            for (int j = 0; j < k; ++j) o[j] = "ACGT"[(keys[i] >> (2 * (k - 1 - j))) & 3u];
+            o += k;
+        } else {
+            o = std::to_chars(o, o + 20, keys[i]).ptr;
+        }
+        *o++ = '\t';
+        o = std::to_chars(o, o + 20, counts[i]).ptr;
+        *o++ = '\n';
+    }
+    out->resize((size_t)(o - out->data()));
 }
 
 }  // namespace
@@ -383,16 +445,7 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
     if (device_guard.err != cudaSuccess) return ktb_internal_fail(KTB_ERR_CUDA, "cudaSetDevice failed");
     const uint64_t dim = ktb_oligo_dim(h, cgr ? 1 : o->canonical);
 
-    // `-t` (kmertools/src/args.rs:249-251; 0 = all cores): threads of the output writer and of the host formatter
-    // (all cores = the CPUs this process may run on, at most 8: sixteen writer threads measured no faster on tmpfs —
-    // 149 against 145 ms per GB, profiles/r2_cli_writer.txt — and write() on a disk file system uses one anyway)
-    int hw = (int)std::max(1u, std::thread::hardware_concurrency());
-    {
-        cpu_set_t set;
-        CPU_ZERO(&set);
-        if (sched_getaffinity(0, sizeof(set), &set) == 0 && CPU_COUNT(&set) > 0) hw = CPU_COUNT(&set);
-    }
-    const int nthreads = o->threads > 0 ? std::min(o->threads, 64) : std::min(hw, 8);
+    const int nthreads = host_threads(o->threads);
     ktb::SpanWriter wr;
     if (!wr.open(o->out_path, nthreads, &err)) return ktb_internal_fail(KTB_ERR_IO, err.c_str());
     ktb::SpanWriter::Ticket header_ticket;
@@ -424,15 +477,7 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
     // inode lock); the writer now copies spans through a shared mapping instead, which does not.
     const size_t OUT_CAP = 64u << 20;
     const size_t max_records = std::max<size_t>(1, std::min<size_t>(OUT_CAP / out_per_row, 4u << 20));
-    size_t bases_cap = 32u << 20;
-    {   // small inputs should not page-lock 32 MB per buffer set
-        struct stat sb;
-        if (in != "-" && stat(in.c_str(), &sb) == 0 && S_ISREG(sb.st_mode)) {
-            const bool gz = in.size() > 3 && in.compare(in.size() - 3, 3, ".gz") == 0;
-            const size_t est = (size_t)sb.st_size * (gz ? 8 : 1) + (1u << 20);
-            if (est < bases_cap) bases_cap = est;
-        }
-    }
+    size_t bases_cap = input_bases_cap(in);
 
     SetPair *pair = acquire_sets(o->device);
     if (!pair) return ktb_internal_fail(KTB_ERR_CUDA, "cudaStreamCreate failed");
@@ -496,19 +541,8 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
         if (!s.h_bases.ensure(bases_cap)) return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
         const double tp0 = now_ms();
         alloc_ms += tp0 - ta0;
-        offs.assign(1, 0);
         size_t used = 0;
-        long got = 0;
-        for (;;) {
-            got = parser.fill((uint8_t *)s.h_bases.p, s.h_bases.cap, &used, &offs, max_records);
-            if (got < 0) return ktb_internal_fail(KTB_ERR_IO, parser.error().c_str());
-            if (got == 0 && parser.need_bytes() && used == 0) {  // one record larger than the buffer
-                bases_cap = parser.need_bytes() + (parser.need_bytes() >> 2) + 4096;
-                if (!s.h_bases.grow_keep(bases_cap, 0)) return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
-                continue;
-            }
-            break;
-        }
+        if (int rc = fill_batch(parser, s.h_bases, &bases_cap, max_records, &used, &offs)) return rc;
         st.parse_ms += now_ms() - tp0;
         const uint64_t n = offs.size() - 1;
         if (n == 0) break;
@@ -597,6 +631,127 @@ void ktb_release_cached_buffers(void) {
 int ktb_comp_cgr_file(const ktb_file_opts *o, int vecsize, ktb_file_stats *stats) {
     if (vecsize < 1) return ktb_internal_fail(KTB_ERR_ARG, "vecsize must be positive");
     return run_file(o, stats, vecsize);
+}
+
+int ktb_count_file(const ktb_file_opts *o, int acgt, ktb_file_stats *stats) {
+    const double t_start = now_ms();
+    if (!o || !o->in_path || !o->out_path) return ktb_internal_fail(KTB_ERR_ARG, "null argument");
+    ktb_file_stats st{};
+    const std::string in = o->in_path;
+    ktb::ByteSource src;
+    std::string err;
+    if (!src.open(in, &err)) return ktb_internal_fail(KTB_ERR_IO, err.c_str());
+    ktb::SeqFormat fmt;
+    if (in == "-") fmt = (src.peek_first_byte() == '>') ? ktb::SeqFormat::Fasta : ktb::SeqFormat::Fastq;
+    else if (!ktb::format_from_path(in, &fmt))
+        return ktb_internal_fail(KTB_ERR_IO, "unknown sequence file extension (expected .fa/.fasta/.fna/.fq/.fastq[.gz])");
+    ktb::FastxParser parser(&src, fmt);
+
+    ktb_counter *c = nullptr;
+    if (int rc = ktb_counter_create(o->k, 1, o->device, &c)) return rc;
+    struct Guard { ktb_counter *c; ~Guard() { ktb_counter_destroy(c); } } guard{c};
+    ktb::DeviceGuard device_guard(o->device);   // page-locked buffers and the read-back stream belong to this device
+    if (device_guard.err != cudaSuccess) return ktb_internal_fail(KTB_ERR_CUDA, "cudaSetDevice failed");
+    std::error_code ec;
+    std::filesystem::create_directories(o->out_path, ec);
+    if (ec) return ktb_internal_fail(KTB_ERR_IO, ("cannot create the output directory: " + ec.message()).c_str());
+    const std::string out_file = std::string(o->out_path) + "/kmers.counts";
+    const int nthreads = host_threads(o->threads);
+
+    // ---- count: batch b is added on a worker thread while the caller parses batch b + 1 into the other buffer
+    Pinned hbases[2];
+    std::vector<uint64_t> offs[2];
+    size_t bases_cap = input_bases_cap(in);
+    const size_t max_records = 4u << 20;
+    std::thread adder;
+    int add_rc = KTB_OK;
+    std::string add_err;
+    auto join = [&]() -> int {
+        if (!adder.joinable()) return KTB_OK;
+        const double t0 = now_ms();
+        adder.join();
+        st.gpu_wait_ms += now_ms() - t0;
+        return add_rc ? ktb_internal_fail(add_rc, add_err.c_str()) : KTB_OK;
+    };
+    struct JoinGuard { std::thread *t; ~JoinGuard() { if (t->joinable()) t->join(); } } join_guard{&adder};
+    for (int b = 0;; ++b) {
+        Pinned &hb = hbases[b & 1];
+        std::vector<uint64_t> &of = offs[b & 1];
+        const double tp0 = now_ms();
+        if (!hb.ensure(bases_cap)) return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
+        size_t used = 0;
+        if (int rc = fill_batch(parser, hb, &bases_cap, max_records, &used, &of)) return rc;
+        st.parse_ms += now_ms() - tp0;
+        if (int rc = join()) return rc;
+        const uint64_t n = of.size() - 1;
+        if (n == 0) break;
+        st.records += n;
+        st.bases += used;
+        adder = std::thread([&, n, b] {
+            add_rc = ktb_counter_add(c, (const uint8_t *)hbases[b & 1].p, offs[b & 1].data(), n);
+            if (add_rc) add_err = ktb_last_error();
+        });
+        if (parser.eof()) break;
+    }
+    if (int rc = join()) return rc;
+
+    // ---- write: slices of the table through page-locked staging (slice s + 1 is copied while slice s is formatted)
+    const double tw0 = now_ms();
+    uint64_t nkeys = 0;
+    ktb_counter_size(c, &nkeys, nullptr);
+    const uint64_t *d_keys, *d_counts;
+    ktb_internal_counter_table(c, &d_keys, &d_counts);
+    ktb::SpanWriter wr;
+    if (!wr.open(out_file.c_str(), nthreads, &err)) return ktb_internal_fail(KTB_ERR_IO, err.c_str());
+    const uint64_t SLICE = 1u << 22;
+    struct Slice {
+        Pinned keys, counts;
+        std::vector<Text> parts;
+        ktb::SpanWriter::Ticket ticket;
+        bool writing = false;
+    } sl[2];
+    // on every exit the writer threads stop before the text they read goes away
+    struct WriterGuard { ktb::SpanWriter *w; ~WriterGuard() { w->close(); } } writer_guard{&wr};
+    cudaStream_t st_copy = nullptr;
+    if (cudaStreamCreateWithFlags(&st_copy, cudaStreamNonBlocking) != cudaSuccess)
+        return ktb_internal_fail(KTB_ERR_CUDA, "cudaStreamCreate failed");
+    struct StreamGuard { cudaStream_t s; ~StreamGuard() { cudaStreamSynchronize(s); cudaStreamDestroy(s); } } stream_guard{st_copy};
+    const uint64_t nslices = (nkeys + SLICE - 1) / SLICE;
+    auto copy_out = [&](uint64_t si) -> int {
+        Slice &x = sl[si & 1];
+        const uint64_t a = si * SLICE, m = std::min(SLICE, nkeys - a);
+        if (!x.keys.ensure(std::min(SLICE, nkeys) * 8) || !x.counts.ensure(std::min(SLICE, nkeys) * 8))
+            return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
+        if (cudaMemcpyAsync(x.keys.p, d_keys + a, m * 8, cudaMemcpyDeviceToHost, st_copy) != cudaSuccess ||
+            cudaMemcpyAsync(x.counts.p, d_counts + a, m * 8, cudaMemcpyDeviceToHost, st_copy) != cudaSuccess)
+            return ktb_internal_fail(KTB_ERR_CUDA, "cudaMemcpyAsync(table slice) failed");
+        return KTB_OK;
+    };
+    if (nslices)
+        if (int rc = copy_out(0)) return rc;
+    for (uint64_t si = 0; si < nslices; ++si) {
+        Slice &x = sl[si & 1];
+        if (cudaStreamSynchronize(st_copy) != cudaSuccess)
+            return ktb_internal_fail(KTB_ERR_CUDA, cudaGetErrorString(cudaGetLastError()));
+        if (si + 1 < nslices)   // the other slice's staging was formatted in the previous iteration
+            if (int rc = copy_out(si + 1)) return rc;
+        if (x.writing && !wr.wait(&x.ticket)) return ktb_internal_fail(KTB_ERR_IO, "write to the output file failed");
+        const uint64_t m = std::min(SLICE, nkeys - si * SLICE);
+        const uint64_t *keys = (const uint64_t *)x.keys.p, *counts = (const uint64_t *)x.counts.p;
+        format_parallel(m, nthreads, &x.parts, [&](uint64_t r0, uint64_t r1, Text *part) {
+            format_count_lines(keys, counts, r0, r1, o->k, acgt != 0, part);
+        });
+        for (auto &part : x.parts) wr.submit(part.data(), part.size(), &x.ticket);
+        x.writing = true;
+    }
+    for (Slice &x : sl)
+        if (x.writing && !wr.wait(&x.ticket)) return ktb_internal_fail(KTB_ERR_IO, "write to the output file failed");
+    st.bytes_written = wr.bytes();
+    if (!wr.close()) return ktb_internal_fail(KTB_ERR_IO, "closing the output file failed");
+    st.write_ms = now_ms() - tw0;
+    st.total_ms = now_ms() - t_start;
+    if (stats) *stats = st;
+    return KTB_OK;
 }
 
 }  // extern "C"

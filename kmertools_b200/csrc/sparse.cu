@@ -1,8 +1,8 @@
 // sparse.cu — C ABI of the sparse per-sequence k-mer count rows (CSR): ktb_sparse_vectorise_device enqueues the
 // kernels of sparse_kernels.cuh; ktb_sparse_vectorise runs it over host buffers in chunks of sequences.
 #include "device_guard.h"
+#include "device_scan.cuh"
 #include "sparse_kernels.cuh"
-#include "../../include/kmertools_b200.h"
 
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -10,26 +10,12 @@
 #include <cstdio>
 #include <vector>
 
-int ktb_internal_fail(int code, const char *msg);
-
 namespace {
 
 using namespace ktb;
 
 // bases of one chunk of the host entry point (a longer single sequence is a chunk of its own)
 constexpr uint64_t SPARSE_CHUNK_BASES = 1ull << 26;
-
-int cuda_fail(const char *what, cudaError_t e) {
-    char msg[256];
-    snprintf(msg, sizeof msg, "%s failed: %s", what, cudaGetErrorString(e));
-    return ktb_internal_fail(e == cudaErrorMemoryAllocation ? KTB_ERR_NOMEM : KTB_ERR_CUDA, msg);
-}
-
-#define CUP(call)                                           \
-    do {                                                    \
-        cudaError_t e_ = (call);                            \
-        if (e_ != cudaSuccess) return cuda_fail(#call, e_); \
-    } while (0)
 
 int check_args(int k, int canonical, int norm_mode, int out_dtype) {
     char msg[128];
@@ -45,11 +31,11 @@ int check_args(int k, int canonical, int norm_mode, int out_dtype) {
     return KTB_OK;
 }
 
-uint64_t div_up(uint64_t a, uint64_t b) { return (a + b - 1) / b; }
+}  // namespace
 
-// exclusive scan of in[0..n) into out[0..n], bsum: div_up(n, SP_WB) entries
-int scan_u64(const unsigned long long *in, uint64_t n, unsigned long long *out, unsigned long long *bsum,
-             cudaStream_t st) {
+__attribute__((visibility("hidden"))) int ktb::scan_u64(const unsigned long long *in, uint64_t n,
+                                                         unsigned long long *out, unsigned long long *bsum,
+                                                         cudaStream_t st) {
     if (n == 0) {
         CUP(cudaMemsetAsync(out, 0, sizeof(uint64_t), st));
         return KTB_OK;
@@ -61,19 +47,6 @@ int scan_u64(const unsigned long long *in, uint64_t n, unsigned long long *out, 
     CUP(cudaGetLastError());
     return KTB_OK;
 }
-
-// bump allocator over one stream-ordered allocation
-struct Carve {
-    char *base = nullptr;
-    size_t used = 0;
-    template <typename T> T *take(uint64_t count) {
-        T *p = reinterpret_cast<T *>(base ? base + used : nullptr);
-        used += (count * sizeof(T) + 255) & ~(size_t)255;
-        return p;
-    }
-};
-
-}  // namespace
 
 int ktb_sparse_vectorise_device(const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n, uint64_t total_bases,
                                 int k, int canonical, int norm_mode, int out_dtype, uint64_t *d_row_ptr,
