@@ -178,8 +178,10 @@ int ktb_sparse_vectorise_device(const uint8_t *d_bases, const uint64_t *d_offset
  * The table lives on the counter's device: 16 bytes per distinct key.  An add also needs scratch from the
  * stream-ordered allocator: 33 bytes per base of the batch (per base of total_bases for a device add; per base of a
  * chunk for a host add) plus, while the merge runs, the new table: 16 bytes per distinct key of the old table plus
- * 16 bytes per base (at most 16 * 4^k in all).  A table or scratch that does not fit device memory is KTB_ERR_NOMEM
- * and leaves the counter as it was; nothing spills to the host or to disk.
+ * 16 bytes per base (at most 16 * 4^k in all).  A host add of more than one chunk also holds the table it started
+ * from, 16 bytes per key of it, until it returns.  A table or scratch that does not fit device memory is KTB_ERR_NOMEM
+ * and leaves the counter as it was (a host add restores the table it started from, so none of the batch is counted);
+ * nothing spills to the host or to disk.
  * Every add returns when the batch is in the table: it waits for its stream once, at the end, to learn the new table
  * size.  Calls on ONE counter must be ordered by the caller; different counters are independent. */
 typedef struct ktb_counter ktb_counter;
@@ -212,7 +214,8 @@ int ktb_counter_size(ktb_counter *c, uint64_t *nkeys, uint64_t *nwindows);
 int ktb_counter_read(ktb_counter *c, uint64_t *keys, uint64_t *counts, uint64_t cap);
 
 /* Same into DEVICE memory of the counter's device: device-to-device copies enqueued on `stream`, returns after
- * enqueueing.  The copies read the table in place, so the next add on the counter must be ordered after them. */
+ * enqueueing.  The copies read the table in place, so the next add on the counter must be ordered after them: a
+ * device add by its stream, a host add (which runs on streams of its own) by waiting for the copies on the host. */
 int ktb_counter_read_device(ktb_counter *c, uint64_t *d_keys, uint64_t *d_counts, uint64_t cap, void *stream);
 
 /* Stats of the most recent vectorise call (host entry point: complete; device entry point: launch

@@ -24,6 +24,7 @@ class KmerCounter:
         self.mins = bool(mins)
         self.device = int(device)
         self._h = C.c_void_p()
+        self._read = None   # CUDA event after the copies of the last result_tensors: the next add waits for it
         _lib.check(_lib.load().ktb_counter_create(self.ksize, int(self.mins), self.device, C.byref(self._h)))
 
     def _handle(self):
@@ -32,16 +33,21 @@ class KmerCounter:
         return self._h
 
     def add(self, seqs_or_packed) -> None:
-        """Counts a list of str / bytes, or a packed (bases u8, offsets u64[n+1]) pair, from host memory."""
+        """Counts a list of str / bytes, or a packed (bases u8, offsets u64[n+1]) pair, from host memory.  Waits on the
+        host for the copies of an earlier result_tensors, which read the table this add replaces."""
         bases, offsets = _packed(seqs_or_packed)
         n = len(offsets) - 1
+        if self._read is not None:
+            self._read.synchronize()
+            self._read = None
         _lib.check(_lib.load().ktb_counter_add(self._handle(), bases.ctypes.data if bases.size else None,
                                                offsets.ctypes.data, max(n, 0)))
 
     def add_tensors(self, bases, offsets) -> None:
         """Counts CUDA tensors on the counter's device, on torch's current stream: `bases` uint8, `offsets` int64 (n+1,
         absolute positions in `bases`).  The scratch is sized from bases.numel(): for a small batch inside a large
-        buffer, pass the slice bases[offsets[0]:offsets[n]] and offsets - offsets[0]."""
+        buffer, pass the slice bases[offsets[0]:offsets[n]] and offsets - offsets[0].  The current stream first waits
+        for the copies of an earlier result_tensors, which read the table this add replaces."""
         import torch
         if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
             raise ValueError("bases and offsets must be CUDA tensors on one device")
@@ -54,7 +60,10 @@ class KmerCounter:
         n = offsets.numel() - 1
         total = bases.numel()
         with torch.cuda.device(bases.device):
-            stream = torch.cuda.current_stream(bases.device).cuda_stream
+            current = torch.cuda.current_stream(bases.device)
+            if self._read is not None:
+                current.wait_event(self._read)
+            stream = current.cuda_stream
             _lib.check(_lib.load().ktb_counter_add_device(self._handle(), bases.data_ptr() if total else None,
                                                           offsets.data_ptr(), max(n, 0), total, stream))
 
@@ -81,7 +90,8 @@ class KmerCounter:
         return keys, counts
 
     def result_tensors(self):
-        """(keys, counts) as int64 CUDA tensors on the counter's device, copied on torch's current stream."""
+        """(keys, counts) as int64 CUDA tensors on the counter's device, copied on torch's current stream.  The copies
+        read the table in place; the next add or add_tensors waits for them, so the tensors hold this table."""
         import torch
         n = len(self)
         dev = torch.device("cuda", self.device)
@@ -91,6 +101,9 @@ class KmerCounter:
             stream = torch.cuda.current_stream(dev).cuda_stream
             _lib.check(_lib.load().ktb_counter_read_device(self._handle(), keys.data_ptr() if n else None,
                                                            counts.data_ptr() if n else None, n, stream))
+            if n:
+                self._read = torch.cuda.Event()
+                self._read.record()
         return keys, counts
 
     def close(self) -> None:

@@ -37,9 +37,9 @@ int check_k(int k, int canonical) {
 
 // Enqueues the add of one batch (device buffers) on st and points the counter at the new table; the caller then waits
 // for st and takes the sizes from h_sizes (finish_add).  Nothing is enqueued when the scratch or the new table does not
-// fit: the counter is unchanged.
+// fit: the counter is unchanged.  free_old = false leaves the old table allocated: the caller owns it from then on.
 int enqueue_add(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n, uint64_t total,
-                cudaStream_t st) {
+                cudaStream_t st, bool free_old = true) {
     const uint64_t nt_k = div_up(total, CT_T);               // key tiles
     if (nt_k > 0x7fffffffull) return ktb_internal_fail(KTB_ERR_ARG, "batch too large for one add");
     const uint64_t W = total;                                // bound of the valid windows
@@ -150,8 +150,10 @@ int enqueue_add(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offset
         cudaFreeAsync(ocnt, st);
         return rc;
     }
-    step(cudaFreeAsync(c->keys, st), "cudaFreeAsync(table)");
-    step(cudaFreeAsync(c->counts, st), "cudaFreeAsync(table)");
+    if (free_old) {
+        step(cudaFreeAsync(c->keys, st), "cudaFreeAsync(table)");
+        step(cudaFreeAsync(c->counts, st), "cudaFreeAsync(table)");
+    }
     c->keys = okey;
     c->counts = ocnt;
     return rc;
@@ -242,6 +244,10 @@ int ktb_counter_add(ktb_counter *c, const uint8_t *bases, const uint64_t *offset
              "cudaHostAlloc(offsets)");
     }
     const uint64_t nchunks = cut.size() - 1;
+    // Over several chunks, the table the add started from is kept until the add returns, so that a chunk that fails
+    // (a scratch that does not fit) can restore it: the counter then holds none of the batch, not part of it.
+    const ktb_counter saved = *c;
+    const bool keep = nchunks > 1;
     auto copy_in = [&](uint64_t ci) {
         Slot &s = slot[ci & 1];
         const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, b0 = offsets[i0], nb = offsets[cut[ci + 1]] - b0;
@@ -255,7 +261,7 @@ int ktb_counter_add(ktb_counter *c, const uint8_t *bases, const uint64_t *offset
         Slot &s = slot[ci & 1];
         const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, nb = offsets[cut[ci + 1]] - offsets[i0];
         const bool work = nb > 0;
-        if (work) rc = enqueue_add(c, s.bases, s.offsets, cn, nb, s.st);
+        if (work) rc = enqueue_add(c, s.bases, s.offsets, cn, nb, s.st, !(keep && c->keys == saved.keys));
         if (rc == KTB_OK && ci + 1 < nchunks) {   // the other slot's stream finished its chunk in the last iteration
             copy_in(ci + 1);
         }
@@ -267,6 +273,19 @@ int ktb_counter_add(ktb_counter *c, const uint8_t *bases, const uint64_t *offset
         cudaFree(s.offsets);
         cudaFreeHost(s.h_offsets);
         if (s.st) cudaStreamDestroy(s.st);
+    }
+    if (keep && c->keys != saved.keys) {   // the streams are idle: nothing reads either table any more
+        if (rc == KTB_OK) {
+            cudaFree(saved.keys);
+            cudaFree(saved.counts);
+        } else {
+            cudaFree(c->keys);
+            cudaFree(c->counts);
+            c->keys = saved.keys;
+            c->counts = saved.counts;
+            c->nkeys = saved.nkeys;
+            c->nwindows = saved.nwindows;
+        }
     }
     return rc;
 }
