@@ -218,6 +218,42 @@ int ktb_counter_read(ktb_counter *c, uint64_t *keys, uint64_t *counts, uint64_t 
  * device add by its stream, a host add (which runs on streams of its own) by waiting for the copies on the host. */
 int ktb_counter_read_device(ktb_counter *c, uint64_t *d_keys, uint64_t *d_counts, uint64_t cap, void *stream);
 
+/* ---- per-read k-mer coverage histograms against a counter's table ---------------------------------------------
+ * This build's own semantics (the reference's coverage tool is not reproduced).  For every sequence s of a batch and
+ * every valid window of s (same decoding, validity and keys as the counter's adds: canonical or raw after the counter),
+ * the window's abundance is a = the key's count in the table, or 0 when the key is absent (a table built from other
+ * data).  Its bin is min(floor(a / bin_size), bin_count - 1), with a as u64.  Row s is the histogram of the bins of its
+ * windows: bin_count u32 counts that sum to totals[s], the valid windows of s.  KTB_NORM_CLI divides each count by
+ * max(1, totals[s]) exactly as the dense rows do (f64 the IEEE quotient, f32 that quotient rounded once);
+ * KTB_NORM_COUNTS gives the counts (KTB_OUT_U32 needs it); KTB_NORM_PY is KTB_ERR_ARG.  Empty sequences, sequences
+ * shorter than k and all-ambiguous ones give all-zero rows with total 0.  1 <= bin_size, 1 <= bin_count <= 65536; a
+ * sequence must have fewer than 2^32 windows.  Arguments are checked before any device work.
+ *
+ * Lookups go through a directory over the top b bits of the 2k-bit key, b = floor(log2(distinct keys)) capped at 2k
+ * (a direct index) and at 30: 8 * (2^b + 1) bytes on the counter's device, about half the table at most.  The first coverage call after an add
+ * (or on a fresh counter) builds it and waits for its stream once; later calls only enqueue.  The next add frees it, as
+ * does ktb_counter_destroy.  Each window then binary-searches one bucket of at most 2^(2k-b) keys.
+ * Scratch: none per base; 4 bytes per row element with KTB_OUT_F64 (4-byte outputs are counted in place).  A directory
+ * or scratch that does not fit device memory is KTB_ERR_NOMEM and leaves the counter usable. */
+
+/* HOST buffers, layout of ktb_counter_add; chunks of whole sequences (about 2^26 bases each) on two streams, chunk c + 1
+ * copied in and computed while the rows of chunk c are copied out.  out: n x bin_count row-major of out_dtype; totals
+ * may be NULL (out too when n = 0).  Synchronous; a sequence with 2^32 or more windows is KTB_ERR_ARG. */
+int ktb_counter_coverage(ktb_counter *c, const uint8_t *bases, const uint64_t *offsets, uint64_t n,
+                         uint32_t bin_size, uint32_t bin_count, int norm_mode, int out_dtype,
+                         void *out, uint64_t *totals);
+
+/* DEVICE buffers on the counter's device, enqueued on `stream`; returns after enqueueing (after the directory build,
+ * which waits for `stream`, on the first call after an add).  Offsets are absolute, total_bases >= offsets[n] as in
+ * ktb_counter_add_device.  d_out (n x bin_count) and d_totals (n, may be NULL) are always complete.  The kernels read
+ * the table and the directory in place, so the next add on the counter must be ordered after them: a device add by its
+ * stream, a host add by waiting for them on the host (as for ktb_counter_read_device).  Once the directory exists a
+ * coverage call changes nothing in the counter, so such calls may run concurrently on several streams.  Precondition:
+ * every sequence has fewer than 2^32 windows. */
+int ktb_counter_coverage_device(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
+                                uint64_t total_bases, uint32_t bin_size, uint32_t bin_count, int norm_mode,
+                                int out_dtype, void *d_out, uint64_t *d_totals, void *stream);
+
 /* Stats of the most recent vectorise call (host entry point: complete; device entry point: launch
  * counts and class sizes only). */
 int ktb_oligo_last_stats(const ktb_oligo *h, ktb_stats *out);
@@ -331,6 +367,15 @@ int ktb_comp_cgr_file(const ktb_file_opts *opts, int vecsize, ktb_file_stats *st
  * the k-mer as k characters of ACGT (first base first).  The table is read back in slices through page-locked staging
  * and formatted by `threads` host threads.  stats->bases counts the bases parsed, stats->bytes_written the text. */
 int ktb_count_file(const ktb_file_opts *opts, int acgt, ktb_file_stats *stats /* optional */);
+
+/* `kmertools cov`: counts the canonical k-mers of count_path (NULL = in_path) into a counter, then writes one line per
+ * record of in_path: the record's coverage histogram (ktb_counter_coverage, KTB_NORM_CLI), bin_count values "{:.6}"
+ * joined by ' ', '\n'-terminated, in input order.  Uses in_path, out_path, k, threads, device of opts.  Both inputs
+ * follow ktb_count_file's format rule; in_path "-" (stdin) needs a count_path other than "-", since the input would be
+ * read twice.  k, bin_size, bin_count and that rule are checked before any device work.  The line form is this build's
+ * own.  stats describe the second pass (records and bases of in_path). */
+int ktb_coverage_file(const ktb_file_opts *opts, const char *count_path, uint32_t bin_size, uint32_t bin_count,
+                      ktb_file_stats *stats /* optional */);
 
 /* The file-level drivers keep their pinned / device buffer sets (at most ~0.5 GB) for the next call on the same
  * device; this frees them. */

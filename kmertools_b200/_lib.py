@@ -64,7 +64,10 @@ SYMBOLS = {
     "ktb_counter_size": (_I, [_VP, C.POINTER(_U64), C.POINTER(_U64)]),
     "ktb_counter_read": (_I, [_VP, _VP, _VP, _U64]),
     "ktb_counter_read_device": (_I, [_VP, _VP, _VP, _U64, _VP]),
+    "ktb_counter_coverage": (_I, [_VP, _VP, _VP, _U64, C.c_uint32, C.c_uint32, _I, _I, _VP, _VP]),
+    "ktb_counter_coverage_device": (_I, [_VP, _VP, _VP, _U64, _U64, C.c_uint32, C.c_uint32, _I, _I, _VP, _VP, _VP]),
     "ktb_count_file": (_I, [C.POINTER(FileOpts), _I, C.POINTER(FileStats)]),
+    "ktb_coverage_file": (_I, [C.POINTER(FileOpts), C.c_char_p, C.c_uint32, C.c_uint32, C.POINTER(FileStats)]),
     "ktb_oligo_last_stats": (_I, [_VP, C.POINTER(Stats)]),
     "ktb_oligo_set_option": (_I, [_VP, C.c_char_p, C.c_int64]),
     "ktb_host_alloc": (_VP, [_SZ]),

@@ -4,6 +4,10 @@ A KmerCounter keeps one table on its GPU: every distinct key seen so far (canoni
 raw: forward) in ascending order, with a u64 count of its windows.  Keys are 2-bit codes (A=0 C=1 G=2 T=3, first base
 most significant), as kmer_pairs and kmer_counts return them.  The table does not depend on how the input is split
 into adds or on their order.
+
+coverage / coverage_tensors look every window of a batch up in that table and return per-sequence histograms of the
+abundances (this build's own semantics, include/kmertools_b200.h): bin min(a // bin_size, bin_count - 1) of a window
+whose key has count a (0 when absent), rows normalised by the sequence's valid windows or as u32 counts.
 """
 from __future__ import annotations
 
@@ -49,14 +53,7 @@ class KmerCounter:
         buffer, pass the slice bases[offsets[0]:offsets[n]] and offsets - offsets[0].  The current stream first waits
         for the copies of an earlier result_tensors, which read the table this add replaces."""
         import torch
-        if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
-            raise ValueError("bases and offsets must be CUDA tensors on one device")
-        if bases.device.index != self.device:
-            raise ValueError(f"the tensors are on {bases.device}, the counter on cuda:{self.device}")
-        if bases.dtype != torch.uint8 or offsets.dtype != torch.int64:
-            raise TypeError(f"bases must be uint8 and offsets int64 (got {bases.dtype}, {offsets.dtype})")
-        if not (bases.is_contiguous() and offsets.is_contiguous()):
-            raise ValueError("bases and offsets must be contiguous")
+        self._check_tensors(bases, offsets)
         n = offsets.numel() - 1
         total = bases.numel()
         with torch.cuda.device(bases.device):
@@ -66,6 +63,17 @@ class KmerCounter:
             stream = current.cuda_stream
             _lib.check(_lib.load().ktb_counter_add_device(self._handle(), bases.data_ptr() if total else None,
                                                           offsets.data_ptr(), max(n, 0), total, stream))
+
+    def _check_tensors(self, bases, offsets):
+        import torch
+        if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
+            raise ValueError("bases and offsets must be CUDA tensors on one device")
+        if bases.device.index != self.device:
+            raise ValueError(f"the tensors are on {bases.device}, the counter on cuda:{self.device}")
+        if bases.dtype != torch.uint8 or offsets.dtype != torch.int64:
+            raise TypeError(f"bases must be uint8 and offsets int64 (got {bases.dtype}, {offsets.dtype})")
+        if not (bases.is_contiguous() and offsets.is_contiguous()):
+            raise ValueError("bases and offsets must be contiguous")
 
     def _size(self):
         nkeys, nwin = C.c_uint64(), C.c_uint64()
@@ -105,6 +113,61 @@ class KmerCounter:
                 self._read = torch.cuda.Event()
                 self._read.record()
         return keys, counts
+
+    def _coverage_args(self, bin_size, bin_count, norm, dtype, torch_dtypes=None):
+        bin_size, bin_count = int(bin_size), int(bin_count)
+        if not 1 <= bin_size < 2 ** 32:
+            raise ValueError(f"bin_size must be in 1..2^32-1 (got {bin_size})")
+        if not 1 <= bin_count <= 65536:
+            raise ValueError(f"bin_count must be in 1..65536 (got {bin_count})")
+        codes = torch_dtypes or {np.dtype(np.uint32): _lib.OUT_U32, np.dtype(np.float32): _lib.OUT_F32,
+                                 np.dtype(np.float64): _lib.OUT_F64}
+        key = dtype if torch_dtypes else np.dtype(dtype)
+        if key not in codes:
+            raise TypeError(f"dtype must be uint32, float32 or float64 (got {dtype})")
+        out = codes[key]
+        if out == _lib.OUT_U32 and norm:
+            raise ValueError("uint32 rows are counts: pass norm=False")
+        return bin_size, bin_count, (_lib.NORM_CLI if norm else _lib.NORM_COUNTS), out
+
+    def coverage(self, seqs_or_packed, bin_size: int = 16, bin_count: int = 16, norm: bool = True, dtype=np.float32):
+        """Coverage histograms of a list of str / bytes, or a packed (bases u8, offsets u64[n+1]) pair, from host
+        memory: (rows (n, bin_count) of dtype, totals u64 (n,)).  Synchronous; reads the table in place."""
+        bin_size, bin_count, norm_mode, out = self._coverage_args(bin_size, bin_count, norm, dtype)
+        bases, offsets = _packed(seqs_or_packed)
+        n = max(len(offsets) - 1, 0)
+        rows = np.zeros((n, bin_count), dtype=np.dtype(dtype))
+        totals = np.zeros(n, dtype=np.uint64)
+        _lib.check(_lib.load().ktb_counter_coverage(self._handle(), bases.ctypes.data if bases.size else None,
+                                                    offsets.ctypes.data, n, bin_size, bin_count, norm_mode, out,
+                                                    rows.ctypes.data, totals.ctypes.data))
+        return rows, totals
+
+    def coverage_tensors(self, bases, offsets, bin_size: int = 16, bin_count: int = 16, norm: bool = True, dtype=None):
+        """coverage of CUDA tensors (the arguments of add_tensors) on torch's current stream: (rows (n, bin_count),
+        totals int64 (n,)) as CUDA tensors; dtype torch.float32 (default), torch.float64 or torch.int32 (u32 counts,
+        norm=False).  The kernels read the table in place; the next add or add_tensors waits for them."""
+        import torch
+        if dtype is None:
+            dtype = torch.float32
+        bin_size, bin_count, norm_mode, out = self._coverage_args(
+            bin_size, bin_count, norm, dtype,
+            {torch.int32: _lib.OUT_U32, torch.float32: _lib.OUT_F32, torch.float64: _lib.OUT_F64})
+        self._check_tensors(bases, offsets)
+        n = max(offsets.numel() - 1, 0)
+        total = bases.numel()
+        rows = torch.empty((n, bin_count), dtype=dtype, device=bases.device)
+        totals = torch.empty(n, dtype=torch.int64, device=bases.device)
+        with torch.cuda.device(bases.device):
+            current = torch.cuda.current_stream(bases.device)
+            _lib.check(_lib.load().ktb_counter_coverage_device(
+                self._handle(), bases.data_ptr() if total else None, offsets.data_ptr(), n, total, bin_size,
+                bin_count, norm_mode, out, rows.data_ptr() if n else None, totals.data_ptr() if n else None,
+                current.cuda_stream))
+            if n:
+                self._read = torch.cuda.Event()
+                self._read.record(current)
+        return rows, totals
 
     def close(self) -> None:
         if self._h:

@@ -1,7 +1,9 @@
 // counter.cu — C ABI of batch-wide k-mer counting (ktb_counter_*): a table of (key, u64 count) in ascending key order
 // on one GPU, grown by adds of batches.  An add enqueues the kernels of count_kernels.cuh and waits for its stream once,
-// at the end, to learn the new table size.
+// at the end, to learn the new table size.  Coverage histograms (ktb_counter_coverage*) look each window of a batch up
+// in that table through a directory built on first use (coverage_kernels.cuh).
 #include "count_kernels.cuh"
+#include "coverage_kernels.cuh"
 #include "device_guard.h"
 #include "device_scan.cuh"
 
@@ -18,6 +20,8 @@ struct ktb_counter {
     uint64_t *keys = nullptr, *counts = nullptr;   // the table (stream-ordered allocations)
     uint64_t nkeys = 0, nwindows = 0;
     unsigned long long *h_sizes = nullptr;         // page-locked [2]: valid windows and table keys of the last add
+    uint64_t *dir = nullptr;                       // coverage directory of this table (NULL until built; freed by an add)
+    uint32_t dir_bits = 0;
 };
 
 namespace {
@@ -154,6 +158,10 @@ int enqueue_add(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offset
         step(cudaFreeAsync(c->keys, st), "cudaFreeAsync(table)");
         step(cudaFreeAsync(c->counts, st), "cudaFreeAsync(table)");
     }
+    if (c->dir) {   // it indexes the old table
+        step(cudaFreeAsync(c->dir, st), "cudaFreeAsync(coverage directory)");
+        c->dir = nullptr;
+    }
     c->keys = okey;
     c->counts = ocnt;
     return rc;
@@ -164,6 +172,108 @@ int finish_add(ktb_counter *c, cudaStream_t st) {
     c->nwindows += c->h_sizes[0];
     c->nkeys = c->h_sizes[1];
     return KTB_OK;
+}
+
+// Directory bits for a table of nkeys keys: 2^b <= nkeys < 2^(b + 1), capped at 2k (a direct index) and at
+// COV_MAX_DIR_BITS.
+uint32_t dir_bits(uint64_t nkeys, int k) {
+    const uint32_t b = nkeys ? 63u - (uint32_t)__builtin_clzll(nkeys) : 0u;
+    return std::min<uint32_t>({b, 2u * (uint32_t)k, (uint32_t)COV_MAX_DIR_BITS});
+}
+
+// Builds the coverage directory of the current table on st and waits for it, once per table.  An empty table needs
+// none.  A directory that does not fit is KTB_ERR_NOMEM and leaves the counter as it was.
+int ensure_dir(ktb_counter *c, cudaStream_t st) {
+    if (c->dir || c->nkeys == 0) return KTB_OK;
+    const uint32_t b = dir_bits(c->nkeys, c->k);
+    const uint64_t nb = 1ull << b;
+    uint64_t *dir = nullptr;
+    if (const cudaError_t e = cudaMallocAsync((void **)&dir, (nb + 1) * sizeof(uint64_t), st)) {
+        cudaGetLastError();   // not sticky: later calls must not see it
+        return cuda_fail("cudaMallocAsync(coverage directory)", e);
+    }
+    int dev = 0, sms = 148;
+    CUP(cudaGetDevice(&dev));
+    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    const unsigned grid = (unsigned)std::min<uint64_t>(div_up(c->nkeys + 1, COV_DIR_THREADS), (uint64_t)sms * 8);
+    cov_dir_kernel<<<grid, COV_DIR_THREADS, 0, st>>>(c->keys, c->nkeys, 2u * (uint32_t)c->k - b, nb, dir);
+    cudaError_t e = cudaGetLastError();
+    const cudaError_t es = cudaStreamSynchronize(st);
+    if (e == cudaSuccess) e = es;
+    if (e != cudaSuccess) {
+        cudaFreeAsync(dir, st);
+        return cuda_fail("cov_dir_kernel", e);
+    }
+    c->dir = dir;
+    c->dir_bits = b;
+    return KTB_OK;
+}
+
+int check_coverage_args(uint32_t bin_size, uint32_t bin_count, int norm_mode, int out_dtype) {
+    if (bin_size < 1) return ktb_internal_fail(KTB_ERR_ARG, "bin_size must be at least 1");
+    if (bin_count < 1 || bin_count > COV_MAX_BINS) return ktb_internal_fail(KTB_ERR_ARG, "bin_count must be in 1..65536");
+    if (norm_mode != KTB_NORM_COUNTS && norm_mode != KTB_NORM_CLI)
+        return ktb_internal_fail(KTB_ERR_ARG, "norm_mode must be KTB_NORM_COUNTS or KTB_NORM_CLI for coverage rows");
+    if (out_dtype < KTB_OUT_U32 || out_dtype > KTB_OUT_F64) return ktb_internal_fail(KTB_ERR_ARG, "unknown out_dtype");
+    if (out_dtype == KTB_OUT_U32 && norm_mode != KTB_NORM_COUNTS)
+        return ktb_internal_fail(KTB_ERR_ARG, "KTB_OUT_U32 needs KTB_NORM_COUNTS");
+    return KTB_OK;
+}
+
+// Enqueues the coverage rows of one batch (device buffers, arguments checked, directory built) on st.
+int enqueue_coverage(const ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
+                     uint64_t total, uint32_t bin_size, uint32_t bin_count, int norm_mode, int out_dtype, void *d_out,
+                     uint64_t *d_totals, cudaStream_t st) {
+    const uint64_t nel = n * (uint64_t)bin_count;
+    const size_t esize = out_dtype == KTB_OUT_F64 ? 8 : 4;
+    if (total == 0) {   // every sequence is empty
+        CUP(cudaMemsetAsync(d_out, 0, nel * esize, st));
+        if (d_totals) CUP(cudaMemsetAsync(d_totals, 0, n * sizeof(uint64_t), st));
+        return KTB_OK;
+    }
+    const uint64_t nt = div_up(total, CT_T);
+    if (nt > 0x7fffffffull) return ktb_internal_fail(KTB_ERR_ARG, "batch too large for one call");
+    int dev = 0, sms = 148;
+    CUP(cudaGetDevice(&dev));
+    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    uint32_t *rows = (uint32_t *)d_out;   // 4-byte outputs are counted in place
+    if (esize == 8)
+        if (const cudaError_t e = cudaMallocAsync((void **)&rows, nel * sizeof(uint32_t), st)) {
+            cudaGetLastError();
+            return cuda_fail("cudaMallocAsync(coverage rows)", e);
+        }
+    int rc = KTB_OK;
+    auto step = [&](cudaError_t e, const char *what) {
+        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
+    };
+    step(cudaMemsetAsync(rows, 0, nel * sizeof(uint32_t), st), "cudaMemsetAsync(coverage rows)");
+    CovParams p{};
+    p.kp.bases = d_bases;
+    p.kp.offsets = d_offsets;
+    p.kp.n = n;
+    p.kp.k = (uint32_t)c->k;
+    p.kp.canonical = c->canonical;
+    p.tkey = c->keys;
+    p.tcnt = c->counts;
+    p.nkeys = c->nkeys;
+    p.dir = c->dir;
+    p.shift = 2u * (uint32_t)c->k - c->dir_bits;
+    p.bin_size = bin_size;
+    p.bin_count = bin_count;
+    p.rows = rows;
+    if (rc == KTB_OK) {
+        cov_hist_kernel<<<(unsigned)nt, CT_THREADS, 0, st>>>(p);
+        step(cudaGetLastError(), "cov_hist_kernel");
+    }
+    if (rc == KTB_OK) {
+        const unsigned grid = (unsigned)std::min<uint64_t>(div_up(n, COV_WTHREADS / 32), (uint64_t)sms * 16);
+        if (out_dtype == KTB_OUT_U32) cov_write_kernel<OUT_U32><<<grid, COV_WTHREADS, 0, st>>>(rows, d_out, d_totals, n, bin_count, norm_mode);
+        else if (out_dtype == KTB_OUT_F32) cov_write_kernel<OUT_F32><<<grid, COV_WTHREADS, 0, st>>>(rows, d_out, d_totals, n, bin_count, norm_mode);
+        else cov_write_kernel<OUT_F64><<<grid, COV_WTHREADS, 0, st>>>(rows, d_out, d_totals, n, bin_count, norm_mode);
+        step(cudaGetLastError(), "cov_write_kernel");
+    }
+    if (esize == 8) step(cudaFreeAsync(rows, st), "cudaFreeAsync(coverage rows)");
+    return rc;
 }
 
 }  // namespace
@@ -198,6 +308,7 @@ void ktb_counter_destroy(ktb_counter *c) {
     ktb::DeviceGuard device_guard(c->device);
     cudaFree(c->keys);   // the adds that used the table have finished: every add waits for its stream
     cudaFree(c->counts);
+    cudaFree(c->dir);
     cudaFreeHost(c->h_sizes);
     delete c;
 }
@@ -335,7 +446,117 @@ int ktb_counter_read_device(ktb_counter *c, uint64_t *d_keys, uint64_t *d_counts
     return KTB_OK;
 }
 
+int ktb_counter_coverage_device(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offsets, uint64_t n,
+                                uint64_t total_bases, uint32_t bin_size, uint32_t bin_count, int norm_mode,
+                                int out_dtype, void *d_out, uint64_t *d_totals, void *stream) {
+    if (!c || !d_offsets || (n > 0 && !d_out)) return ktb_internal_fail(KTB_ERR_ARG, "counter / d_offsets / d_out is NULL");
+    if (int rc = check_coverage_args(bin_size, bin_count, norm_mode, out_dtype)) return rc;
+    if (total_bases > 0 && !d_bases) return ktb_internal_fail(KTB_ERR_ARG, "d_bases is NULL");
+    if (n == 0) return KTB_OK;
+    ktb::DeviceGuard device_guard(c->device);
+    CUP(device_guard.err);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (int rc = ensure_dir(c, st)) return rc;
+    return enqueue_coverage(c, d_bases, d_offsets, n, total_bases, bin_size, bin_count, norm_mode, out_dtype, d_out,
+                            d_totals, st);
+}
+
+int ktb_counter_coverage(ktb_counter *c, const uint8_t *bases, const uint64_t *offsets, uint64_t n, uint32_t bin_size,
+                         uint32_t bin_count, int norm_mode, int out_dtype, void *out, uint64_t *totals) {
+    if (!c || !offsets || (n > 0 && !out)) return ktb_internal_fail(KTB_ERR_ARG, "counter / offsets / out is NULL");
+    if (int rc = check_coverage_args(bin_size, bin_count, norm_mode, out_dtype)) return rc;
+    char msg[160];
+    const uint64_t k = (uint64_t)c->k;
+    for (uint64_t i = 0; i < n; ++i) {
+        if (offsets[i + 1] < offsets[i]) {
+            snprintf(msg, sizeof msg, "offsets must be non-decreasing (at %llu)", (unsigned long long)i);
+            return ktb_internal_fail(KTB_ERR_ARG, msg);
+        }
+        const uint64_t len = offsets[i + 1] - offsets[i];
+        if (len >= k && len - k + 1 > 0xFFFFFFFFull) {
+            snprintf(msg, sizeof msg, "sequence %llu has %llu windows; counts are 32-bit (at most 2^32 - 1 windows)",
+                     (unsigned long long)i, (unsigned long long)(len - k + 1));
+            return ktb_internal_fail(KTB_ERR_ARG, msg);
+        }
+    }
+    if (offsets[n] > offsets[0] && !bases) return ktb_internal_fail(KTB_ERR_ARG, "bases is NULL");
+    if (n == 0) return KTB_OK;
+    ktb::DeviceGuard device_guard(c->device);
+    CUP(device_guard.err);
+
+    // chunks of whole sequences, at most COUNT_CHUNK_BASES bases each unless one sequence is longer
+    std::vector<uint64_t> cut{0};
+    uint64_t max_bases = 0, max_n = 0;
+    for (uint64_t i0 = 0; i0 < n;) {
+        uint64_t i1 = i0 + 1;
+        while (i1 < n && offsets[i1 + 1] - offsets[i0] <= COUNT_CHUNK_BASES) ++i1;
+        max_bases = std::max(max_bases, offsets[i1] - offsets[i0]);
+        max_n = std::max(max_n, i1 - i0);
+        cut.push_back(i1);
+        i0 = i1;
+    }
+    const size_t esize = out_dtype == KTB_OUT_F64 ? 8 : 4;
+    const uint64_t row_bytes = (uint64_t)bin_count * esize;
+    // Two slots: chunk c + 1 is copied in and computed on one stream while the rows of chunk c are copied out on the
+    // other.  A slot's host offsets are rewritten only after its stream has finished the chunk before.
+    struct Slot {
+        cudaStream_t st = nullptr;
+        uint8_t *bases = nullptr;
+        uint64_t *offsets = nullptr, *h_offsets = nullptr, *totals = nullptr;
+        void *out = nullptr;
+    } slot[2];
+    int rc = KTB_OK;
+    auto step = [&](cudaError_t e, const char *what) {
+        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
+    };
+    for (Slot &s : slot) {
+        step(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking), "cudaStreamCreate");
+        step(cudaMalloc((void **)&s.bases, std::max<uint64_t>(max_bases, 1)), "cudaMalloc(bases)");
+        step(cudaMalloc((void **)&s.offsets, (max_n + 1) * sizeof(uint64_t)), "cudaMalloc(offsets)");
+        step(cudaMalloc((void **)&s.totals, max_n * sizeof(uint64_t)), "cudaMalloc(totals)");
+        step(cudaMalloc(&s.out, max_n * row_bytes), "cudaMalloc(rows)");
+        step(cudaHostAlloc((void **)&s.h_offsets, (max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
+             "cudaHostAlloc(offsets)");
+    }
+    if (rc == KTB_OK) rc = ensure_dir(c, slot[0].st);
+    const uint64_t nchunks = cut.size() - 1;
+    for (uint64_t ci = 0; ci < nchunks && rc == KTB_OK; ++ci) {
+        Slot &s = slot[ci & 1];
+        step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");   // chunk ci - 2 has left the slot
+        if (rc != KTB_OK) break;
+        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, b0 = offsets[i0], nb = offsets[cut[ci + 1]] - b0;
+        for (uint64_t i = 0; i <= cn; ++i) s.h_offsets[i] = offsets[i0 + i] - b0;
+        if (nb) step(cudaMemcpyAsync(s.bases, bases + b0, nb, cudaMemcpyHostToDevice, s.st), "cudaMemcpyAsync(bases)");
+        step(cudaMemcpyAsync(s.offsets, s.h_offsets, (cn + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s.st),
+             "cudaMemcpyAsync(offsets)");
+        if (rc == KTB_OK)
+            rc = enqueue_coverage(c, s.bases, s.offsets, cn, nb, bin_size, bin_count, norm_mode, out_dtype, s.out,
+                                  s.totals, s.st);
+        step(cudaMemcpyAsync((char *)out + i0 * row_bytes, s.out, cn * row_bytes, cudaMemcpyDeviceToHost, s.st),
+             "cudaMemcpyAsync(rows)");
+        if (totals)
+            step(cudaMemcpyAsync(totals + i0, s.totals, cn * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
+                 "cudaMemcpyAsync(totals)");
+    }
+    for (Slot &s : slot) {
+        if (s.st) step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");
+        cudaFree(s.bases);
+        cudaFree(s.offsets);
+        cudaFree(s.totals);
+        cudaFree(s.out);
+        cudaFreeHost(s.h_offsets);
+        if (s.st) cudaStreamDestroy(s.st);
+    }
+    return rc;
+}
+
 }  // extern "C"
+
+// The argument checks of the coverage entry points, for the file driver's checks before any device work (file_api.cu).
+__attribute__((visibility("hidden"))) int ktb_internal_coverage_args(uint32_t bin_size, uint32_t bin_count,
+                                                                      int norm_mode, int out_dtype) {
+    return check_coverage_args(bin_size, bin_count, norm_mode, out_dtype);
+}
 
 // The table in place, for the file driver's read-back in slices (file_api.cu).
 __attribute__((visibility("hidden"))) void ktb_internal_counter_table(const ktb_counter *c, const uint64_t **keys,

@@ -30,6 +30,7 @@ int ktb_internal_fail(int code, const char *msg);
 int ktb_internal_sms(const ktb_oligo *h);
 uint64_t ktb_internal_launches(const ktb_oligo *h);
 void ktb_internal_counter_table(const ktb_counter *c, const uint64_t **keys, const uint64_t **counts);
+int ktb_internal_coverage_args(uint32_t bin_size, uint32_t bin_count, int norm_mode, int out_dtype);
 
 namespace {
 
@@ -196,6 +197,55 @@ int fill_batch(ktb::FastxParser &parser, Pinned &bases, size_t *cap, size_t max_
         }
         return KTB_OK;
     }
+}
+
+// Opens a sequence input of the counting drivers: "-" (stdin) sniffs the first byte, a path's extension decides.
+int open_seq_input(const std::string &path, ktb::ByteSource *src, ktb::SeqFormat *fmt) {
+    std::string err;
+    if (!src->open(path, &err)) return ktb_internal_fail(KTB_ERR_IO, err.c_str());
+    if (path == "-") *fmt = (src->peek_first_byte() == '>') ? ktb::SeqFormat::Fasta : ktb::SeqFormat::Fastq;
+    else if (!ktb::format_from_path(path, fmt))
+        return ktb_internal_fail(KTB_ERR_IO, "unknown sequence file extension (expected .fa/.fasta/.fna/.fq/.fastq[.gz])");
+    return KTB_OK;
+}
+
+// Counts every record of `parser` into c: batch b is added on a worker thread while the caller parses batch b + 1 into
+// the other buffer.  Adds the records, bases, parse time and the time spent waiting for adds to *st.
+int count_into(ktb_counter *c, ktb::FastxParser &parser, size_t bases_cap, ktb_file_stats *st) {
+    Pinned hbases[2];
+    std::vector<uint64_t> offs[2];
+    const size_t max_records = 4u << 20;
+    std::thread adder;
+    int add_rc = KTB_OK;
+    std::string add_err;
+    auto join = [&]() -> int {
+        if (!adder.joinable()) return KTB_OK;
+        const double t0 = now_ms();
+        adder.join();
+        st->gpu_wait_ms += now_ms() - t0;
+        return add_rc ? ktb_internal_fail(add_rc, add_err.c_str()) : KTB_OK;
+    };
+    struct JoinGuard { std::thread *t; ~JoinGuard() { if (t->joinable()) t->join(); } } join_guard{&adder};
+    for (int b = 0;; ++b) {
+        Pinned &hb = hbases[b & 1];
+        std::vector<uint64_t> &of = offs[b & 1];
+        const double tp0 = now_ms();
+        if (!hb.ensure(bases_cap)) return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
+        size_t used = 0;
+        if (int rc = fill_batch(parser, hb, &bases_cap, max_records, &used, &of)) return rc;
+        st->parse_ms += now_ms() - tp0;
+        if (int rc = join()) return rc;
+        const uint64_t n = of.size() - 1;
+        if (n == 0) break;
+        st->records += n;
+        st->bases += used;
+        adder = std::thread([&, n, b] {
+            add_rc = ktb_counter_add(c, (const uint8_t *)hbases[b & 1].p, offs[b & 1].data(), n);
+            if (add_rc) add_err = ktb_last_error();
+        });
+        if (parser.eof()) break;
+    }
+    return join();
 }
 
 // u32 counts of rows [r0, r1) -> "c0<d>c1<d>...\n" (format!("{}", f64) prints integral values without ".0", oligo.rs:138)
@@ -418,7 +468,15 @@ int ktb_debug_fastx_batches(const char *path, int sniff, uint64_t max_records, u
     return KTB_OK;
 }
 
-static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsize) {
+// The counter and bins of `kmertools cov`, whose rows are coverage histograms of bin_count values.
+struct CoverageRows {
+    ktb_counter *c;
+    uint32_t bin_size, bin_count;
+};
+
+// The drivers that write one line per record: `comp oligo` and `comp cgr` (k-mer rows of a ktb_oligo handle) and, with
+// cov, `cov` (coverage rows of a counter).  Only the compute step of a batch differs between them.
+static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsize, const CoverageRows *cov = nullptr) {
     const bool cgr = cgr_vecsize > 0;
     const double t_start = now_ms();
     if (!o || !o->in_path || !o->out_path) return ktb_internal_fail(KTB_ERR_ARG, "null argument");
@@ -439,11 +497,16 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
     ktb::FastxParser parser(&src, fmt);
 
     ktb_oligo *h = nullptr;
-    if (int rc = ktb_oligo_create(o->k, o->device, &h)) return rc;
+    if (!cov)
+        if (int rc = ktb_oligo_create(o->k, o->device, &h)) return rc;
     struct Guard { ktb_oligo *h; ~Guard() { ktb_oligo_destroy(h); } } guard{h};
     ktb::DeviceGuard device_guard(o->device);   // buffers and streams of this run live on the handle's device
     if (device_guard.err != cudaSuccess) return ktb_internal_fail(KTB_ERR_CUDA, "cudaSetDevice failed");
-    const uint64_t dim = ktb_oligo_dim(h, cgr ? 1 : o->canonical);
+    const uint64_t dim = cov ? cov->bin_count : ktb_oligo_dim(h, cgr ? 1 : o->canonical);
+    int sms = 0;
+    if (h) sms = ktb_internal_sms(h);
+    else if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, o->device) != cudaSuccess)
+        return ktb_internal_fail(KTB_ERR_CUDA, "cudaDeviceGetAttribute failed");
 
     const int nthreads = host_threads(o->threads);
     ktb::SpanWriter wr;
@@ -529,6 +592,24 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
         return KTB_OK;
     };
 
+    // the compute step of one batch: u32 rows (f64 for normalised CGR rows) and totals of the batch on s.stream
+    auto compute = [&](Set &s, bool f64rows) -> int {
+        const uint8_t *d_bases = (const uint8_t *)s.d_bases.p;
+        const uint64_t *d_offsets = (const uint64_t *)s.d_offsets.p;
+        if (cov) {
+            launches += 2;   // cov_hist_kernel, cov_write_kernel
+            return ktb_counter_coverage_device(cov->c, d_bases, d_offsets, s.n, s.nbases, cov->bin_size, cov->bin_count,
+                                               KTB_NORM_COUNTS, KTB_OUT_U32, s.d_counts.p, (uint64_t *)s.d_totals.p,
+                                               s.stream);
+        }
+        const uint64_t l0 = ktb_internal_launches(h);
+        const int rc = ktb_internal_dispatch(h, d_bases, d_offsets, s.n, s.nbases, cgr ? 1 : o->canonical,
+                                             f64rows ? KTB_NORM_CLI : KTB_NORM_COUNTS, f64rows ? KTB_OUT_F64 : KTB_OUT_U32,
+                                             s.d_counts.p, (uint64_t *)s.d_totals.p, s.stream);
+        launches += ktb_internal_launches(h) - l0;
+        return rc;
+    };
+
     std::vector<uint64_t> offs;
     double alloc_ms = 0;   // page-locking / device allocation of the buffer sets (first two batches)
     const double t_loop = now_ms();
@@ -561,19 +642,12 @@ static int run_file(const ktb_file_opts *o, ktb_file_stats *stats, int cgr_vecsi
         alloc_ms += now_ms() - ta1;
         cudaMemcpyAsync(s.d_bases.p, s.h_bases.p, used, cudaMemcpyHostToDevice, s.stream);
         cudaMemcpyAsync(s.d_offsets.p, s.h_offsets.p, (n + 1) * 8, cudaMemcpyHostToDevice, s.stream);
-        const uint64_t l0 = ktb_internal_launches(h);
         if (prev_kernels_done) cudaStreamWaitEvent(s.stream, prev_kernels_done, 0);
-        const bool f64rows = cgr && norm;   // CGR prints the f64 quotient itself ("{}")
-        if (int rc = ktb_internal_dispatch(h, (const uint8_t *)s.d_bases.p, (const uint64_t *)s.d_offsets.p, n, used,
-                                           cgr ? 1 : o->canonical, f64rows ? KTB_NORM_CLI : KTB_NORM_COUNTS,
-                                           f64rows ? KTB_OUT_F64 : KTB_OUT_U32, s.d_counts.p,
-                                           (uint64_t *)s.d_totals.p, s.stream))
-            return rc;
-        launches += ktb_internal_launches(h) - l0;
+        if (int rc = compute(s, cgr && norm)) return rc;   // CGR prints the f64 quotient itself ("{}")
         if (gpu_text) {
             const uint64_t nel = n * dim;
             uint64_t grid = (nel + 255) / 256;
-            const uint64_t cap = (uint64_t)ktb_internal_sms(h) * 16;
+            const uint64_t cap = (uint64_t)sms * 16;
             if (grid > cap) grid = cap;
             ktb::format_norm_kernel<<<(unsigned)grid, 256, 0, s.stream>>>(
                 (const uint32_t *)s.d_counts.p, (const uint64_t *)s.d_totals.p, (uint8_t *)s.d_text.p, n, (uint32_t)dim,
@@ -639,12 +713,8 @@ int ktb_count_file(const ktb_file_opts *o, int acgt, ktb_file_stats *stats) {
     ktb_file_stats st{};
     const std::string in = o->in_path;
     ktb::ByteSource src;
-    std::string err;
-    if (!src.open(in, &err)) return ktb_internal_fail(KTB_ERR_IO, err.c_str());
     ktb::SeqFormat fmt;
-    if (in == "-") fmt = (src.peek_first_byte() == '>') ? ktb::SeqFormat::Fasta : ktb::SeqFormat::Fastq;
-    else if (!ktb::format_from_path(in, &fmt))
-        return ktb_internal_fail(KTB_ERR_IO, "unknown sequence file extension (expected .fa/.fasta/.fna/.fq/.fastq[.gz])");
+    if (int rc = open_seq_input(in, &src, &fmt)) return rc;
     ktb::FastxParser parser(&src, fmt);
 
     ktb_counter *c = nullptr;
@@ -658,42 +728,7 @@ int ktb_count_file(const ktb_file_opts *o, int acgt, ktb_file_stats *stats) {
     const std::string out_file = std::string(o->out_path) + "/kmers.counts";
     const int nthreads = host_threads(o->threads);
 
-    // ---- count: batch b is added on a worker thread while the caller parses batch b + 1 into the other buffer
-    Pinned hbases[2];
-    std::vector<uint64_t> offs[2];
-    size_t bases_cap = input_bases_cap(in);
-    const size_t max_records = 4u << 20;
-    std::thread adder;
-    int add_rc = KTB_OK;
-    std::string add_err;
-    auto join = [&]() -> int {
-        if (!adder.joinable()) return KTB_OK;
-        const double t0 = now_ms();
-        adder.join();
-        st.gpu_wait_ms += now_ms() - t0;
-        return add_rc ? ktb_internal_fail(add_rc, add_err.c_str()) : KTB_OK;
-    };
-    struct JoinGuard { std::thread *t; ~JoinGuard() { if (t->joinable()) t->join(); } } join_guard{&adder};
-    for (int b = 0;; ++b) {
-        Pinned &hb = hbases[b & 1];
-        std::vector<uint64_t> &of = offs[b & 1];
-        const double tp0 = now_ms();
-        if (!hb.ensure(bases_cap)) return ktb_internal_fail(KTB_ERR_NOMEM, "pinned allocation failed");
-        size_t used = 0;
-        if (int rc = fill_batch(parser, hb, &bases_cap, max_records, &used, &of)) return rc;
-        st.parse_ms += now_ms() - tp0;
-        if (int rc = join()) return rc;
-        const uint64_t n = of.size() - 1;
-        if (n == 0) break;
-        st.records += n;
-        st.bases += used;
-        adder = std::thread([&, n, b] {
-            add_rc = ktb_counter_add(c, (const uint8_t *)hbases[b & 1].p, offs[b & 1].data(), n);
-            if (add_rc) add_err = ktb_last_error();
-        });
-        if (parser.eof()) break;
-    }
-    if (int rc = join()) return rc;
+    if (int rc = count_into(c, parser, input_bases_cap(in), &st)) return rc;
 
     // ---- write: slices of the table through page-locked staging (slice s + 1 is copied while slice s is formatted)
     const double tw0 = now_ms();
@@ -701,6 +736,7 @@ int ktb_count_file(const ktb_file_opts *o, int acgt, ktb_file_stats *stats) {
     ktb_counter_size(c, &nkeys, nullptr);
     const uint64_t *d_keys, *d_counts;
     ktb_internal_counter_table(c, &d_keys, &d_counts);
+    std::string err;
     ktb::SpanWriter wr;
     if (!wr.open(out_file.c_str(), nthreads, &err)) return ktb_internal_fail(KTB_ERR_IO, err.c_str());
     const uint64_t SLICE = 1u << 22;
@@ -749,6 +785,47 @@ int ktb_count_file(const ktb_file_opts *o, int acgt, ktb_file_stats *stats) {
     st.bytes_written = wr.bytes();
     if (!wr.close()) return ktb_internal_fail(KTB_ERR_IO, "closing the output file failed");
     st.write_ms = now_ms() - tw0;
+    st.total_ms = now_ms() - t_start;
+    if (stats) *stats = st;
+    return KTB_OK;
+}
+
+int ktb_coverage_file(const ktb_file_opts *o, const char *count_path, uint32_t bin_size, uint32_t bin_count,
+                      ktb_file_stats *stats) {
+    const double t_start = now_ms();
+    if (!o || !o->in_path || !o->out_path) return ktb_internal_fail(KTB_ERR_ARG, "null argument");
+    if (o->k < 1 || o->k > KTB_MAX_SPARSE_K) {
+        char msg[96];
+        snprintf(msg, sizeof msg, "k must be in 1..%d for coverage rows (got %d)", KTB_MAX_SPARSE_K, o->k);
+        return ktb_internal_fail(KTB_ERR_ARG, msg);
+    }
+    if (int rc = ktb_internal_coverage_args(bin_size, bin_count, KTB_NORM_COUNTS, KTB_OUT_U32)) return rc;
+    const std::string in = o->in_path, counted = count_path ? count_path : o->in_path;
+    if (in == "-" && counted == "-")
+        return ktb_internal_fail(KTB_ERR_ARG, "stdin input needs a separate input to count (it would be read twice)");
+    ktb::ByteSource src;
+    ktb::SeqFormat fmt;
+    if (int rc = open_seq_input(counted, &src, &fmt)) return rc;
+    ktb::FastxParser parser(&src, fmt);
+
+    ktb_counter *c = nullptr;
+    if (int rc = ktb_counter_create(o->k, 1, o->device, &c)) return rc;
+    struct Guard { ktb_counter *c; ~Guard() { ktb_counter_destroy(c); } } guard{c};
+    ktb::DeviceGuard device_guard(o->device);   // page-locked buffers of the count pass belong to this device
+    if (device_guard.err != cudaSuccess) return ktb_internal_fail(KTB_ERR_CUDA, "cudaSetDevice failed");
+    ktb_file_stats count_st{};
+    if (int rc = count_into(c, parser, input_bases_cap(counted), &count_st)) return rc;
+
+    ktb_file_opts ro = *o;
+    ro.canonical = 1;
+    ro.norm = 1;
+    ro.delim = ' ';
+    ro.header = 0;
+    const CoverageRows cov{c, bin_size, bin_count};
+    ktb_file_stats st{};
+    if (int rc = run_file(&ro, &st, 0, &cov)) return rc;
+    st.parse_ms += count_st.parse_ms;
+    st.gpu_wait_ms += count_st.gpu_wait_ms;
     st.total_ms = now_ms() - t_start;
     if (stats) *stats = st;
     return KTB_OK;
