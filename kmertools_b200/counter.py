@@ -16,7 +16,8 @@ import ctypes as C
 import numpy as np
 
 from . import _lib
-from .sparse import _check_k, _packed
+from .oligo import _CODES
+from .sparse import _check_k, _check_tensors, _packed
 
 
 class KmerCounter:
@@ -53,7 +54,7 @@ class KmerCounter:
         buffer, pass the slice bases[offsets[0]:offsets[n]] and offsets - offsets[0].  The current stream first waits
         for the copies of an earlier result_tensors, which read the table this add replaces."""
         import torch
-        self._check_tensors(bases, offsets)
+        _check_tensors(bases, offsets, self.device)
         n = offsets.numel() - 1
         total = bases.numel()
         with torch.cuda.device(bases.device):
@@ -63,17 +64,6 @@ class KmerCounter:
             stream = current.cuda_stream
             _lib.check(_lib.load().ktb_counter_add_device(self._handle(), bases.data_ptr() if total else None,
                                                           offsets.data_ptr(), max(n, 0), total, stream))
-
-    def _check_tensors(self, bases, offsets):
-        import torch
-        if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
-            raise ValueError("bases and offsets must be CUDA tensors on one device")
-        if bases.device.index != self.device:
-            raise ValueError(f"the tensors are on {bases.device}, the counter on cuda:{self.device}")
-        if bases.dtype != torch.uint8 or offsets.dtype != torch.int64:
-            raise TypeError(f"bases must be uint8 and offsets int64 (got {bases.dtype}, {offsets.dtype})")
-        if not (bases.is_contiguous() and offsets.is_contiguous()):
-            raise ValueError("bases and offsets must be contiguous")
 
     def _size(self):
         nkeys, nwin = C.c_uint64(), C.c_uint64()
@@ -120,8 +110,7 @@ class KmerCounter:
             raise ValueError(f"bin_size must be in 1..2^32-1 (got {bin_size})")
         if not 1 <= bin_count <= 65536:
             raise ValueError(f"bin_count must be in 1..65536 (got {bin_count})")
-        codes = torch_dtypes or {np.dtype(np.uint32): _lib.OUT_U32, np.dtype(np.float32): _lib.OUT_F32,
-                                 np.dtype(np.float64): _lib.OUT_F64}
+        codes = torch_dtypes or _CODES
         key = dtype if torch_dtypes else np.dtype(dtype)
         if key not in codes:
             raise TypeError(f"dtype must be uint32, float32 or float64 (got {dtype})")
@@ -153,7 +142,7 @@ class KmerCounter:
         bin_size, bin_count, norm_mode, out = self._coverage_args(
             bin_size, bin_count, norm, dtype,
             {torch.int32: _lib.OUT_U32, torch.float32: _lib.OUT_F32, torch.float64: _lib.OUT_F64})
-        self._check_tensors(bases, offsets)
+        _check_tensors(bases, offsets, self.device)
         n = max(offsets.numel() - 1, 0)
         total = bases.numel()
         rows = torch.empty((n, bin_count), dtype=dtype, device=bases.device)

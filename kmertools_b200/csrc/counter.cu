@@ -11,7 +11,6 @@
 #include <stdint.h>
 #include <algorithm>
 #include <cstdio>
-#include <vector>
 
 using namespace ktb;
 
@@ -25,9 +24,6 @@ struct ktb_counter {
 };
 
 namespace {
-
-// bases of one chunk of the host entry point (a longer single sequence is a chunk of its own)
-constexpr uint64_t COUNT_CHUNK_BASES = 1ull << 26;
 
 int check_k(int k, int canonical) {
     char msg[128];
@@ -53,9 +49,8 @@ int enqueue_add(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offset
     const uint64_t ncap = c->nkeys + std::min(W, space);     // bound of the merged table
     const uint64_t nbsum = div_up(std::max({nt_k, (uint64_t)RX_DIGITS * nt_r, nblk, W}), SP_WB);
 
-    int dev = 0, sms = 148;
-    CUP(cudaGetDevice(&dev));
-    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 148;
+    if (int rc = sm_count(&sms)) return rc;
 
     Carve s;
     unsigned long long *tile_valid, *tile_base, *hist, *hoff, *bheads, *bbase, *R, *D, *bsum, *sizes;
@@ -92,9 +87,7 @@ int enqueue_add(ktb_counter *c, const uint8_t *d_bases, const uint64_t *d_offset
     layout();
 
     int rc = KTB_OK;
-    auto step = [&](cudaError_t e, const char *what) {
-        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
-    };
+    FirstError step{rc};
     // keys: count, scan, write
     CountKeysParams kp{d_bases, d_offsets, n, (uint32_t)c->k, c->canonical, tile_valid, tile_base, X};
     count_valid_kernel<<<(unsigned)nt_k, CT_THREADS, 0, st>>>(kp);
@@ -187,14 +180,13 @@ int ensure_dir(ktb_counter *c, cudaStream_t st) {
     if (c->dir || c->nkeys == 0) return KTB_OK;
     const uint32_t b = dir_bits(c->nkeys, c->k);
     const uint64_t nb = 1ull << b;
+    int sms = 148;
+    if (int rc = sm_count(&sms)) return rc;
     uint64_t *dir = nullptr;
     if (const cudaError_t e = cudaMallocAsync((void **)&dir, (nb + 1) * sizeof(uint64_t), st)) {
         cudaGetLastError();   // not sticky: later calls must not see it
         return cuda_fail("cudaMallocAsync(coverage directory)", e);
     }
-    int dev = 0, sms = 148;
-    CUP(cudaGetDevice(&dev));
-    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
     const unsigned grid = (unsigned)std::min<uint64_t>(div_up(c->nkeys + 1, COV_DIR_THREADS), (uint64_t)sms * 8);
     cov_dir_kernel<<<grid, COV_DIR_THREADS, 0, st>>>(c->keys, c->nkeys, 2u * (uint32_t)c->k - b, nb, dir);
     cudaError_t e = cudaGetLastError();
@@ -233,9 +225,8 @@ int enqueue_coverage(const ktb_counter *c, const uint8_t *d_bases, const uint64_
     }
     const uint64_t nt = div_up(total, CT_T);
     if (nt > 0x7fffffffull) return ktb_internal_fail(KTB_ERR_ARG, "batch too large for one call");
-    int dev = 0, sms = 148;
-    CUP(cudaGetDevice(&dev));
-    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 148;
+    if (int rc = sm_count(&sms)) return rc;
     uint32_t *rows = (uint32_t *)d_out;   // 4-byte outputs are counted in place
     if (esize == 8)
         if (const cudaError_t e = cudaMallocAsync((void **)&rows, nel * sizeof(uint32_t), st)) {
@@ -243,9 +234,7 @@ int enqueue_coverage(const ktb_counter *c, const uint8_t *d_bases, const uint64_
             return cuda_fail("cudaMallocAsync(coverage rows)", e);
         }
     int rc = KTB_OK;
-    auto step = [&](cudaError_t e, const char *what) {
-        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
-    };
+    FirstError step{rc};
     step(cudaMemsetAsync(rows, 0, nel * sizeof(uint32_t), st), "cudaMemsetAsync(coverage rows)");
     CovParams p{};
     p.kp.bases = d_bases;
@@ -285,9 +274,7 @@ int ktb_counter_create(int k, int canonical, int device, ktb_counter **out) {
     *out = nullptr;
     if (int rc = check_k(k, canonical)) return rc;
     if (device < 0) return ktb_internal_fail(KTB_ERR_ARG, "device out of range");
-    const int ndev = ktb_device_count();
-    if (ndev <= 0) return ktb_internal_fail(KTB_ERR_NODEVICE, "no CUDA device available (this library has no CPU path)");
-    if (device < 0 || device >= ndev) return ktb_internal_fail(KTB_ERR_ARG, "device out of range");
+    if (int rc = check_device(device)) return rc;
     ktb::DeviceGuard device_guard(device);
     CUP(device_guard.err);
     ktb_counter *c = new ktb_counter();
@@ -315,76 +302,34 @@ void ktb_counter_destroy(ktb_counter *c) {
 
 int ktb_counter_add(ktb_counter *c, const uint8_t *bases, const uint64_t *offsets, uint64_t n) {
     if (!c || !offsets) return ktb_internal_fail(KTB_ERR_ARG, "counter / offsets is NULL");
-    char msg[160];
-    for (uint64_t i = 0; i < n; ++i)
-        if (offsets[i + 1] < offsets[i]) {
-            snprintf(msg, sizeof msg, "offsets must be non-decreasing (at %llu)", (unsigned long long)i);
-            return ktb_internal_fail(KTB_ERR_ARG, msg);
-        }
-    if (offsets[n] > offsets[0] && !bases) return ktb_internal_fail(KTB_ERR_ARG, "bases is NULL");
+    if (int rc = check_offsets(bases, offsets, n, c->k, false)) return rc;
     if (n == 0 || offsets[n] == offsets[0]) return KTB_OK;
     ktb::DeviceGuard device_guard(c->device);
     CUP(device_guard.err);
 
-    // chunks of whole sequences, at most COUNT_CHUNK_BASES bases each unless one sequence is longer
-    std::vector<uint64_t> cut{0};
-    uint64_t max_bases = 0, max_n = 0;
-    for (uint64_t i0 = 0; i0 < n;) {
-        uint64_t i1 = i0 + 1;
-        while (i1 < n && offsets[i1 + 1] - offsets[i0] <= COUNT_CHUNK_BASES) ++i1;
-        max_bases = std::max(max_bases, offsets[i1] - offsets[i0]);
-        max_n = std::max(max_n, i1 - i0);
-        cut.push_back(i1);
-        i0 = i1;
-    }
+    const ChunkPlan plan(bases, offsets, n);
     // Two slots: chunk c + 1 is copied in on one stream while chunk c is counted and merged on the other.
-    struct Slot {
-        cudaStream_t st = nullptr;
-        uint8_t *bases = nullptr;
-        uint64_t *offsets = nullptr, *h_offsets = nullptr;
-    } slot[2];
+    ChunkSlot slot[2];
     int rc = KTB_OK;
-    auto step = [&](cudaError_t e, const char *what) {
-        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
-    };
-    for (Slot &s : slot) {
-        step(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking), "cudaStreamCreate");
-        step(cudaMalloc((void **)&s.bases, std::max<uint64_t>(max_bases, 1)), "cudaMalloc(bases)");
-        step(cudaMalloc((void **)&s.offsets, (max_n + 1) * sizeof(uint64_t)), "cudaMalloc(offsets)");
-        step(cudaHostAlloc((void **)&s.h_offsets, (max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
-             "cudaHostAlloc(offsets)");
-    }
-    const uint64_t nchunks = cut.size() - 1;
+    FirstError step{rc};
+    for (ChunkSlot &s : slot) s.alloc(plan, step);
+    const uint64_t nchunks = plan.chunks();
     // Over several chunks, the table the add started from is kept until the add returns, so that a chunk that fails
     // (a scratch that does not fit) can restore it: the counter then holds none of the batch, not part of it.
     const ktb_counter saved = *c;
     const bool keep = nchunks > 1;
-    auto copy_in = [&](uint64_t ci) {
-        Slot &s = slot[ci & 1];
-        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, b0 = offsets[i0], nb = offsets[cut[ci + 1]] - b0;
-        for (uint64_t i = 0; i <= cn; ++i) s.h_offsets[i] = offsets[i0 + i] - b0;
-        if (nb) step(cudaMemcpyAsync(s.bases, bases + b0, nb, cudaMemcpyHostToDevice, s.st), "cudaMemcpyAsync(bases)");
-        step(cudaMemcpyAsync(s.offsets, s.h_offsets, (cn + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s.st),
-             "cudaMemcpyAsync(offsets)");
-    };
-    if (rc == KTB_OK) copy_in(0);
+    if (rc == KTB_OK) slot[0].copy_in(plan, 0, step);
     for (uint64_t ci = 0; ci < nchunks && rc == KTB_OK; ++ci) {
-        Slot &s = slot[ci & 1];
-        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, nb = offsets[cut[ci + 1]] - offsets[i0];
-        const bool work = nb > 0;
-        if (work) rc = enqueue_add(c, s.bases, s.offsets, cn, nb, s.st, !(keep && c->keys == saved.keys));
+        ChunkSlot &s = slot[ci & 1];
+        const Chunk ch = plan[ci];
+        const bool work = ch.nb > 0;
+        if (work) rc = enqueue_add(c, s.bases, s.offsets, ch.n, ch.nb, s.st, !(keep && c->keys == saved.keys));
         if (rc == KTB_OK && ci + 1 < nchunks) {   // the other slot's stream finished its chunk in the last iteration
-            copy_in(ci + 1);
+            slot[(ci + 1) & 1].copy_in(plan, ci + 1, step);
         }
         if (rc == KTB_OK && work) rc = finish_add(c, s.st);
     }
-    for (Slot &s : slot) {
-        if (s.st) step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");
-        cudaFree(s.bases);
-        cudaFree(s.offsets);
-        cudaFreeHost(s.h_offsets);
-        if (s.st) cudaStreamDestroy(s.st);
-    }
+    for (ChunkSlot &s : slot) s.release(step);
     if (keep && c->keys != saved.keys) {   // the streams are idle: nothing reads either table any more
         if (rc == KTB_OK) {
             cudaFree(saved.keys);
@@ -465,87 +410,48 @@ int ktb_counter_coverage(ktb_counter *c, const uint8_t *bases, const uint64_t *o
                          uint32_t bin_count, int norm_mode, int out_dtype, void *out, uint64_t *totals) {
     if (!c || !offsets || (n > 0 && !out)) return ktb_internal_fail(KTB_ERR_ARG, "counter / offsets / out is NULL");
     if (int rc = check_coverage_args(bin_size, bin_count, norm_mode, out_dtype)) return rc;
-    char msg[160];
-    const uint64_t k = (uint64_t)c->k;
-    for (uint64_t i = 0; i < n; ++i) {
-        if (offsets[i + 1] < offsets[i]) {
-            snprintf(msg, sizeof msg, "offsets must be non-decreasing (at %llu)", (unsigned long long)i);
-            return ktb_internal_fail(KTB_ERR_ARG, msg);
-        }
-        const uint64_t len = offsets[i + 1] - offsets[i];
-        if (len >= k && len - k + 1 > 0xFFFFFFFFull) {
-            snprintf(msg, sizeof msg, "sequence %llu has %llu windows; counts are 32-bit (at most 2^32 - 1 windows)",
-                     (unsigned long long)i, (unsigned long long)(len - k + 1));
-            return ktb_internal_fail(KTB_ERR_ARG, msg);
-        }
-    }
-    if (offsets[n] > offsets[0] && !bases) return ktb_internal_fail(KTB_ERR_ARG, "bases is NULL");
+    if (int rc = check_offsets(bases, offsets, n, c->k, true)) return rc;
     if (n == 0) return KTB_OK;
     ktb::DeviceGuard device_guard(c->device);
     CUP(device_guard.err);
 
-    // chunks of whole sequences, at most COUNT_CHUNK_BASES bases each unless one sequence is longer
-    std::vector<uint64_t> cut{0};
-    uint64_t max_bases = 0, max_n = 0;
-    for (uint64_t i0 = 0; i0 < n;) {
-        uint64_t i1 = i0 + 1;
-        while (i1 < n && offsets[i1 + 1] - offsets[i0] <= COUNT_CHUNK_BASES) ++i1;
-        max_bases = std::max(max_bases, offsets[i1] - offsets[i0]);
-        max_n = std::max(max_n, i1 - i0);
-        cut.push_back(i1);
-        i0 = i1;
-    }
+    const ChunkPlan plan(bases, offsets, n);
     const size_t esize = out_dtype == KTB_OUT_F64 ? 8 : 4;
     const uint64_t row_bytes = (uint64_t)bin_count * esize;
     // Two slots: chunk c + 1 is copied in and computed on one stream while the rows of chunk c are copied out on the
     // other.  A slot's host offsets are rewritten only after its stream has finished the chunk before.
-    struct Slot {
-        cudaStream_t st = nullptr;
-        uint8_t *bases = nullptr;
-        uint64_t *offsets = nullptr, *h_offsets = nullptr, *totals = nullptr;
+    struct Slot : ChunkSlot {
+        uint64_t *totals = nullptr;
         void *out = nullptr;
     } slot[2];
     int rc = KTB_OK;
-    auto step = [&](cudaError_t e, const char *what) {
-        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
-    };
+    FirstError step{rc};
     for (Slot &s : slot) {
-        step(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking), "cudaStreamCreate");
-        step(cudaMalloc((void **)&s.bases, std::max<uint64_t>(max_bases, 1)), "cudaMalloc(bases)");
-        step(cudaMalloc((void **)&s.offsets, (max_n + 1) * sizeof(uint64_t)), "cudaMalloc(offsets)");
-        step(cudaMalloc((void **)&s.totals, max_n * sizeof(uint64_t)), "cudaMalloc(totals)");
-        step(cudaMalloc(&s.out, max_n * row_bytes), "cudaMalloc(rows)");
-        step(cudaHostAlloc((void **)&s.h_offsets, (max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
-             "cudaHostAlloc(offsets)");
+        s.alloc(plan, step);
+        step(cudaMalloc((void **)&s.totals, plan.max_n * sizeof(uint64_t)), "cudaMalloc(totals)");
+        step(cudaMalloc(&s.out, plan.max_n * row_bytes), "cudaMalloc(rows)");
     }
     if (rc == KTB_OK) rc = ensure_dir(c, slot[0].st);
-    const uint64_t nchunks = cut.size() - 1;
+    const uint64_t nchunks = plan.chunks();
     for (uint64_t ci = 0; ci < nchunks && rc == KTB_OK; ++ci) {
         Slot &s = slot[ci & 1];
         step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");   // chunk ci - 2 has left the slot
         if (rc != KTB_OK) break;
-        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, b0 = offsets[i0], nb = offsets[cut[ci + 1]] - b0;
-        for (uint64_t i = 0; i <= cn; ++i) s.h_offsets[i] = offsets[i0 + i] - b0;
-        if (nb) step(cudaMemcpyAsync(s.bases, bases + b0, nb, cudaMemcpyHostToDevice, s.st), "cudaMemcpyAsync(bases)");
-        step(cudaMemcpyAsync(s.offsets, s.h_offsets, (cn + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s.st),
-             "cudaMemcpyAsync(offsets)");
+        const Chunk ch = plan[ci];
+        s.copy_in(plan, ci, step);
         if (rc == KTB_OK)
-            rc = enqueue_coverage(c, s.bases, s.offsets, cn, nb, bin_size, bin_count, norm_mode, out_dtype, s.out,
+            rc = enqueue_coverage(c, s.bases, s.offsets, ch.n, ch.nb, bin_size, bin_count, norm_mode, out_dtype, s.out,
                                   s.totals, s.st);
-        step(cudaMemcpyAsync((char *)out + i0 * row_bytes, s.out, cn * row_bytes, cudaMemcpyDeviceToHost, s.st),
+        step(cudaMemcpyAsync((char *)out + ch.i0 * row_bytes, s.out, ch.n * row_bytes, cudaMemcpyDeviceToHost, s.st),
              "cudaMemcpyAsync(rows)");
         if (totals)
-            step(cudaMemcpyAsync(totals + i0, s.totals, cn * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
+            step(cudaMemcpyAsync(totals + ch.i0, s.totals, ch.n * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
                  "cudaMemcpyAsync(totals)");
     }
     for (Slot &s : slot) {
-        if (s.st) step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");
-        cudaFree(s.bases);
-        cudaFree(s.offsets);
+        s.release(step);
         cudaFree(s.totals);
         cudaFree(s.out);
-        cudaFreeHost(s.h_offsets);
-        if (s.st) cudaStreamDestroy(s.st);
     }
     return rc;
 }

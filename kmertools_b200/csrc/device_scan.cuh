@@ -1,28 +1,13 @@
-// device_scan.cuh — host helpers shared by the sparse rows (sparse.cu) and the k-mer counter (counter.cu): error
-// reporting of CUDA calls, the u64 exclusive scan, and a bump allocator over one stream-ordered allocation.
+// device_scan.cuh — host helpers shared by the sparse rows (sparse.cu) and the k-mer counter (counter.cu): the u64
+// exclusive scan and a bump allocator over one stream-ordered allocation.
 #pragma once
+#include "host_common.h"
 #include "sparse_common.cuh"
-#include "../../include/kmertools_b200.h"
 
 #include <cuda_runtime.h>
 #include <stdint.h>
-#include <cstdio>
-
-int ktb_internal_fail(int code, const char *msg);
 
 namespace ktb {
-
-inline int cuda_fail(const char *what, cudaError_t e) {
-    char msg[256];
-    snprintf(msg, sizeof msg, "%s failed: %s", what, cudaGetErrorString(e));
-    return ktb_internal_fail(e == cudaErrorMemoryAllocation ? KTB_ERR_NOMEM : KTB_ERR_CUDA, msg);
-}
-
-#define CUP(call)                                                \
-    do {                                                         \
-        cudaError_t e_ = (call);                                 \
-        if (e_ != cudaSuccess) return ktb::cuda_fail(#call, e_); \
-    } while (0)
 
 inline uint64_t div_up(uint64_t a, uint64_t b) { return (a + b - 1) / b; }
 

@@ -7,15 +7,15 @@
 // Output-bound (16 bytes per k-mer against 1 byte per base), so the spans are short and re-derived rather
 // than staged.
 #include "device_guard.h"
-#include "../../include/kmertools_b200.h"
+#include "host_common.h"
 
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <cstdio>
 
-int ktb_internal_fail(int code, const char *msg);
-
 namespace {
+
+using ktb::cuda_fail;
 
 constexpr int PAIR_THREADS = 256;
 constexpr int PAIR_SPAN = 16;                                  // window end positions per thread
@@ -126,18 +126,6 @@ __global__ void __launch_bounds__(PAIR_THREADS) pair_write_kernel(const uint8_t 
     });
 }
 
-int cuda_fail(const char *what, cudaError_t e) {
-    char msg[256];
-    snprintf(msg, sizeof msg, "%s failed: %s", what, cudaGetErrorString(e));
-    return ktb_internal_fail(e == cudaErrorMemoryAllocation ? KTB_ERR_NOMEM : KTB_ERR_CUDA, msg);
-}
-
-#define CUP(call)                                        \
-    do {                                                 \
-        cudaError_t e_ = (call);                         \
-        if (e_ != cudaSuccess) return cuda_fail(#call, e_); \
-    } while (0)
-
 int check_k(int k) {
     if (k < 1 || k > 31) {
         char msg[96];
@@ -183,9 +171,7 @@ int ktb_kmer_pairs(const uint8_t *seq, uint64_t len, int k, int device, uint64_t
     if (!count) return ktb_internal_fail(KTB_ERR_ARG, "count is NULL");
     if (cap > 0 && (!out_f || !out_r)) return ktb_internal_fail(KTB_ERR_ARG, "output arrays are NULL");
     if (len > 0 && !seq) return ktb_internal_fail(KTB_ERR_ARG, "seq is NULL");
-    const int ndev = ktb_device_count();
-    if (ndev <= 0) return ktb_internal_fail(KTB_ERR_NODEVICE, "no CUDA device available (this library has no CPU path)");
-    if (device < 0 || device >= ndev) return ktb_internal_fail(KTB_ERR_ARG, "device out of range");
+    if (int rc = ktb::check_device(device)) return rc;
     ktb::DeviceGuard device_guard(device);
     CUP(device_guard.err);
     *count = 0;

@@ -8,14 +8,10 @@
 #include <stdint.h>
 #include <algorithm>
 #include <cstdio>
-#include <vector>
 
 namespace {
 
 using namespace ktb;
-
-// bases of one chunk of the host entry point (a longer single sequence is a chunk of its own)
-constexpr uint64_t SPARSE_CHUNK_BASES = 1ull << 26;
 
 int check_args(int k, int canonical, int norm_mode, int out_dtype) {
     char msg[128];
@@ -71,9 +67,8 @@ int ktb_sparse_vectorise_device(const uint8_t *d_bases, const uint64_t *d_offset
     const uint64_t nblocks = div_up(total_bases, SP_WB);   // the lists hold at most one entry per window
     const uint64_t nbsum = std::max(div_up(n, SP_WB), div_up(nblocks, SP_WB));
 
-    int dev = 0, sms = 148;
-    CUP(cudaGetDevice(&dev));
-    CUP(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    int sms = 148;
+    if (int rc = sm_count(&sms)) return rc;
 
     Carve c;
     auto layout = [&](SparseParams &p, SparseOutParams &o, unsigned long long *&V, unsigned long long *&bsum,
@@ -108,9 +103,7 @@ int ktb_sparse_vectorise_device(const uint8_t *d_bases, const uint64_t *d_offset
     p.k = (uint32_t)k;
     p.canonical = canonical;
     int rc = KTB_OK;
-    auto step = [&](cudaError_t e, const char *what) {
-        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
-    };
+    FirstError step{rc};
     step(cudaMemsetAsync(p.tot, 0, 3 * ((n * 8 + 255) & ~(size_t)255), st), "cudaMemsetAsync(per-sequence counters)");
     step(cudaMemsetAsync(p.desc, 0xFF, ntiles * sizeof(SparseDesc), st), "cudaMemsetAsync(tile descriptors)");
     step(cudaFuncSetAttribute(sparse_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SP_SM_TOTAL),
@@ -164,92 +157,51 @@ int ktb_sparse_vectorise(const uint8_t *bases, const uint64_t *offsets, uint64_t
     if (int rc = check_args(k, canonical, norm_mode, out_dtype)) return rc;
     if (!offsets || !row_ptr) return ktb_internal_fail(KTB_ERR_ARG, "offsets / row_ptr is NULL");
     if (cap > 0 && (!codes || !values)) return ktb_internal_fail(KTB_ERR_ARG, "output arrays are NULL with cap > 0");
-    char msg[160];
-    for (uint64_t i = 0; i < n; ++i) {
-        if (offsets[i + 1] < offsets[i]) {
-            snprintf(msg, sizeof msg, "offsets must be non-decreasing (at %llu)", (unsigned long long)i);
-            return ktb_internal_fail(KTB_ERR_ARG, msg);
-        }
-        const uint64_t len = offsets[i + 1] - offsets[i];
-        if (len >= (uint64_t)k && len - (uint64_t)k + 1 > 0xFFFFFFFFull) {
-            snprintf(msg, sizeof msg, "sequence %llu has %llu windows; counts are 32-bit (at most 2^32 - 1 windows)",
-                     (unsigned long long)i, (unsigned long long)(len - (uint64_t)k + 1));
-            return ktb_internal_fail(KTB_ERR_ARG, msg);
-        }
-    }
-    if (offsets[n] > offsets[0] && !bases) return ktb_internal_fail(KTB_ERR_ARG, "bases is NULL");
-    const int ndev = ktb_device_count();
-    if (ndev <= 0) return ktb_internal_fail(KTB_ERR_NODEVICE, "no CUDA device available (this library has no CPU path)");
-    if (device < 0 || device >= ndev) return ktb_internal_fail(KTB_ERR_ARG, "device out of range");
+    if (int rc = check_offsets(bases, offsets, n, k, true)) return rc;
+    if (int rc = check_device(device)) return rc;
     ktb::DeviceGuard device_guard(device);
     CUP(device_guard.err);
-
-    // chunks of whole sequences, at most SPARSE_CHUNK_BASES bases each unless one sequence is longer
-    std::vector<uint64_t> cut{0};
-    uint64_t max_bases = 0, max_n = 0, max_windows = 0;
-    for (uint64_t i0 = 0; i0 < n;) {
-        uint64_t i1 = i0 + 1;
-        while (i1 < n && offsets[i1 + 1] - offsets[i0] <= SPARSE_CHUNK_BASES) ++i1;
-        uint64_t windows = 0;
-        for (uint64_t i = i0; i < i1; ++i) {
-            const uint64_t len = offsets[i + 1] - offsets[i];
-            windows += len >= (uint64_t)k ? len - (uint64_t)k + 1 : 0;
-        }
-        max_bases = std::max(max_bases, offsets[i1] - offsets[i0]);
-        max_n = std::max(max_n, i1 - i0);
-        max_windows = std::max(max_windows, windows);
-        cut.push_back(i1);
-        i0 = i1;
-    }
     if (n == 0) {
         row_ptr[0] = 0;
         return KTB_OK;
     }
+    const ChunkPlan plan(bases, offsets, n);
+    const uint64_t max_windows = std::max<uint64_t>(plan.max_windows(k), 1);
     const size_t esize = out_dtype == KTB_OUT_F64 ? 8 : 4;
 
     // Two slots.  Everything of chunk c + 1 is enqueued (bases in, kernels, row_ptr and totals out to page-locked
     // staging) before the host waits for chunk c, so the copy-out of chunk c's codes and values into the caller's
     // memory runs while chunk c + 1 computes on the other stream.
-    struct Slot {
-        cudaStream_t st = nullptr;
-        uint8_t *bases = nullptr;
-        uint64_t *offsets = nullptr, *row_ptr = nullptr, *codes = nullptr, *totals = nullptr;
+    struct Slot : ChunkSlot {
+        uint64_t *row_ptr = nullptr, *codes = nullptr, *totals = nullptr;
         void *values = nullptr;
-        uint64_t *h_offsets = nullptr, *h_row_ptr = nullptr, *h_totals = nullptr;   // page-locked staging
+        uint64_t *h_row_ptr = nullptr, *h_totals = nullptr;   // page-locked staging
     } slot[2];
     int rc = KTB_OK;
-    auto step = [&](cudaError_t e, const char *what) {
-        if (rc == KTB_OK && e != cudaSuccess) rc = cuda_fail(what, e);
-    };
+    FirstError step{rc};
     for (Slot &s : slot) {
-        step(cudaStreamCreateWithFlags(&s.st, cudaStreamNonBlocking), "cudaStreamCreate");
-        step(cudaMalloc((void **)&s.bases, std::max<uint64_t>(max_bases, 1)), "cudaMalloc(bases)");
-        step(cudaMalloc((void **)&s.offsets, (max_n + 1) * sizeof(uint64_t)), "cudaMalloc(offsets)");
-        step(cudaMalloc((void **)&s.row_ptr, (max_n + 1) * sizeof(uint64_t)), "cudaMalloc(row_ptr)");
-        step(cudaMalloc((void **)&s.totals, max_n * sizeof(uint64_t)), "cudaMalloc(totals)");
-        step(cudaMalloc((void **)&s.codes, std::max<uint64_t>(max_windows, 1) * sizeof(uint64_t)), "cudaMalloc(codes)");
-        step(cudaMalloc(&s.values, std::max<uint64_t>(max_windows, 1) * esize), "cudaMalloc(values)");
-        step(cudaHostAlloc((void **)&s.h_offsets, (max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
-             "cudaHostAlloc(offsets)");
-        step(cudaHostAlloc((void **)&s.h_row_ptr, (max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
+        s.alloc(plan, step);
+        step(cudaMalloc((void **)&s.row_ptr, (plan.max_n + 1) * sizeof(uint64_t)), "cudaMalloc(row_ptr)");
+        step(cudaMalloc((void **)&s.totals, plan.max_n * sizeof(uint64_t)), "cudaMalloc(totals)");
+        step(cudaMalloc((void **)&s.codes, max_windows * sizeof(uint64_t)), "cudaMalloc(codes)");
+        step(cudaMalloc(&s.values, max_windows * esize), "cudaMalloc(values)");
+        step(cudaHostAlloc((void **)&s.h_row_ptr, (plan.max_n + 1) * sizeof(uint64_t), cudaHostAllocDefault),
              "cudaHostAlloc(row_ptr)");
-        step(cudaHostAlloc((void **)&s.h_totals, max_n * sizeof(uint64_t), cudaHostAllocDefault), "cudaHostAlloc(totals)");
+        step(cudaHostAlloc((void **)&s.h_totals, plan.max_n * sizeof(uint64_t), cudaHostAllocDefault),
+             "cudaHostAlloc(totals)");
     }
-    const uint64_t nchunks = cut.size() - 1;
+    const uint64_t nchunks = plan.chunks();
     auto enqueue = [&](uint64_t ci) {
         Slot &s = slot[ci & 1];
-        const uint64_t i0 = cut[ci], i1 = cut[ci + 1], cn = i1 - i0, b0 = offsets[i0], nb = offsets[i1] - b0;
-        for (uint64_t i = 0; i <= cn; ++i) s.h_offsets[i] = offsets[i0 + i] - b0;
-        if (nb) step(cudaMemcpyAsync(s.bases, bases + b0, nb, cudaMemcpyHostToDevice, s.st), "cudaMemcpyAsync(bases)");
-        step(cudaMemcpyAsync(s.offsets, s.h_offsets, (cn + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s.st),
-             "cudaMemcpyAsync(offsets)");
+        const Chunk ch = plan[ci];
+        s.copy_in(plan, ci, step);
         if (rc == KTB_OK)
-            rc = ktb_sparse_vectorise_device(s.bases, s.offsets, cn, nb, k, canonical, norm_mode, out_dtype, s.row_ptr,
-                                             s.codes, s.values, std::max<uint64_t>(max_windows, 1), s.totals, s.st);
-        step(cudaMemcpyAsync(s.h_row_ptr, s.row_ptr, (cn + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
+            rc = ktb_sparse_vectorise_device(s.bases, s.offsets, ch.n, ch.nb, k, canonical, norm_mode, out_dtype,
+                                             s.row_ptr, s.codes, s.values, max_windows, s.totals, s.st);
+        step(cudaMemcpyAsync(s.h_row_ptr, s.row_ptr, (ch.n + 1) * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
              "cudaMemcpyAsync(row_ptr)");
         if (totals)
-            step(cudaMemcpyAsync(s.h_totals, s.totals, cn * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
+            step(cudaMemcpyAsync(s.h_totals, s.totals, ch.n * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
                  "cudaMemcpyAsync(totals)");
     };
     uint64_t written = 0;   // entries of the rows before the current chunk
@@ -259,9 +211,10 @@ int ktb_sparse_vectorise(const uint8_t *bases, const uint64_t *offsets, uint64_t
         Slot &s = slot[ci & 1];
         step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");
         if (rc != KTB_OK) break;
-        const uint64_t i0 = cut[ci], cn = cut[ci + 1] - i0, nnz = s.h_row_ptr[cn];
-        for (uint64_t i = 0; i <= cn; ++i) row_ptr[i0 + i] = written + s.h_row_ptr[i];
-        if (totals) std::copy(s.h_totals, s.h_totals + cn, totals + i0);
+        const Chunk ch = plan[ci];
+        const uint64_t nnz = s.h_row_ptr[ch.n];
+        for (uint64_t i = 0; i <= ch.n; ++i) row_ptr[ch.i0 + i] = written + s.h_row_ptr[i];
+        if (totals) std::copy(s.h_totals, s.h_totals + ch.n, totals + ch.i0);
         const uint64_t ncopy = written >= cap ? 0 : std::min(nnz, cap - written);
         if (ncopy) {   // ordered on this slot's stream before its next chunk is copied in
             step(cudaMemcpyAsync(codes + written, s.codes, ncopy * sizeof(uint64_t), cudaMemcpyDeviceToHost, s.st),
@@ -272,17 +225,13 @@ int ktb_sparse_vectorise(const uint8_t *bases, const uint64_t *offsets, uint64_t
         written += nnz;
     }
     for (Slot &s : slot) {
-        if (s.st) step(cudaStreamSynchronize(s.st), "cudaStreamSynchronize");
-        cudaFree(s.bases);
-        cudaFree(s.offsets);
+        s.release(step);
         cudaFree(s.row_ptr);
         cudaFree(s.totals);
         cudaFree(s.codes);
         cudaFree(s.values);
-        cudaFreeHost(s.h_offsets);
         cudaFreeHost(s.h_row_ptr);
         cudaFreeHost(s.h_totals);
-        if (s.st) cudaStreamDestroy(s.st);
     }
     return rc;
 }

@@ -12,10 +12,9 @@ import numpy as np
 
 from . import _lib
 from ._lib import NORM_CLI, NORM_COUNTS, OUT_F32, OUT_F64, OUT_U32
-from .oligo import _pack
+from .oligo import _CODES, _pack
 
 MAX_SPARSE_K = 31
-_CODES = {np.dtype(np.uint32): OUT_U32, np.dtype(np.float32): OUT_F32, np.dtype(np.float64): OUT_F64}
 
 
 def _packed(seqs_or_packed):
@@ -29,6 +28,20 @@ def _check_k(ksize: int) -> int:
     if not 1 <= int(ksize) <= MAX_SPARSE_K:
         raise ValueError(f"ksize must be in 1..{MAX_SPARSE_K} (got {ksize})")
     return int(ksize)
+
+
+def _check_tensors(bases, offsets, device=None):
+    """Checks the CUDA tensors of a batch (uint8 bases, int64 offsets); a counter also passes the device index they must
+    be on."""
+    import torch
+    if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
+        raise ValueError("bases and offsets must be CUDA tensors on one device")
+    if device is not None and bases.device.index != device:
+        raise ValueError(f"the tensors are on {bases.device}, the counter on cuda:{device}")
+    if bases.dtype != torch.uint8 or offsets.dtype != torch.int64:
+        raise TypeError(f"bases must be uint8 and offsets int64 (got {bases.dtype}, {offsets.dtype})")
+    if not (bases.is_contiguous() and offsets.is_contiguous()):
+        raise ValueError("bases and offsets must be contiguous")
 
 
 @functools.lru_cache(maxsize=4)
@@ -82,12 +95,7 @@ def kmer_counts_tensors(bases, offsets, ksize: int, mins: bool = True, norm_mode
     buffer, pass the slice bases[offsets[0]:offsets[n]] and offsets - offsets[0]."""
     import torch
     k = _check_k(ksize)
-    if not (bases.is_cuda and offsets.is_cuda and bases.device == offsets.device):
-        raise ValueError("bases and offsets must be CUDA tensors on one device")
-    if bases.dtype != torch.uint8 or offsets.dtype != torch.int64:
-        raise TypeError(f"bases must be uint8 and offsets int64 (got {bases.dtype}, {offsets.dtype})")
-    if not (bases.is_contiguous() and offsets.is_contiguous()):
-        raise ValueError("bases and offsets must be contiguous")
+    _check_tensors(bases, offsets)
     if columns not in ("code", "rank"):
         raise ValueError(f"columns must be 'code' or 'rank' (got {columns!r})")
     if columns == "rank" and (not mins or k > _lib.MAX_K):

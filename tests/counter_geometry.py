@@ -21,7 +21,7 @@ SP_WB = 4096                 # SP_WB (sparse_common.cuh): entries per block of t
 SP_WITEMS = 16               # SP_WITEMS: consecutive entries per thread of those kernels
 SCAN_TOP = 1024              # block sums sparse_scan_top_kernel scans per pass of its carry loop
 SCAN_PASS = SCAN_TOP * SP_WB                     # 2^22 entries: one pass of that loop
-COUNT_CHUNK_BASES = 1 << 26  # COUNT_CHUNK_BASES (counter.cu): bases per chunk of the host entry point
+HOST_CHUNK_BASES = 1 << 26   # HOST_CHUNK_BASES (host_common.h): bases per chunk of the host entry points
 SLICE = 1 << 22              # keys per output slice of ktb_count_file
 MAX_RECORDS = 4 << 20        # records per parse batch of ktb_count_file
 MERGE_GRID = 148 * 16 * 256  # threads of the grid-stride merge kernels on a 148-SM B200 (sms * 16 CTAs of 256)
@@ -179,12 +179,12 @@ def merge_geometry(table_keys, batch_keys) -> Merge:
 
 
 def host_chunks(offsets):
-    """(i0, i1, bases) of the host entry point's chunks: whole sequences, at most COUNT_CHUNK_BASES bases each unless one
-    sequence is longer (the cut loop of ktb_counter_add).  A chunk with no bases is skipped by the add."""
+    """(i0, i1, bases) of the host entry points' chunks: whole sequences, at most HOST_CHUNK_BASES bases each unless one
+    sequence is longer (ChunkPlan in host_common.h).  A chunk with no bases is skipped by the add."""
     off = np.asarray(offsets, dtype=np.int64)
     n, cuts, i0 = len(off) - 1, [], 0
     while i0 < n:
-        i1 = max(i0 + 1, min(n, int(np.searchsorted(off, off[i0] + COUNT_CHUNK_BASES, "right")) - 1))
+        i1 = max(i0 + 1, min(n, int(np.searchsorted(off, off[i0] + HOST_CHUNK_BASES, "right")) - 1))
         cuts.append((i0, i1, int(off[i1] - off[i0])))
         i0 = i1
     return cuts

@@ -127,13 +127,13 @@ def test_merge_geometry_equals_bisect():
 
 
 def test_host_chunks_is_the_cut_loop(monkeypatch):
-    monkeypatch.setattr(cg, "COUNT_CHUNK_BASES", 100)
+    monkeypatch.setattr(cg, "HOST_CHUNK_BASES", 100)
     rng = np.random.default_rng(4)
     for _ in range(200):
         lens = rng.choice([0, 0, 1, 30, 99, 100, 101, 250], size=rng.integers(1, 20))
         off = np.r_[0, np.cumsum(lens)].astype(np.uint64)
         cut, i0, n = [], 0, len(lens)
-        while i0 < n:   # ktb_counter_add's loop, as written there
+        while i0 < n:   # the loop of ChunkPlan (host_common.h), as written there
             i1 = i0 + 1
             while i1 < n and off[i1 + 1] - off[i0] <= 100:
                 i1 += 1

@@ -34,7 +34,7 @@ ROOT = Path(__file__).resolve().parent.parent
 BIN = ROOT / "kmertools_b200" / "bin" / "kmertools"
 DEV = torch.device("cuda", 0)
 T = cg.CT_T
-CHUNK = cg.COUNT_CHUNK_BASES
+CHUNK = cg.HOST_CHUNK_BASES
 
 
 # ------------------------------------------------------------------------------------------------------------- helpers

@@ -17,6 +17,7 @@ from hypothesis import HealthCheck, given, settings, strategies as st
 
 from kmertools_b200 import OligoComputer, _lib, kmer_counts
 from oracle import oracle
+from tests.counter_geometry import HOST_CHUNK_BASES, host_chunks
 from tests.sparse_ref import scatter, sparse_rows
 from tests.test_gpu_hypothesis import ALPHABETS
 from tests.test_gpu_sparse import COMBOS, DT, _dev_rows, _finish
@@ -29,7 +30,6 @@ T = 4096                     # SP_T (sparse_kernels.cuh): window-end positions p
 SP_WB = 4096                 # SP_WB (sparse_kernels.cuh): entries per block of the scans and the count / write passes
 SCAN_TOP = 1024              # block sums sparse_scan_top_kernel (sparse_kernels.cuh) scans per pass of its carry loop
 SCAN_PASS = SCAN_TOP * SP_WB                      # 4,194,304 sequences: one pass of the carry loop
-CHUNK = 1 << 26              # SPARSE_CHUNK_BASES (sparse.cu): bases of one chunk of the host entry point
 SENT = np.uint64(0xFFFF_FFFF_FFFF_FFF7)          # above every code (< 4^31), offset and total of these batches
 VSENT = {0: np.uint32(0xFFFF_FFF9), 1: np.float32(-7.5), 2: np.float64(-7.25)}
 
@@ -88,18 +88,6 @@ def piece_keys(bases, offsets, k: int, canonical, s: int):
         f, r, _ = oracle.kmer_arrays(bases[lo:hi], k)
         out.append(np.unique(np.minimum(f, r) if canonical else f))
     return out
-
-
-def host_chunks(offsets):
-    """[i0, i1) sequence ranges of the host entry point's chunks: whole sequences, at most CHUNK bases each unless one
-    sequence is longer (the cut loop of ktb_sparse_vectorise)."""
-    off = np.asarray(offsets, dtype=np.int64)
-    n, cuts, i0 = len(off) - 1, [], 0
-    while i0 < n:
-        i1 = max(i0 + 1, min(n, int(np.searchsorted(off, off[i0] + CHUNK, "right")) - 1))
-        cuts.append((i0, i1))
-        i0 = i1
-    return cuts
 
 
 # ---------------------------------------------------------------------------------------------------------- references
@@ -456,7 +444,7 @@ def test_scan_carry_loop(short_reads, canonical):
         assert_rows(got, w, np.uint32, f"device n={n}")
     del tb, to
     torch.cuda.empty_cache()
-    cuts = host_chunks(offsets)
+    cuts = [c[:2] for c in host_chunks(offsets)]
     assert len(cuts) >= 2 and max(i1 - i0 for i0, i1 in cuts) > SCAN_PASS
     assert_rows(kmer_counts((bases, offsets), k, bool(canonical), 0, np.uint32), want, np.uint32, "host")
 
@@ -515,7 +503,7 @@ def chunked_batch():
     repeat with 20,000 point changes.  Returns bases, offsets and the reference rows at k = 21, canonical, NORM_CLI."""
     rng = np.random.default_rng(500)
     k = 21
-    big = np.resize(np.frombuffer(b"GATTACA", np.uint8), CHUNK + 5000)
+    big = np.resize(np.frombuffer(b"GATTACA", np.uint8), HOST_CHUNK_BASES + 5000)
     big[rng.choice(len(big), size=20_000, replace=False)] = ALPHA[rng.integers(0, 4, 20_000)]
     parts = []
     for lens in ([150] + list(rng.integers(0, 400, size=3000)), [0, 0] + list(rng.integers(0, 400, size=3000)) + [0]):
@@ -532,10 +520,11 @@ def chunked_batch():
 def test_host_entry_chunks_and_cap(chunked_batch):
     bases, offsets, want = chunked_batch
     k, cn, norm, code = 21, 1, 1, 1
-    cuts = host_chunks(offsets)
+    cuts = [c[:2] for c in host_chunks(offsets)]
     nb = [int(offsets[i1] - offsets[i0]) for i0, i1 in cuts]
     assert len(cuts) == 5 and cuts[1][1] - cuts[1][0] == 1 and cuts[3][1] - cuts[3][0] == 1
-    assert nb[1] == nb[3] == CHUNK + 5000 and nb[4] == 0 and cuts[4][1] - cuts[4][0] == 3   # the empty last chunk
+    assert nb[1] == nb[3] == HOST_CHUNK_BASES + 5000
+    assert nb[4] == 0 and cuts[4][1] - cuts[4][0] == 3   # the empty last chunk
     rp = want[0]
     first = [int(rp[i0]) for i0, _ in cuts] + [int(rp[-1])]       # first entry of each chunk
     nnz = first[-1]
